@@ -1,14 +1,15 @@
 #!/usr/bin/env python
 """bench.py — headline benchmark of the self-play hot path (contract: see DESIGN.md §Measurement).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--boards B]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--boards B] [--dump-outputs DIR]
 
 A "step" is one pass of legal-placement enumeration over BASELINE config 2: B = 1,000,000
 random s2 boards x 7 current pieces with a second (hold) piece = 7,000,000 get_move_matrix
 calls per GPU (weak scaling: every rank owns its own board shard, no collective on the data
 path).  `value` = placements/s with inputs resident in HBM; `e2e` = the same metric through the
 reference-facing C-ABI call with pinned HOST buffers (H2D + kernel + D2H inside the timed region).
-One JSON line is printed by rank 0.
+One JSON line is printed by rank 0.  The workload is seeded, so the same arguments give the same inputs in every
+run; --dump-outputs DIR writes what the last timed step returned (see dump_outputs) for comparing two builds.
 """
 import argparse
 import json
@@ -148,6 +149,30 @@ class ClockSampler:
 def make_workload(n_boards, rank):
     from tetris_reinforcement_learning_b200 import synth
     return synth.movegen_workload(n_boards, seed=synth.DEFAULT_SEED + 1000 * rank)
+
+
+DUMP_CALLS = 8192   # sampled calls: 8192 x 1448 mask bytes x 4 B = 47.4 MB keeps a dump under 64 MB
+
+
+def dump_outputs(out_dir, d_mask, d_n, d_st):
+    """What the sweep returned to its caller for a fixed, seeded sample of the calls, as out_dir/<name>.npy:
+    call_index (which calls), mask_bytes (the bit-packed (27,39,11) masks as their 1448 little-endian bytes),
+    n_moves, and status_bits (the 32 TRL_ST_* bits of the status word, bit j in column j).  Values are small
+    integers in float32, so a single flipped mask bit or status flag fails a comparison at any relative tolerance
+    below 1e-3.  Two builds run with the same arguments dump the same calls and can be compared array by array."""
+    import torch
+    n = d_mask.shape[0]
+    idx = np.sort(np.random.default_rng(0).choice(n, size=min(n, DUMP_CALLS), replace=False))
+    sel = torch.from_numpy(idx).to(d_mask.device)
+    mask = np.ascontiguousarray(d_mask[sel].cpu().numpy().astype("<u4"))
+    status = np.ascontiguousarray(d_st[sel].cpu().numpy().astype("<u4"))
+    arrays = {"call_index": idx.astype(np.float64),
+              "mask_bytes": mask.view(np.uint8).astype(np.float32),
+              "n_moves": d_n[sel].cpu().numpy().view(np.uint16).astype(np.float32),
+              "status_bits": np.unpackbits(status.view(np.uint8).reshape(-1, 4), axis=1, bitorder="little").astype(np.float32)}
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), a)
 
 
 def cpu_baseline(boards, cur, alt, target_s=12.0, device_masks=None, device_counts=None):
@@ -553,6 +578,8 @@ def run_ours(args, rank, world, local_rank):
     clocks = sampler.stop()
     kernel_ms = [ev[k].elapsed_time(ev[k + 1]) for k in range(args.steps)]
     total_ms = ev[0].elapsed_time(ev[args.steps])
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, d_mask, d_n, d_st)
 
     # ---- e2e: the reference-facing host call with pinned host buffers ----
     h_boards = torch.from_numpy(boards.view(np.int16)).pin_memory()
@@ -745,7 +772,14 @@ def main():
     ap.add_argument("--cpu-selfplay-seconds", type=float, default=12.0)
     ap.add_argument("--cpu-selfplay-worker", type=float, default=0.0, help=argparse.SUPPRESS)
     ap.add_argument("--worker-index", type=int, default=0, help=argparse.SUPPRESS)
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write a seeded sample of the last sweep's outputs (rank 0's shard) "
+                         "as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs needs --impl ours")
     if args.cpu_selfplay_worker > 0:
         os.dup2(_REAL_STDOUT, 1)
         cpu_selfplay_worker(args.cpu_selfplay_worker, args.worker_index)

@@ -79,11 +79,12 @@ def test_generate_games_raises_on_device_status():
         assert lib.trl_debug_movegen_fifo_limit(0) == 0
 
 
-def test_save_all_with_random_openings_generates_a_set():
+def test_save_all_with_random_openings_generates_a_set(tmp_path, monkeypatch):
     """ADVICE r1: save_all + use_random_starting_moves used to store records of one-iteration opening searches with
     zero visits, which crashed the target construction (assert total != 0)."""
     import torch
     from tetris_reinforcement_learning_b200 import ai
+    monkeypatch.setenv("TRL_STORAGE", str(tmp_path / "Storage"))   # generate_games numbers the set from <data_dir>
     cfg = _cfg(use_random_starting_moves=True, save_all=True, use_playout_cap_randomization=True, MAX_ITER=8)
     for compact in (False, True):
         data, stats = ai.generate_games(cfg, fake_evaluator_torch(torch.device("cuda:0")), 12, seed=5, dtype=torch.float32,
