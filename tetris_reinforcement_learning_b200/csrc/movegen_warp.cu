@@ -112,7 +112,8 @@ __device__ __forceinline__ void flag_cell(uint32_t* fu_row, uint32_t bit, bool u
 // (rows 12..43; the spawn row is >= 19 and nothing above it can be entered without kicks):
 //
 //   * two rotations share a register (16 bits each, validity rows are 14 bits wide, the two spare bits
-//     stop the carries of hflood): VA/VB validity, RA/RB reached;
+//     stop the carries of hflood): VA/VB validity, RA/RB reached; A holds rotations 0 | 2 << 16, B 1 | 3 << 16,
+//     so that each pair of kick passes with equal kick lists runs in one word (kick_pass_pair);
 //   * fill = alternate "expand along rows" (hflood, O(1)) and "fall straight down" (a segmented
 //     Hillis-Steele OR-scan over lanes, 5 shuffles, propagate masks precomputed) until nothing changes —
 //     all four rotations at once, instead of one serial row scan per queue entry;
@@ -201,22 +202,50 @@ constexpr KickList kIKicks[4][3] = {
     {{5, {{0, 0}, {1, 0}, {-2, 0}, {1, -2}, {-2, 1}, {0, 0}}}, {2, {{0, 0}, {-1, 0}, {0, 0}, {0, 0}, {0, 0}, {0, 0}}}, {5, {{0, 0}, {-2, 0}, {1, 0}, {-2, -1}, {1, 2}, {0, 0}}}},
 };
 
+constexpr bool same_kicks(const KickList& a, const KickList& b) {
+    if (a.n != b.n) return false;
+    for (int ki = 0; ki < a.n; ++ki)
+        if (a.k[ki][0] != b.k[ki][0] || a.k[ki][1] != b.k[ki][1]) return false;
+    return true;
+}
+// The four twin pairs kick_pass_pair runs in one 32-bit word (lists equal offset for offset, const.py:191-212)
+static_assert(same_kicks(kWallKicks[0][0], kWallKicks[2][2]), "twin pair (0, 0) / (2, 2)");
+static_assert(same_kicks(kWallKicks[0][2], kWallKicks[2][0]), "twin pair (0, 2) / (2, 0)");
+static_assert(same_kicks(kWallKicks[1][0], kWallKicks[1][2]), "twin pair (1, 0) / (1, 2)");
+static_assert(same_kicks(kWallKicks[3][0], kWallKicks[3][2]), "twin pair (3, 0) / (3, 2)");
+
+#ifdef TRL_MOVEGEN_STATS
+#define TRL_COUNT(x) (++(x))
+#else
+#define TRL_COUNT(x) ((void)0)
+#endif
+
+// Rotation r's validity row (<< 2) in the packed planes vv[r & 1], shifted right by `sh`: source bit ex of a kick test
+// <-> target bit ex + kx for sh = kx + 2.  The other rotation of the plane starts at bit 18, above anything a 14-bit edge
+// row reaches with kx <= 2.
+#define TRL_VV(S, r, row, sh) ((S).vv[(r) & 1][row] >> ((sh) + 16 * ((r) >> 1)))
+
 // One (source rotation R, direction KD) pass over the new edge cells `ne` of this lane's row; TAB 0 = the six pieces
 // with the common wall-kick table, 1 = the I piece.
 template <int TAB, int R, int KD, class St>
-__device__ __forceinline__ void kick_pass_wall(St& S, int lane, uint32_t ne, uint32_t VA, uint32_t VB, uint32_t& a0A, uint32_t& a0B, bool is_T) {
+__device__ __forceinline__ void kick_pass_wall(St& S, int lane, uint32_t ne, uint32_t VA, uint32_t VB, uint32_t& a0A, uint32_t& a0B, bool is_T,
+                                               unsigned& n_pass, unsigned& n_test) {
     constexpr int nrot = (R + KD + 1) & 3;
     constexpr KickList K = TAB ? kIKicks[R][KD] : kWallKicks[R][KD];
+#ifdef TRL_MOVEGEN_STATS
+    if (__any_sync(0xffffffffu, ne)) TRL_COUNT(n_pass);
+#endif
     // kick 0 is (0, 0) in every list (const.py:191-235): target = same cell of the new rotation
-    const uint32_t Vn = ((nrot & 2) ? VB : VA) >> (16 * (nrot & 1));
+    const uint32_t Vn = ((nrot & 1) ? VB : VA) >> (16 * (nrot >> 1));
     const uint32_t c0 = ne & Vn;
-    if (nrot & 2) a0B |= c0 << (16 * (nrot & 1)); else a0A |= c0 << (16 * (nrot & 1));
+    if (nrot & 1) a0B |= c0 << (16 * (nrot >> 1)); else a0A |= c0 << (16 * (nrot >> 1));
     uint32_t rem = ne & ~c0;
     if (!__any_sync(0xffffffffu, rem)) return;
 #pragma unroll
     for (int ki = 1; ki < K.n; ++ki) {
+        TRL_COUNT(n_test);
         const int kx = K.k[ki][0], ky = K.k[ki][1];
-        const uint32_t cand = rem & (S.vv[nrot][lane + 2 - ky] >> (kx + 2));   // source bit ex <-> target bit ex + kx
+        const uint32_t cand = rem & TRL_VV(S, nrot, lane + 2 - ky, kx + 2);   // source bit ex <-> target bit ex + kx
         rem &= ~cand;
         if (cand) {
             uint32_t arr = kx >= 0 ? (cand << kx) : (cand >> -kx);
@@ -228,13 +257,79 @@ __device__ __forceinline__ void kick_pass_wall(St& S, int lane, uint32_t ne, uin
 }
 
 template <int TAB, int R, class St>
-__device__ __forceinline__ void kick_passes_wall(St& S, int lane, uint32_t ne, uint32_t VA, uint32_t VB, uint32_t& a0A, uint32_t& a0B, bool is_T) {
-    kick_pass_wall<TAB, R, 0>(S, lane, ne, VA, VB, a0A, a0B, is_T);
-    kick_pass_wall<TAB, R, 1>(S, lane, ne, VA, VB, a0A, a0B, is_T);
-    kick_pass_wall<TAB, R, 2>(S, lane, ne, VA, VB, a0A, a0B, is_T);
+__device__ __forceinline__ void kick_passes_wall(St& S, int lane, uint32_t ne, uint32_t VA, uint32_t VB, uint32_t& a0A, uint32_t& a0B, bool is_T,
+                                                 unsigned& n_pass, unsigned& n_test) {
+    kick_pass_wall<TAB, R, 0>(S, lane, ne, VA, VB, a0A, a0B, is_T, n_pass, n_test);
+    kick_pass_wall<TAB, R, 1>(S, lane, ne, VA, VB, a0A, a0B, is_T, n_pass, n_test);
+    kick_pass_wall<TAB, R, 2>(S, lane, ne, VA, VB, a0A, a0B, is_T, n_pass, n_test);
 }
 
-// St: anything with uint32_t vv[4][>= kWinRows], fu[4][>= kWinRows] in shared memory.  The loops are kept
+// Two (source rotation, direction) passes of the common wall-kick table with equal kick lists, one per 16-bit half:
+//   R even (pair (R, KD) / (R ^ 2, KD ^ 2)): src = the packed rot0 | rot2 edge cells, both halves target the odd
+//     rotation nrot, whose validity row is duplicated into both halves;
+//   R odd (pair (R, KD) / (R, KD ^ 2)): src = rotation R's edge cells in both halves, the low half targets rotation 0,
+//     the high half rotation 2: the packed validity plane vv[0] as it is.
+// "First valid kick wins" runs per bit, so each half computes exactly its own pass.  No bit crosses between the halves: the
+// edge bits of a half sit in 0..13, a kick test reads target bits ex + kx + 2 <= 16 (bit 16 of the word, and of the
+// duplicated word, is always 0), and an arrival cannot leave its half downwards since `cand` implies ex + kx >= 0.  Both
+// directions of every pair are != 1 (KD ^ 2 = 2 - KD), so the used-last-kick rule is the same for the two halves.
+template <int R, int KD, class St>
+__device__ __forceinline__ void kick_pass_pair(St& S, int lane, uint32_t src, uint32_t VA, uint32_t VB, uint32_t& a0A, uint32_t& a0B, bool is_T,
+                                               unsigned& n_pass, unsigned& n_test) {
+    static_assert(KD != 1, "the 180-degree passes have no twin");
+    constexpr KickList K = kWallKicks[R][KD];
+    constexpr int nrot = (R + KD + 1) & 3;
+    static_assert((R & 1) ? nrot == 0 : (nrot & 1) != 0, "low half of an odd source targets rotation 0, an even source an odd rotation");
+    constexpr uint32_t dup = nrot == 1 ? 0x1010u : 0x3232u;   // PRMT: the low / high half of the odd plane in both halves
+#ifdef TRL_MOVEGEN_STATS
+    if (__any_sync(0xffffffffu, src)) TRL_COUNT(n_pass);
+#endif
+    uint32_t rem;
+    if constexpr ((R & 1) == 0) {
+        const uint32_t c0 = src & __byte_perm(VB, 0u, dup);
+        a0B |= nrot == 1 ? ((c0 | (c0 >> 16)) & 0xFFFFu) : ((c0 | (c0 << 16)) & 0xFFFF0000u);
+        rem = src & ~c0;
+    } else {
+        const uint32_t c0 = src & VA;
+        a0A |= c0;
+        rem = src & ~c0;
+    }
+    if (!__any_sync(0xffffffffu, rem)) return;
+#pragma unroll
+    for (int ki = 1; ki < K.n; ++ki) {
+        TRL_COUNT(n_test);
+        const int kx = K.k[ki][0], ky = K.k[ki][1];
+        const int row = lane + 2 - ky;
+        uint32_t tw;
+        if constexpr ((R & 1) == 0) tw = __byte_perm(S.vv[1][row], 0u, dup);
+        else tw = S.vv[0][row];
+        const uint32_t cand = rem & (tw >> (kx + 2));
+        rem &= ~cand;
+        if (cand) {
+            const uint32_t arr = kx >= 0 ? (cand << kx) : (cand >> -kx);
+            const bool ulk = ki == K.n - 1 && is_T;                           // nulk (:469)
+            if constexpr ((R & 1) == 0) {
+                const uint32_t a = (arr | (arr >> 16)) & 0xFFFFu;
+                atomicOr(&S.fu[nrot][row], ulk ? a << 16 : a);
+            } else {
+                const uint32_t lo = ulk ? arr << 16 : arr & 0xFFFFu, hi = ulk ? arr & 0xFFFF0000u : arr >> 16;
+                if (lo) atomicOr(&S.fu[0][row], lo);
+                if (hi) atomicOr(&S.fu[2][row], hi);
+            }
+        }
+        if (ki + 1 < K.n && !__any_sync(0xffffffffu, rem)) return;
+    }
+}
+
+// (rot0 | rot2 << 16, rot1 | rot3 << 16) <-> (rot0 | rot1 << 16, rot2 | rot3 << 16): exchange the high half of A with the
+// low half of B (its own inverse)
+__device__ __forceinline__ void swap_mid_halves(uint32_t& A, uint32_t& B) {
+    const uint32_t a = __byte_perm(A, B, 0x5410), b = __byte_perm(A, B, 0x7632);
+    A = a;
+    B = b;
+}
+
+// St: anything with uint32_t vv[>= 2][>= kWinRows], fu[4][>= kWinRows] in shared memory.  The loops are kept
 // rolled on purpose: the kernels that call this are bound by instruction fetch, not by loop overhead.
 // ---------------------------------------------------------------------------------------
 // T: which flag did the LAST rotation-flagged emission of a cell carry, when it received both?
@@ -268,6 +363,12 @@ __device__ __noinline__ bool t_order_decide(St& S, int lane, uint32_t VA, uint32
                                             uint32_t placedA, uint32_t placedB, uint32_t a0A, uint32_t a0B, bool snapped,
                                             uint32_t mixed_rots, uint32_t& ulkA, uint32_t& ulkB) {
     constexpr unsigned kAll = 0xffffffffu;
+    // The closure search packs rotations (0 | 2, 1 | 3); this cold function works on (0 | 1, 2 | 3) pairs.
+    swap_mid_halves(VA, VB);
+    swap_mid_halves(placedA, placedB);
+    swap_mid_halves(a0A, a0B);
+    uint32_t oulkA = ulkA, oulkB = ulkB;
+    swap_mid_halves(oulkA, oulkB);
     const uint32_t PA1 = lane >= 1 ? VA : 0u, PB1 = lane >= 1 ? VB : 0u;
     const uint32_t PA2 = PA1 & __shfl_up_sync(kAll, PA1, 1), PB2 = PB1 & __shfl_up_sync(kAll, PB1, 1);
     const uint32_t PA4 = PA2 & __shfl_up_sync(kAll, PA2, 2), PB4 = PB2 & __shfl_up_sync(kAll, PB2, 2);
@@ -296,7 +397,7 @@ __device__ __noinline__ bool t_order_decide(St& S, int lane, uint32_t VA, uint32
 #pragma unroll 1
         for (int ki = 0; ki < kn; ++ki) {
             const int kx = K.k[ki][0], ky = K.k[ki][1];
-            const uint32_t cand = rem & (S.vv[nrot][lane + 2 - ky] >> (kx + 2));
+            const uint32_t cand = rem & TRL_VV(S, nrot, lane + 2 - ky, kx + 2);
             rem &= ~cand;
             const bool is_u = kd != 1 && ki == kn - 1;
             const bool hi = kd != 1 && !is_u && (ky > lky || (ky == lky && kx < lkx));   // source later in the scan than the last kick's
@@ -365,7 +466,7 @@ __device__ __noinline__ bool t_order_decide(St& S, int lane, uint32_t VA, uint32
 #pragma unroll 1
     for (int R = 0; R < 4; ++R) {
         if (!((mixed_rots >> R) & 1u)) {   // no cell of this rotation needs a decision: its flags are the union of the arrivals
-            ulk[R] = (((R & 2) ? ulkB : ulkA) >> (16 * (R & 1))) & 0xFFFFu;
+            ulk[R] = (((R & 2) ? oulkB : oulkA) >> (16 * (R & 1))) & 0xFFFFu;
             continue;
         }
         zero_planes();
@@ -418,8 +519,8 @@ __device__ __noinline__ bool t_order_decide(St& S, int lane, uint32_t VA, uint32
     }
     if (__any_sync(kAll, undecided)) { TRL_REASON(14); return false; }
     TRL_REASON(15);
-    ulkA = ulk[0] | (ulk[1] << 16);
-    ulkB = ulk[2] | (ulk[3] << 16);
+    ulkA = ulk[0] | (ulk[2] << 16);
+    ulkB = ulk[1] | (ulk[3] << 16);
     return true;
 }
 
@@ -451,7 +552,7 @@ __device__ __forceinline__ void validity_rows(const uint32_t (&e)[4], uint32_t (
     v[3] = validity_row<TYPE, 3>(e);
 }
 
-// SPECIAL: kick passes of the non-I pieces with compile-time tables (the closure kernel; costs 11 KB of code).
+// SPECIAL: kick passes of the non-I pieces with compile-time tables, twin passes packed (the closure kernel).
 template <bool SPECIAL, class St>
 __device__ __forceinline__ bool search_piece_rows(St& S, const uint16_t* rows, int hi, int type, bool via_hold, uint32_t* mask) {
     const int lane = threadIdx.x & 31;
@@ -474,15 +575,8 @@ __device__ __forceinline__ bool search_piece_rows(St& S, const uint16_t* rows, i
             case 5: validity_rows<5>(e, v); break;
             default: validity_rows<6>(e, v); break;
         }
-        const int pad = lane < 2 ? lane : lane + 32;
-#pragma unroll
-        for (int r = 0; r < 4; ++r) {
-            S.vv[r][lane + 2] = v[r] << 2;
-            S.fu[r][lane + 2] = 0u;
-            if (lane < 4) { S.vv[r][pad] = 0u; S.fu[r][pad] = 0u; }
-        }
-        VA = v[0] | (v[1] << 16);
-        VB = v[2] | (v[3] << 16);
+        VA = v[0] | (v[2] << 16);
+        VB = v[1] | (v[3] << 16);
     } else {
 #pragma unroll 1
     for (int r = 0; r < 4; ++r) {
@@ -494,18 +588,22 @@ __device__ __forceinline__ bool search_piece_rows(St& S, const uint16_t* rows, i
             const uint32_t ek = ro == 0 ? e[0] : (ro == 1 ? e[1] : (ro == 2 ? e[2] : e[3]));
             acc &= ek >> co;
         }
-        // shared planes, row index lane + 2: validity << 2 for the kick tests, arrivals (T: low half = flag
-        // clear, high half = used-last-kick)
-        S.vv[r][lane + 2] = acc << 2;
-        S.fu[r][lane + 2] = 0u;
-        if (lane < 4) {
-            const int pad = lane < 2 ? lane : lane + 32;
-            S.vv[r][pad] = 0u;
-            S.fu[r][pad] = 0u;
-        }
-        const uint32_t sh = acc << (16 * (r & 1));
-        if (r & 2) VB |= sh; else VA |= sh;
+        const uint32_t sh = acc << (16 * (r >> 1));
+        if (r & 1) VB |= sh; else VA |= sh;
     }
+    }
+    // shared planes, row index lane + 2: validity << 2 for the kick tests, packed like VA / VB (TRL_VV); arrivals per
+    // rotation (T: low half = flag clear, high half = used-last-kick)
+    {
+        const int pad = lane < 2 ? lane : lane + 32;
+        S.vv[0][lane + 2] = VA << 2;
+        S.vv[1][lane + 2] = VB << 2;
+        if (lane < 4) { S.vv[0][pad] = 0u; S.vv[1][pad] = 0u; }
+#pragma unroll
+        for (int r = 0; r < 4; ++r) {
+            S.fu[r][lane + 2] = 0u;
+            if (lane < 4) S.fu[r][pad] = 0u;
+        }
     }
     // Player.hold_piece -> create_piece spawn test (player.py:37-44, move_generation.py:112-121): the spawn
     // cell (sx, 17) is validity row 19 = lane 7 of rotation 0
@@ -548,8 +646,9 @@ __device__ __forceinline__ bool search_piece_rows(St& S, const uint16_t* rows, i
     uint32_t a0A = 0u, a0B = 0u;   // arrivals by the in-place kick (0, 0): same lane, never the last kick
     int kick_rounds = 0;           // T: the arrivals of the first two kick rounds are set aside (t_order_decide)
     bool snapped = false;
+    unsigned stat_4 = 0, stat_5 = 0;   // counted with -DTRL_MOVEGEN_STATS only
 #ifdef TRL_MOVEGEN_STATS
-    unsigned stat_2 = 0, stat_3 = 0, stat_4 = 0, stat_5 = 0, stat_6 = 0, stat_7 = 0;
+    unsigned stat_2 = 0, stat_3 = 0, stat_6 = 0;
 #endif
     while (true) {
         TRL_STAT(2);
@@ -568,26 +667,35 @@ __device__ __forceinline__ bool search_piece_rows(St& S, const uint16_t* rows, i
         const uint32_t nA = EA & ~doneA, nB = EB & ~doneB;
         doneA = EA; doneB = EB;
         if (!__any_sync(0xffffffffu, nA | nB)) break;
+        if (SPECIAL && tab == 0) {
+            // the eight passes with a twin as four packed passes, then the four 180-degree passes
+            if (__any_sync(0xffffffffu, nA)) {
+                kick_pass_pair<0, 0>(S, lane, nA, VA, VB, a0A, a0B, is_T, stat_4, stat_5);   // + (2, 2): target 1
+                kick_pass_pair<0, 2>(S, lane, nA, VA, VB, a0A, a0B, is_T, stat_4, stat_5);   // + (2, 0): target 3
+                kick_pass_wall<0, 0, 1>(S, lane, nA & 0xFFFFu, VA, VB, a0A, a0B, is_T, stat_4, stat_5);
+                kick_pass_wall<0, 2, 1>(S, lane, nA >> 16, VA, VB, a0A, a0B, is_T, stat_4, stat_5);
+            }
+            const uint32_t n1 = nB & 0xFFFFu, n3 = nB >> 16;
+            if (__any_sync(0xffffffffu, n1)) {
+                kick_pass_pair<1, 2>(S, lane, n1 | (n1 << 16), VA, VB, a0A, a0B, is_T, stat_4, stat_5);   // + (1, 0): targets 0 | 2
+                kick_pass_wall<0, 1, 1>(S, lane, n1, VA, VB, a0A, a0B, is_T, stat_4, stat_5);
+            }
+            if (__any_sync(0xffffffffu, n3)) {
+                kick_pass_pair<3, 0>(S, lane, n3 | (n3 << 16), VA, VB, a0A, a0B, is_T, stat_4, stat_5);   // + (3, 2): targets 0 | 2
+                kick_pass_wall<0, 3, 1>(S, lane, n3, VA, VB, a0A, a0B, is_T, stat_4, stat_5);
+            }
+        } else {
 #pragma unroll 1
         for (int r = 0; r < 4; ++r) {
-            const uint32_t X = (r & 2) ? nB : nA;
-            const uint32_t ne = (r & 1) ? (X >> 16) : (X & 0xFFFFu);
+            const uint32_t X = (r & 1) ? nB : nA;
+            const uint32_t ne = (r & 2) ? (X >> 16) : (X & 0xFFFFu);
             if (!__any_sync(0xffffffffu, ne)) continue;
-            if (SPECIAL && tab == 0) {
-                switch (r) {
-                    case 0: kick_passes_wall<0, 0>(S, lane, ne, VA, VB, a0A, a0B, is_T); break;
-                    case 1: kick_passes_wall<0, 1>(S, lane, ne, VA, VB, a0A, a0B, is_T); break;
-                    case 2: kick_passes_wall<0, 2>(S, lane, ne, VA, VB, a0A, a0B, is_T); break;
-                    default: kick_passes_wall<0, 3>(S, lane, ne, VA, VB, a0A, a0B, is_T); break;
-                }
-                continue;
-            }
             if (SPECIAL && TRL_ROWS_SPECIAL_I) {
                 switch (r) {
-                    case 0: kick_passes_wall<1, 0>(S, lane, ne, VA, VB, a0A, a0B, false); break;
-                    case 1: kick_passes_wall<1, 1>(S, lane, ne, VA, VB, a0A, a0B, false); break;
-                    case 2: kick_passes_wall<1, 2>(S, lane, ne, VA, VB, a0A, a0B, false); break;
-                    default: kick_passes_wall<1, 3>(S, lane, ne, VA, VB, a0A, a0B, false); break;
+                    case 0: kick_passes_wall<1, 0>(S, lane, ne, VA, VB, a0A, a0B, false, stat_4, stat_5); break;
+                    case 1: kick_passes_wall<1, 1>(S, lane, ne, VA, VB, a0A, a0B, false, stat_4, stat_5); break;
+                    case 2: kick_passes_wall<1, 2>(S, lane, ne, VA, VB, a0A, a0B, false, stat_4, stat_5); break;
+                    default: kick_passes_wall<1, 3>(S, lane, ne, VA, VB, a0A, a0B, false, stat_4, stat_5); break;
                 }
                 continue;
             }
@@ -604,7 +712,7 @@ __device__ __forceinline__ bool search_piece_rows(St& S, const uint16_t* rows, i
                         if (!tt) return;
                         __syncwarp();
                         const uint32_t d = S.fu[nrot][lane + 2];
-                        const uint32_t k0 = (((nrot & 2) ? a0B : a0A) >> (16 * (nrot & 1))) & 0xFFFFu;
+                        const uint32_t k0 = (((nrot & 1) ? a0B : a0A) >> (16 * (nrot >> 1))) & 0xFFFFu;
                         if (round < 8) tt[((round * 4 + nrot) * 3 + kd) * 32 + lane] |= d | k0;
                         S.fu[nrot][lane + 2] = saved | d;
                         a0A |= sA; a0B |= sB;
@@ -613,21 +721,22 @@ __device__ __forceinline__ bool search_piece_rows(St& S, const uint16_t* rows, i
                 } trace_end{S, ttrace, nrot, kd, lane, tround, t_saved, t_a0A, t_a0B, a0A, a0B};
 #endif
                 // kick 0 is (0, 0) in every list (const.py:191-235): target = same cell of the new rotation
-                const uint32_t Vn = ((nrot & 2) ? VB : VA) >> (16 * (nrot & 1));
+                const uint32_t Vn = ((nrot & 1) ? VB : VA) >> (16 * (nrot >> 1));
                 const uint32_t c0 = ne & Vn;
-                const uint32_t c0s = c0 << (16 * (nrot & 1));
-                if (nrot & 2) a0B |= c0s; else a0A |= c0s;
+                const uint32_t c0s = c0 << (16 * (nrot >> 1));
+                if (nrot & 1) a0B |= c0s; else a0A |= c0s;
                 uint32_t rem = ne & ~c0;
                 if (!__any_sync(0xffffffffu, rem)) continue;
                 const TrlKicks& K = c_kicks[tab][r][kd];
                 const int kn = K.n;
-                const uint32_t* vt = &S.vv[nrot][lane + 2];
+                const uint32_t* vt = &S.vv[nrot & 1][lane + 2];
+                const int vsh = 2 + 16 * (nrot >> 1);
                 uint32_t* at = &S.fu[nrot][lane + 2];
 #pragma unroll 1
                 for (int ki = 1; ki < kn; ++ki) {
                     TRL_STAT(5);
                     const int kx = K.k[ki][0], ky = K.k[ki][1];
-                    const uint32_t cand = rem & (vt[-ky] >> (kx + 2));   // source bit ex <-> target bit ex + kx
+                    const uint32_t cand = rem & (vt[-ky] >> (kx + vsh));   // source bit ex <-> target bit ex + kx (TRL_VV)
                     rem &= ~cand;
                     if (cand) {
                         uint32_t arr = (cand << 4) >> (4 - kx);
@@ -637,6 +746,7 @@ __device__ __forceinline__ bool search_piece_rows(St& S, const uint16_t* rows, i
                     if (!__any_sync(0xffffffffu, rem)) break;            // every edge cell has found its kick
                 }
             }
+        }
         }
 #ifdef TRL_T_TRACE
         ++tround;
@@ -648,16 +758,16 @@ __device__ __forceinline__ bool search_piece_rows(St& S, const uint16_t* rows, i
 #ifdef TRL_MOVEGEN_STATS
             if (is_T && stat_2 == 1) {   // mixed flags on a stuck cell after the first round of kicks?
                 const uint32_t stA = VA & ~dA, stB = VB & ~dB;
-                const uint32_t mA = (((f0 | a0A) & (f0 >> 16)) & 0xFFFFu) | ((((f1 << 16) | a0A) & f1) & 0xFFFF0000u);
-                const uint32_t mB = (((f2 | a0B) & (f2 >> 16)) & 0xFFFFu) | ((((f3 << 16) | a0B) & f3) & 0xFFFF0000u);
+                const uint32_t mA = (((f0 | a0A) & (f0 >> 16)) & 0xFFFFu) | ((((f2 << 16) | a0A) & f2) & 0xFFFF0000u);
+                const uint32_t mB = (((f1 | a0B) & (f1 >> 16)) & 0xFFFFu) | ((((f3 << 16) | a0B) & f3) & 0xFFFF0000u);
                 if (__any_sync(0xffffffffu, (mA & stA) | (mB & stB))) stat_6 = 1;
             }
 #endif
-            RA |= a0A | ((f0 | (f0 >> 16)) & 0xFFFFu) | ((f1 | (f1 >> 16)) << 16);
-            RB |= a0B | ((f2 | (f2 >> 16)) & 0xFFFFu) | ((f3 | (f3 >> 16)) << 16);
+            RA |= a0A | ((f0 | (f0 >> 16)) & 0xFFFFu) | ((f2 | (f2 >> 16)) << 16);
+            RB |= a0B | ((f1 | (f1 >> 16)) & 0xFFFFu) | ((f3 | (f3 >> 16)) << 16);
             if (is_T && ++kick_rounds == 2) {   // later rounds accumulate from zero
-                S.tsnap[0][lane] = f0 | (a0A & 0xFFFFu); S.tsnap[1][lane] = f1 | (a0A >> 16);
-                S.tsnap[2][lane] = f2 | (a0B & 0xFFFFu); S.tsnap[3][lane] = f3 | (a0B >> 16);
+                S.tsnap[0][lane] = f0 | (a0A & 0xFFFFu); S.tsnap[1][lane] = f1 | (a0B & 0xFFFFu);
+                S.tsnap[2][lane] = f2 | (a0A >> 16); S.tsnap[3][lane] = f3 | (a0B >> 16);
                 S.fu[0][lane + 2] = 0u; S.fu[1][lane + 2] = 0u; S.fu[2][lane + 2] = 0u; S.fu[3][lane + 2] = 0u;
                 a0A = 0u; a0B = 0u;
                 snapped = true;
@@ -677,8 +787,8 @@ __device__ __forceinline__ bool search_piece_rows(St& S, const uint16_t* rows, i
     const uint32_t placedA = RA & ~dA, placedB = RB & ~dB;
 #ifdef TRL_T_TRACE
     if (ttrace) {
-        ttrace[8 * 4 * 3 * 32 + 0 * 32 + lane] = placedA & 0xFFFFu; ttrace[8 * 4 * 3 * 32 + 1 * 32 + lane] = placedA >> 16;
-        ttrace[8 * 4 * 3 * 32 + 2 * 32 + lane] = placedB & 0xFFFFu; ttrace[8 * 4 * 3 * 32 + 3 * 32 + lane] = placedB >> 16;
+        ttrace[8 * 4 * 3 * 32 + 0 * 32 + lane] = placedA & 0xFFFFu; ttrace[8 * 4 * 3 * 32 + 1 * 32 + lane] = placedB & 0xFFFFu;
+        ttrace[8 * 4 * 3 * 32 + 2 * 32 + lane] = placedA >> 16; ttrace[8 * 4 * 3 * 32 + 3 * 32 + lane] = placedB >> 16;
         ttrace[8 * 4 * 3 * 32 + 4 * 32 + lane] = (uint32_t)rows[lane] | (lane < TRL_ROWS - 32 ? (uint32_t)rows[lane + 32] << 16 : 0u);
     }
 #endif
@@ -688,14 +798,14 @@ __device__ __forceinline__ bool search_piece_rows(St& S, const uint16_t* rows, i
 #pragma unroll
         for (int r = 0; r < 4; ++r) {
             const uint32_t fw = S.fu[r][lane + 2] | (snapped ? S.tsnap[r][lane] : 0u);
-            const uint32_t n = (fw & 0xFFFFu) << (16 * (r & 1)), u = (fw >> 16) << (16 * (r & 1));
-            if (r & 2) { nB |= n; uB |= u; } else { nA |= n; uA |= u; }
+            const uint32_t n = (fw & 0xFFFFu) << (16 * (r >> 1)), u = (fw >> 16) << (16 * (r >> 1));
+            if (r & 1) { nB |= n; uB |= u; } else { nA |= n; uA |= u; }
         }
         flagA = nA | uA; flagB = nB | uB;
         ulkA = uA; ulkB = uB;
         const uint32_t mxA = nA & uA & placedA, mxB = nB & uB & placedB;
-        const uint32_t mixed_rots = (__any_sync(0xffffffffu, mxA & 0xFFFFu) ? 1u : 0u) | (__any_sync(0xffffffffu, mxA >> 16) ? 2u : 0u) |
-                                    (__any_sync(0xffffffffu, mxB & 0xFFFFu) ? 4u : 0u) | (__any_sync(0xffffffffu, mxB >> 16) ? 8u : 0u);
+        const uint32_t mixed_rots = (__any_sync(0xffffffffu, mxA & 0xFFFFu) ? 1u : 0u) | (__any_sync(0xffffffffu, mxB & 0xFFFFu) ? 2u : 0u) |
+                                    (__any_sync(0xffffffffu, mxA >> 16) ? 4u : 0u) | (__any_sync(0xffffffffu, mxB >> 16) ? 8u : 0u);
         if (mixed_rots) {
             // cells with both flag values: the order of emissions decides (:671-677)
             if (!t_order_decide(S, lane, VA, VB, slane, sx + 2, placedA, placedB, a0A, a0B, snapped, mixed_rots, ulkA, ulkB)) return false;
@@ -709,7 +819,7 @@ __device__ __forceinline__ bool search_piece_rows(St& S, const uint16_t* rows, i
         const int n_rot = (type == P_O) ? 1 : 4;
 #pragma unroll 1
         for (int rot = 0; rot < n_rot; ++rot) {
-            const uint32_t placed = (((rot & 2) ? placedB : placedA) >> (16 * (rot & 1))) & 0xFFFFu;
+            const uint32_t placed = (((rot & 1) ? placedB : placedA) >> (16 * (rot >> 1))) & 0xFFFFu;
             if (!placed) continue;
             int row = my - 2;
             uint32_t bits = placed;   // bit mx == policy column x + 2
@@ -720,8 +830,8 @@ __device__ __forceinline__ bool search_piece_rows(St& S, const uint16_t* rows, i
             if (!is_T) {
                 or_chunk(mask, pbase + rot % nrot_planes, row, bits & 0x7FFu);
             } else {
-                const uint32_t f = (((rot & 2) ? flagB : flagA) >> (16 * (rot & 1))) & placed;
-                const uint32_t u = (((rot & 2) ? ulkB : ulkA) >> (16 * (rot & 1))) & 0xFFFFu;
+                const uint32_t f = (((rot & 1) ? flagB : flagA) >> (16 * (rot >> 1))) & placed;
+                const uint32_t u = (((rot & 1) ? ulkB : ulkA) >> (16 * (rot >> 1))) & 0xFFFFu;
                 or_chunk(mask, pbase + rot, row, (placed & ~f) & 0x7FFu);
                 or_chunk(mask, pbase + 4 + rot, row, (f & ~u) & 0x7FFu);
                 or_chunk(mask, pbase + 8 + rot, row, (f & u) & 0x7FFu);
@@ -1344,7 +1454,7 @@ movegen_solo_kernel(const uint16_t* __restrict__ boards, const uint8_t* __restri
 constexpr int kRowsWarps = TRL_ROWS_WARPS;
 
 struct RowsState {
-    uint32_t vv[4][kWinRows];
+    uint32_t vv[2][kWinRows];   // packed validity planes (0 | 2, 1 | 3), TRL_VV
     uint32_t fu[4][kWinRows];
     uint32_t tsnap[4][32];
     uint32_t tp[4][2][36];
@@ -1383,6 +1493,7 @@ movegen_rows_kernel(const uint16_t* __restrict__ boards, const uint8_t* __restri
             const int type = which ? a : c;
             if (type == TRL_NONE || (which && a == c)) continue;
             ok = search_piece_rows<TRL_ROWS_SPECIAL != 0>(S.P, C.rows, hi, type, which != 0, C.mask);
+            if (ok) TRL_REASON(0); else TRL_REASON(1);   // instrumented builds (the clean-up pass sends T straight to the FIFO form)
             __syncwarp();
         }
         if (!ok) {

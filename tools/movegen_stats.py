@@ -1,9 +1,15 @@
+"""Search statistics of the movegen sweep's kernel (needs a build with TRL_NVCC_EXTRA=-DTRL_MOVEGEN_STATS):
+python tools/movegen_stats.py.  Runs the two-pass form, as the sweep does: rounds, fill iterations, (rotation, direction)
+passes and kick tests are those of movegen_rows_kernel's specialised closure search; a pair of twin passes packed into
+one word counts as one pass.  The first line mixes two piece types per call, so it also counts the searches the clean-up
+pass repeats for the other piece of an undecided call; the per-piece lines search one piece per call and count each
+search once."""
 import ctypes, sys, os
 import numpy as np, torch
 sys.path.insert(0, os.getcwd())
 from tetris_reinforcement_learning_b200 import _native, move_generation, synth
 from tetris_reinforcement_learning_b200.const import MASK_WORDS
-L=_native.lib(); L.trl_movegen_warp_form(1)
+L=_native.lib(); L.trl_movegen_warp_form(2)
 dev=torch.device("cuda:0")
 boards,cur,alt=synth.movegen_workload(20000)
 n=boards.shape[0]
