@@ -275,6 +275,12 @@ typedef struct TrlSearchParams {
     uint32_t game_id_stride;           /* new game id = previous id + stride (ranks interleave) */
     int32_t use_random_start;          /* use_random_starting_moves (ai.py:1588-1608)      */
     double random_start_scale;         /* 0.04 * DIRICHLET_S: mean of the exponential number of opening plies */
+    int32_t stop_after_search;         /* != 0: analysis mode.  A finished search always emits its TrlSample (saved
+                                          still reports the playout-cap coin), plays no move, emits no TrlGameEnd,
+                                          leaves games[g] untouched and parks the slot (ctl.active = 0, ctl.iter = 0),
+                                          so every game stops after its own search.  Incompatible with
+                                          use_random_start (TRL_E_ARG). */
+    int32_t pad_;
 } TrlSearchParams;
 
 /* Per-game search control block. */
@@ -322,6 +328,26 @@ typedef struct TrlGameEnd {
     int32_t pieces0, lines_sent0, lines_cleared0, pad_;
 } TrlGameEnd;
 
+#define TRL_PV_MAX 16
+
+/* Root statistics of one finished search (the reference's MCTSTree root, ai.py:237-297), written to the slot of
+ * the search's TrlSample: root_stats[i] belongs to samples[i].  Every value is read before policy-target
+ * pruning, which changes visit counts only. */
+typedef struct TrlRootStats {
+    float root_value;                  /* root value_sum / visits (root.value_avg)                 */
+    uint32_t root_visits;
+    int32_t slot;                      /* game index g of the search in the batch                  */
+    uint16_t n_children;               /* = the sample's n_children                                */
+    uint16_t pv_len;                   /* plies in pv (0..TRL_PV_MAX)                               */
+    uint32_t pv_visits[TRL_PV_MAX];    /* visit count of each ply's node                            */
+    uint16_t pv[TRL_PV_MAX];           /* principal variation as policy indices: from the root, the most visited
+                                          child (last maximum, as the move choice), while it has visits   */
+    float prior[TRL_SAMPLE_MOVES];     /* per root child, sample order: the prior the PUCT used (after the root
+                                          softmax temperature and the Gamma noise mix)              */
+    float q[TRL_SAMPLE_MOVES];         /* value_sum / visits; for an unvisited child the FPU value the
+                                          selection used                                            */
+} TrlRootStats;
+
 /* All device buffers of a search batch; caller-allocated (sizes in elements). */
 typedef struct TrlSearchBuffers {
     int32_t n_games, node_cap, state_cap, moves_cap, sample_cap, end_cap, pad0_, pad1_;
@@ -365,10 +391,13 @@ typedef struct TrlSearchBuffers {
                                                 params2[(game_id ^ side to move at the root) & 1], i.e. network 1
                                                 plays player (game_id & 1) (colours alternate, ai.py:2087-2091);
                                                 the `prm` argument of the calls is then ignored             */
+    TrlRootStats* root_stats;                /* [sample_cap] or NULL (off): a search that writes samples[i] also
+                                                writes root_stats[i]                                         */
 } TrlSearchBuffers;
 
 int trl_sizeof_search_ctl(void);
 int trl_sizeof_sample(void);
+int trl_sizeof_root_stats(void);
 
 /* Step part 1: (start a search if needed,) select a leaf per game and materialise its state;
  * writes leaf_state[g] = index into `states` of the position the net must evaluate, or -1, and

@@ -11,7 +11,7 @@ from .state import GAME_DTYPE, PLAYER_DTYPE
 _SO = os.path.join(os.path.dirname(os.path.abspath(__file__)), "libtrl_b200.so")
 _lib = None
 
-ABI_VERSION = 9
+ABI_VERSION = 10
 
 c_void_p, c_int, c_u64, c_u32 = ctypes.c_void_p, ctypes.c_int, ctypes.c_uint64, ctypes.c_uint32
 
@@ -38,6 +38,7 @@ SIGNATURES = {
     "trl_game_setup_host": (c_int, [c_void_p, c_int, c_u32, c_u32, c_u64]),
     "trl_sizeof_search_ctl": (c_int, []),
     "trl_sizeof_sample": (c_int, []),
+    "trl_sizeof_root_stats": (c_int, []),
     "trl_search_select": (c_int, [c_void_p, c_void_p, c_void_p]),
     "trl_search_movegen": (c_int, [c_void_p, c_void_p]),
     "trl_search_policy_legal": (c_int, [c_void_p, c_void_p, c_int, c_void_p, c_void_p, c_void_p, c_void_p]),
@@ -107,7 +108,7 @@ class SearchParams(ctypes.Structure):
                 ("use_forced", ctypes.c_int32), ("use_tanh", ctypes.c_int32), ("save_all", ctypes.c_int32),
                 ("max_rounds", ctypes.c_int32), ("restart_finished", ctypes.c_int32),
                 ("game_id_stride", ctypes.c_uint32), ("use_random_start", ctypes.c_int32),
-                ("random_start_scale", ctypes.c_double)]
+                ("random_start_scale", ctypes.c_double), ("stop_after_search", ctypes.c_int32), ("pad_", ctypes.c_int32)]
 
 
 class SearchBuffers(ctypes.Structure):
@@ -119,4 +120,5 @@ class SearchBuffers(ctypes.Structure):
                                                "samples", "sample_count", "ends", "end_count",
                                                "next_game_id", "noise_override", "leaf_parent",
                                                "legal_cache", "legal_cache_n", "movegen_index", "path",
-                                               "movegen_list", "movegen_count", "movegen_status", "params2")]
+                                               "movegen_list", "movegen_count", "movegen_status", "params2",
+                                               "root_stats")]

@@ -6,9 +6,12 @@ Kept verbatim from the reference (names, argument meaning, defaults, on-disk art
     make_training_set            ai.py:1809-1845
     self_play_loop               ai.py:2117-2198
     MCTS                         ai.py:299-659    (one search of one reference-style Game)
+    evaluate                     ai.py:1222-1319  (network value + softmax policy of one position)
     search_statistics            ai.py:1330-1361
     reflect_grid/pieces/policy   ai.py:1423-1516
     load_model, load_best_model, highest_model_number, highest_data_number   ai.py:2231-2355
+Beyond the reference: analyse() searches many positions at once with root statistics, evaluate_positions()
+evaluates many positions at once.
 Everything that touches game rules, placements, the search or features runs on the GPU through
 libtrl_b200.so; there is no CPU implementation of those in this package.
 """
@@ -16,6 +19,7 @@ import json
 import math
 import os
 import time
+import weakref
 from datetime import datetime, timezone
 from pathlib import Path
 
@@ -379,16 +383,30 @@ def export_training_set_json(config, set_number, out_path=None):
 
 
 class SearchResult:
-    """What MCTS() returns in place of the reference's MCTSTree: the root children of the search
-    (reference order), their priors and pre-/post-prune visit counts."""
+    """What MCTS() and analyse() return in place of the reference's MCTSTree: the root children of the search
+    (reference order), their pre- and post-prune visit counts, the chosen move and the save flag; with the root
+    statistics (include/trl.h, TrlRootStats) also, per child, the prior the PUCT used (after the root softmax
+    temperature and the Gamma noise mix) and the Q value (value_avg; the FPU value for an unvisited child), the
+    root's value_avg and the principal variation (policy indices, most visited child first)."""
 
-    def __init__(self, sample):
+    def __init__(self, sample, stats=None):
         C = int(sample["n_children"])
         self.moves = sample["moves"][:C].astype(np.int64)
         self.visits = sample["visits"][:C].astype(np.int64)
         self.visits_pre = sample["visits_pre"][:C].astype(np.int64)
         self.iterations = int(sample["iterations"])
         self.state = sample["state"].copy()
+        self.chosen_move = int(sample["chosen_move"])
+        self.move = index_to_move(self.chosen_move)
+        self.saved = bool(sample["saved"])
+        self.priors = self.q = self.root_value = self.pv = self.pv_visits = None
+        if stats is not None:
+            self.priors = stats["prior"][:C].copy()
+            self.q = stats["q"][:C].copy()
+            self.root_value = float(stats["root_value"])
+            L = int(stats["pv_len"])
+            self.pv = stats["pv"][:L].astype(np.int64)
+            self.pv_visits = stats["pv_visits"][:L].astype(np.int64)
 
     def root_children(self):
         return [(index_to_move(m), int(n)) for m, n in zip(self.moves, self.visits)]
@@ -398,50 +416,214 @@ _SEARCH_KEYS = ("MAX_ITER", "CPUCT", "DPUCT", "FpuStrategy", "FpuValue", "use_ro
                 "training", "temperature", "use_playout_cap_randomization", "playout_cap_chance", "playout_cap_mult",
                 "use_dirichlet_noise", "DIRICHLET_ALPHA", "DIRICHLET_S", "DIRICHLET_EXPLORATION", "use_dirichlet_s",
                 "use_forced_playouts_and_policy_target_pruning", "CForcedPlayout", "ruleset", "move_algorithm")
-_mcts_engines = {}   # (network identity + weight versions, search settings, seed) -> one-game engine, reused between calls
+_ANALYSE_MAX_BATCH = 4096   # positions searched concurrently by analyse(); larger inputs run in chunks of this size
+_CACHE_ENTRIES = 4
+# Engines and evaluators are built from a copy of the caller's network and kept between calls.  An entry is
+# (weak reference to the network, value): it serves only the very object it was built for, so a network freed and
+# replaced by another one at the same address (same id, same parameter versions after load_state_dict) misses.
+_search_engines = {}   # (network identity + weight versions, search settings, seed, batch) -> entry
+_evaluators = {}       # network identity + weight versions -> entry of evaluate() / evaluate_positions()
 
 
-def _mcts_engine(config, net, seed):
-    """main.py-style callers search move after move with the same network (reference main.py:80,145): keep the
-    one-game engine (evaluator, packed weights, tree buffers) instead of rebuilding it per call.  The key carries
-    the in-place version counters of the parameters, so a trained / re-loaded network gets a fresh engine."""
+def _net_identity(net):
+    """id plus the in-place version counters of the parameters: a trained / re-loaded network gets a new key."""
     if isinstance(net, torch.nn.Module):
-        ident = (id(net), tuple(int(t._version) for t in list(net.parameters()) + list(net.buffers())))
-    else:
-        ident = (id(net),)
-    key = (ident, tuple(repr(getattr(config, k, None)) for k in _SEARCH_KEYS), seed)
-    eng = _mcts_engines.get(key)
+        return (id(net), tuple(int(t._version) for t in list(net.parameters()) + list(net.buffers())))
+    return (id(net),)
+
+
+def _net_ref(net):
+    try:
+        return weakref.ref(net)
+    except TypeError:           # not weak-referenceable: the entry keeps the object alive, so its id stays its own
+        return lambda: net
+
+
+def _cache_get(cache, key, net):
+    entry = cache.get(key)
+    return entry[1] if entry is not None and entry[0]() is net else None
+
+
+def _cache_put(cache, key, net, value):
+    cache.pop(key, None)
+    while len(cache) >= _CACHE_ENTRIES:
+        cache.pop(next(iter(cache)))
+    cache[key] = (_net_ref(net), value)
+
+
+def release_cached_engines():
+    """Drop the search engines and evaluators that MCTS(), analyse(), evaluate() and evaluate_positions() keep
+    between calls (tree arenas of several GB for thousands of positions) and return their device memory."""
+    _search_engines.clear()
+    _evaluators.clear()
+    if torch.cuda.is_available():
+        torch.cuda.empty_cache()
+
+
+def _search_engine(config, net, seed, n_games):
+    """main.py-style callers search move after move with the same network (reference main.py:80,145): keep the
+    analysis engine (evaluator, packed weights, tree buffers, CUDA graphs) instead of rebuilding it per call."""
+    key = (_net_identity(net), tuple(repr(getattr(config, k, None)) for k in _SEARCH_KEYS), seed, int(n_games))
+    eng = _cache_get(_search_engines, key, net)
     if eng is None:
-        if len(_mcts_engines) >= 4:
-            _mcts_engines.pop(next(iter(_mcts_engines)))
-        eng = _engine_for(config, net, 1, seed=seed, restart_finished=False, save_all=True, use_cuda_graph=False)
-        _mcts_engines[key] = eng
+        _search_engines.pop(key, None)      # a stale entry of a freed network frees its buffers before the new one
+        eng = _engine_for(config, net, n_games, seed=seed, restart_finished=False, analysis=True, root_stats=True)
+        _cache_put(_search_engines, key, net, eng)
     return eng
+
+
+def _engine_batch(n):
+    """Engine size for n positions: the next power of two, at most _ANALYSE_MAX_BATCH (extra slots stay inactive),
+    so that varying input lengths share a few engines."""
+    return min(_ANALYSE_MAX_BATCH, 1 << max(0, n - 1).bit_length())
+
+
+def _pack_positions(games):
+    """A GAME_DTYPE array (copied) or a list of reference-style Game objects -> GAME_DTYPE[n]."""
+    if isinstance(games, np.ndarray) and games.dtype == GAME_DTYPE:
+        return games.reshape(-1).copy()
+    recs = np.zeros(len(games), dtype=GAME_DTYPE)
+    for i, g in enumerate(games):
+        pack_game(g, out=recs[i])
+    return recs
+
+
+def _per_position(x, n, name):
+    a = np.broadcast_to(np.asarray(x, dtype=np.int64), (n,))
+    if (a < 0).any() or (a > 0xFFFFFFFF).any():
+        raise ValueError(f"{name} must hold 32-bit unsigned integers")
+    return a
+
+
+def _analyse_packed(config, recs, network, seed, search_no, strict):
+    """One analysis-mode search per packed position, chunks of _ANALYSE_MAX_BATCH games stepped under CUDA graphs
+    until every game has finished its own search.  -> [SearchResult or None] in input order.  strict: any device
+    status bit raises (MCTS); otherwise a root without a legal move (NO_PIECE, also set for a terminal root) only
+    yields None."""
+    from .selfplay import CTL_DTYPE, EngineStatusError
+    n = len(recs)
+    if n == 0:
+        return []
+    cap = _engine_batch(n)
+    eng = _search_engine(config, network, seed, cap)
+    long_iters, _ = config.playout_iterations()
+    budget = long_iters if (config.training and config.use_playout_cap_randomization) else config.MAX_ITER
+    out = [None] * n
+    for lo in range(0, n, cap):     # cap >= n unless n > _ANALYSE_MAX_BATCH
+        k = min(n, lo + cap) - lo
+        games = np.zeros(cap, dtype=GAME_DTYPE)
+        games[:k] = recs[lo:lo + k]
+        ctl = np.zeros(cap, dtype=CTL_DTYPE)
+        ctl["active"][:k] = 1
+        ctl["search_no"][:k] = search_no[lo:lo + k]
+        eng.drain()
+        eng.set_games(games)
+        eng.set_ctl(ctl)
+        eng.step(budget)      # one simulation per game and step: every search ends within the largest budget
+        if eng.get_ctl()["active"].any():
+            raise EngineStatusError("analysis engine: a search did not finish within its iteration budget")
+        samples, _ = eng.drain()
+        stats = eng.drain_root_stats()
+        eng.check_status(ignore=0 if strict else 0x4)
+        for smp, st in zip(samples, stats):
+            out[lo + int(st["slot"])] = SearchResult(smp, st)
+    return out
+
+
+def analyse(config, games, network, seed=None, game_ids=None, search_no=0):
+    """Search many caller-supplied positions at once on the device: one MCTS search per position with `config`'s
+    settings, all positions in lock-step (the reference runs MCTS once per position, ai.py:299).
+
+    games: a list of reference-style Game objects or a GAME_DTYPE array; they are not modified.
+    game_ids, search_no: scalars or per-position arrays keying the Philox streams of each search (playout-cap coin,
+    Gamma noise, temperature choice, garbage columns) exactly as MCTS()'s game_id / search_no do.  By default a
+    GAME_DTYPE array keeps the game_id of its records and Game objects are numbered 0, 1, ...
+    seed: the Philox key (None: a time-based one, as MCTS).
+    -> one SearchResult per position, in input order; None for a position that is already over or has no legal
+    move at the root (MCTS raises there).  Any other device status raises EngineStatusError."""
+    _require_pytorch(config)
+    recs = _pack_positions(games)
+    n = len(recs)
+    if game_ids is not None:
+        recs["game_id"] = _per_position(game_ids, n, "game_ids")
+    elif not (isinstance(games, np.ndarray) and games.dtype == GAME_DTYPE):
+        recs["game_id"] = np.arange(n)
+    return _analyse_packed(config, recs, network, seed, _per_position(search_no, n, "search_no"), strict=False)
 
 
 def MCTS(config, game, interference_network, seed=None, game_id=0, search_no=0):
     """One search of one reference-style `Game` (ai.py:299): returns (move=(plane, col, row),
     SearchResult, save_bool).  `game` is not mutated.  No random opening plies here, whatever
-    config.use_random_starting_moves says: only play_game draws them (ai.py:1588-1608)."""
-    from .selfplay import CTL_DTYPE
+    config.use_random_starting_moves says: only play_game draws them (ai.py:1588-1608).
+    The one-position case of analyse(); a root without a legal move raises EngineStatusError."""
+    _require_pytorch(config)
     rec = np.zeros(1, dtype=GAME_DTYPE)
     pack_game(game, game_id=game_id, out=rec[0])
-    eng = _mcts_engine(config, interference_network, seed)
-    eng.drain()
-    eng.set_games(rec)
-    ctl = np.zeros(1, dtype=CTL_DTYPE)
-    ctl["active"] = 1
-    ctl["search_no"] = search_no
-    eng.set_ctl(ctl)
-    long_iters, _ = config.playout_iterations()
-    budget = long_iters if (config.training and config.use_playout_cap_randomization) else config.MAX_ITER
-    eng.step(budget)
-    samples, _ = eng.drain()
-    eng.check_status()
-    if not len(samples):
+    res = _analyse_packed(config, rec, interference_network, seed, _per_position(search_no, 1, "search_no"), strict=True)[0]
+    if res is None:
         raise RuntimeError("search produced no result (game already over or no legal move)")
-    s = min(samples, key=lambda r: int(r["search_no"]))
-    return index_to_move(int(s["chosen_move"])), SearchResult(s), bool(s["saved"])
+    return res.move, res, res.saved
+
+
+def _evaluator_for(network):
+    """best_evaluator of a copy of `network` in bf16 (fused trunk + heads where supported), cached per network."""
+    from .selfplay import best_evaluator
+    if callable(network) and not isinstance(network, torch.nn.Module):
+        return network
+    key = _net_identity(network)
+    ev = _cache_get(_evaluators, key, network)
+    if ev is None:
+        import copy
+        _evaluators.pop(key, None)
+        ev = best_evaluator(copy.deepcopy(network).to("cuda"), torch.bfloat16)
+        _cache_put(_evaluators, key, network, ev)
+    return ev
+
+
+def _evaluate_packed(network, recs):
+    """Network outputs for packed positions: trl_encode_features (bf16) on the device, then the network's
+    best_evaluator.  -> (values float32 [n], logits float32 [n, 11583]) on the device."""
+    from . import _native
+    from .const import POLICY_SIZE
+    if not torch.cuda.is_available():
+        raise RuntimeError("evaluate needs a CUDA device: the feature encoder and the network kernels run in "
+                           "libtrl_b200.so (there is no CPU fallback)")
+    dev = torch.device("cuda", torch.cuda.current_device())
+    n = len(recs)
+    d_games = torch.from_numpy(np.ascontiguousarray(recs).view(np.uint8).reshape(-1)).to(dev)
+    grids = torch.empty((2 * n, 1, 40, 10), dtype=torch.bfloat16, device=dev)
+    extras = torch.empty((n, 105), dtype=torch.bfloat16, device=dev)
+    rc = _native.lib().trl_encode_features(d_games.data_ptr(), None, n, grids.data_ptr(), extras.data_ptr(), 1,
+                                           torch.cuda.current_stream(dev).cuda_stream)
+    _native.check(rc, "trl_encode_features")
+    with torch.no_grad():
+        values, logits = _evaluator_for(network)(grids, extras)
+    return values.reshape(-1).float(), logits[:, :POLICY_SIZE].float()
+
+
+def evaluate_positions(config, games, network):
+    """Batched evaluate(): games = a list of reference-style Game objects or a GAME_DTYPE array.
+    -> (values float32 [N], policies float32 [N, 27, 39, 11], each the softmax over all 11583 logits)."""
+    _require_pytorch(config)
+    recs = _pack_positions(games)
+    n = len(recs)
+    values = np.zeros(n, dtype=np.float32)
+    policies = np.zeros((n,) + tuple(POLICY_SHAPE), dtype=np.float32)
+    for lo in range(0, n, _ANALYSE_MAX_BATCH):
+        v, logits = _evaluate_packed(network, recs[lo:lo + _ANALYSE_MAX_BATCH])
+        k = v.shape[0]
+        values[lo:lo + k] = v.cpu().numpy()
+        policies[lo:lo + k] = torch.softmax(logits, dim=1).cpu().numpy().reshape((k,) + tuple(POLICY_SHAPE))
+    return values, policies
+
+
+def evaluate(config, game, network):
+    """The reference's evaluate (ai.py:1222-1319): one position -> (value float, policy float32 ndarray (27,39,11),
+    the softmax over all 11583 logits)."""
+    packed = isinstance(game, (np.ndarray, np.void)) and game.dtype == GAME_DTYPE
+    values, policies = evaluate_positions(config, np.array(game, dtype=GAME_DTYPE).reshape(1) if packed else [game],
+                                          network)
+    return float(values[0]), policies[0]
 
 
 def self_play_loop(config, skip_first_set=False):

@@ -46,7 +46,7 @@ cudaStream_t trl_host_stream(int which) {
 int g_trl_pdl = 1;
 extern "C" void trl_set_pdl(int enabled) { g_trl_pdl = enabled ? 1 : 0; }
 
-extern "C" int trl_abi_version(void) { return 9; }
+extern "C" int trl_abi_version(void) { return 10; }
 extern "C" const char* trl_last_error(void) { return g_err; }
 extern "C" int trl_sizeof_player(void) { return (int)sizeof(TrlPlayer); }
 extern "C" int trl_sizeof_game(void) { return (int)sizeof(TrlGame); }

@@ -27,10 +27,11 @@ constexpr int TRL_PATH_INTS = 64;        // per game: [0] depth, [1..31] nodes, 
 constexpr int TRL_PATH_MAX_DEPTH = 30;
 
 static_assert(sizeof(TrlSearchCtl) == 80, "TrlSearchCtl layout");
-static_assert(sizeof(TrlSearchParams) == 160, "TrlSearchParams layout");
-static_assert(sizeof(TrlSearchBuffers) == 272, "TrlSearchBuffers layout");
+static_assert(sizeof(TrlSearchParams) == 168, "TrlSearchParams layout");
+static_assert(sizeof(TrlSearchBuffers) == 280, "TrlSearchBuffers layout");
 static_assert(sizeof(TrlGameEnd) == 32, "TrlGameEnd layout");
 static_assert(sizeof(TrlSample) == 20 + 400 + 3 * 2 * TRL_SAMPLE_MOVES, "TrlSample layout");
+static_assert(sizeof(TrlRootStats) == 112 + 2 * 4 * TRL_SAMPLE_MOVES, "TrlRootStats layout");
 
 // Phase trace of the per-step kernel (builds with -DTRL_SEARCH_TRACE only; tools/search_trace.py): lane 0 of every
 // game's warp stamps clock64() into g_search_trace[game][phase].
@@ -318,7 +319,47 @@ __device__ __forceinline__ float load_logit(const void* p, size_t row_base, cons
     return load_out(p, row_base + (dtype == 2 ? (size_t)c : (size_t)mv[c]), dtype);
 }
 
-// End of a search (ai.py:571-648) + the per-move bookkeeping of play_game (ai.py:1611-1668).
+// Root statistics of a finished search (include/trl.h, TrlRootStats), read before policy-target pruning.  The
+// children are written lane-parallel like the sample's moves; the principal variation walks down from the root,
+// one warp arg-max per ply with the move choice's rule (most visits, last maximum), while the best child has visits.
+__device__ void write_root_stats(const TrlSearchBuffers& B, TrlRootStats* rs, int g, int lane, size_t nb, size_t sb) {
+    const int C = B.n_children[sb], base = B.first_child[sb];
+    const double fpu_q = B.fpu[sb];   // the root's children keep their initial FPU (the refresh skips the root)
+    for (int c = lane; c < C && c < TRL_SAMPLE_MOVES; c += 32) {
+        const int id = base + c;
+        const int n = B.visits[nb + id];
+        rs->prior[c] = (float)B.prior[nb + id];
+        rs->q[c] = (float)(n > 0 ? B.value_sum[nb + id] / (double)n : fpu_q);
+    }
+    int node = 0, ply = 0;
+    for (; ply < TRL_PV_MAX; ++ply) {
+        const int s = B.slot[nb + node];
+        if (s < 0) break;
+        const int Cn = B.n_children[sb + s], fb = B.first_child[sb + s];
+        if (Cn <= 0) break;
+        double bestn = -1.0; int bi = -1;
+        for (int c = lane; c < Cn; c += 32) {
+            const double n = (double)B.visits[nb + fb + c];
+            if (n >= bestn) { bestn = n; bi = c; }
+        }
+        warp_argmax_last(bestn, bi);
+        if (!(bestn > 0.0)) break;
+        node = fb + bi;
+        if (lane == 0) { rs->pv[ply] = B.move[nb + node]; rs->pv_visits[ply] = (uint32_t)bestn; }
+    }
+    if (lane == 0) {
+        const int rv = B.visits[nb];
+        rs->root_value = (float)(rv > 0 ? B.value_sum[nb] / (double)rv : 0.0);
+        rs->root_visits = (uint32_t)rv;
+        rs->slot = g;
+        rs->n_children = (uint16_t)C;
+        rs->pv_len = (uint16_t)ply;
+        for (int k = ply; k < TRL_PV_MAX; ++k) { rs->pv[k] = 0xFFFF; rs->pv_visits[k] = 0; }
+    }
+}
+
+// End of a search (ai.py:571-648) + the per-move bookkeeping of play_game (ai.py:1611-1668).  Analysis mode
+// (P.stop_after_search): the record only; the real game stays as it is and the slot is parked.
 __device__ void finish_search(const TrlSearchBuffers& B, const TrlSearchParams& P, int g, int lane, TrlGame* sgame) {
     TrlSearchCtl* ctl = &B.ctl[g];
     const size_t nb = (size_t)g * B.node_cap, sb = (size_t)g * B.state_cap;
@@ -381,7 +422,7 @@ __device__ void finish_search(const TrlSearchBuffers& B, const TrlSearchParams& 
         chosen = __shfl_sync(kFull, chosen, 0);
 
         const bool save = !ctl->fast;
-        const bool want_rec = (save || P.save_all) && !random_ply;
+        const bool want_rec = (save || P.save_all || P.stop_after_search) && !random_ply;
         uint32_t slot_i = 0;
         if (want_rec) {
             if (lane == 0) slot_i = atomicAdd(B.sample_count, 1u);
@@ -394,6 +435,7 @@ __device__ void finish_search(const TrlSearchBuffers& B, const TrlSearchParams& 
                 rec->moves[c] = B.move[nb + base + c];
                 rec->visits_pre[c] = (uint16_t)B.visits[nb + base + c];
             }
+        if (rec && B.root_stats) write_root_stats(B, &B.root_stats[slot_i], g, lane, nb, sb);
 
         // policy-target pruning (ai.py:619-648): mutates root-children visit counts
         if (P.use_forced && P.training && !ctl->fast) {
@@ -437,6 +479,16 @@ __device__ void finish_search(const TrlSearchBuffers& B, const TrlSearchParams& 
                 rec->total_visits = tot; rec->iterations = ctl->max_iter;
             }
         }
+    }
+
+    if (P.stop_after_search) {
+        if (lane == 0) {
+            if (C <= 0) ctl->status |= TRL_ST_NO_PIECE;   // terminal root or no legal move: no record
+            ctl->iter = 0;
+            ctl->active = 0;
+        }
+        __syncwarp();
+        return;
     }
 
     // ---- play the move on the real game (ai.py:1668: game.make_move(move)) ----
@@ -832,6 +884,10 @@ extern "C" int trl_debug_search_trace(long long* device_buffer) {
 
 extern "C" int trl_sizeof_search_ctl(void) { return (int)sizeof(TrlSearchCtl); }
 extern "C" int trl_sizeof_sample(void) { return (int)sizeof(TrlSample); }
+extern "C" int trl_sizeof_root_stats(void) { return (int)sizeof(TrlRootStats); }
+
+// analysis mode stops every game after its first search: random opening plies would never be followed by one
+static bool params_ok(const TrlSearchParams* p) { return p && !(p->stop_after_search && p->use_random_start); }
 
 static bool buffers_ok(const TrlSearchBuffers* b) {
     return b && b->n_games >= 0 && b->node_cap > 1 && b->state_cap > 1 && b->moves_cap > 0 && b->prior && b->value_sum &&
@@ -848,7 +904,7 @@ static bool logits_ok(const TrlSearchBuffers* b, int stride, int dtype) {
 }
 
 extern "C" int trl_search_select(const TrlSearchBuffers* buf, const TrlSearchParams* prm, void* stream) {
-    if (!buffers_ok(buf) || !prm) return TRL_E_ARG;
+    if (!buffers_ok(buf) || !params_ok(prm)) return TRL_E_ARG;
     if (buf->n_games == 0) return TRL_OK;
     const dim3 grid((buf->n_games + kWarps - 1) / kWarps);
     if (buf->params2) search_select_kernel<true><<<grid, kWarps * 32, 0, (cudaStream_t)stream>>>(*buf, *prm);
@@ -873,7 +929,7 @@ extern "C" int trl_search_movegen(const TrlSearchBuffers* buf, void* stream) {
 
 extern "C" int trl_search_expand(const TrlSearchBuffers* buf, const TrlSearchParams* prm, const void* values,
                                  const void* logits, int logits_stride, int dtype, void* stream) {
-    if (!buffers_ok(buf) || !prm || !values || !logits || !logits_ok(buf, logits_stride, dtype))
+    if (!buffers_ok(buf) || !params_ok(prm) || !values || !logits || !logits_ok(buf, logits_stride, dtype))
         return TRL_E_ARG;
     if (buf->n_games == 0) return TRL_OK;
     const dim3 grid((buf->n_games + kWarps - 1) / kWarps);
@@ -884,7 +940,7 @@ extern "C" int trl_search_expand(const TrlSearchBuffers* buf, const TrlSearchPar
 
 extern "C" int trl_search_expand_select(const TrlSearchBuffers* buf, const TrlSearchParams* prm, const void* values,
                                         const void* logits, int logits_stride, int dtype, void* stream) {
-    if (!buffers_ok(buf) || !prm || !values || !logits || !logits_ok(buf, logits_stride, dtype))
+    if (!buffers_ok(buf) || !params_ok(prm) || !values || !logits || !logits_ok(buf, logits_stride, dtype))
         return TRL_E_ARG;
     if (buf->n_games == 0) return TRL_OK;
     return trl_launch_ex(buf->params2 ? search_expand_select_kernel<true> : search_expand_select_kernel<false>,
@@ -897,7 +953,7 @@ extern "C" int trl_search_expand_select_encode(const TrlSearchBuffers* buf, cons
                                                void* images_bf16, int32_t* image_dest, int32_t* n_images,
                                                void* extras_bf16, int32_t* own_row, int32_t* opp_row, int32_t* row_of,
                                                void* stream) {
-    if (!buffers_ok(buf) || !prm || !values || !logits || !logits_ok(buf, logits_stride, dtype) ||
+    if (!buffers_ok(buf) || !params_ok(prm) || !values || !logits || !logits_ok(buf, logits_stride, dtype) ||
         !buf->leaf_parent || !cache_bf16 || !images_bf16 || !image_dest || !n_images || !extras_bf16 || !own_row || !opp_row ||
         !row_of)
         return TRL_E_ARG;

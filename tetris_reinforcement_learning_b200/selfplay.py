@@ -46,6 +46,17 @@ SAMPLE_DTYPE = np.dtype({
     "itemsize": 420 + 6 * SAMPLE_MOVES,
 })
 
+PV_MAX = 16
+
+# TrlRootStats (include/trl.h): root statistics of one search, at the slot index of its TrlSample
+ROOT_STATS_DTYPE = np.dtype({
+    "names": ["root_value", "root_visits", "slot", "n_children", "pv_len", "pv_visits", "pv", "prior", "q"],
+    "formats": ["<f4", "<u4", "<i4", "<u2", "<u2", ("<u4", (PV_MAX,)), ("<u2", (PV_MAX,)),
+                ("<f4", (SAMPLE_MOVES,)), ("<f4", (SAMPLE_MOVES,))],
+    "offsets": [0, 4, 8, 12, 14, 16, 80, 112, 112 + 4 * SAMPLE_MOVES],
+    "itemsize": 112 + 8 * SAMPLE_MOVES,
+})
+
 GAME_END_DTYPE = np.dtype({
     "names": ["game_id", "winner", "plies", "rounds", "pieces0", "lines_sent0", "lines_cleared0", "pad_"],
     "formats": ["<u4", "<i4", "<u4", "<u4", "<i4", "<i4", "<i4", "<i4"],
@@ -67,9 +78,10 @@ class EngineStatusError(RuntimeError):
 
 
 def search_params_from_config(config, seed=0, restart_finished=True, game_id_stride=1, save_all=None, max_rounds=None,
-                              random_openings=False):
+                              random_openings=False, analysis=False):
     """Config (ai.py:97-137) -> TrlSearchParams.  random_openings: only play_game draws random opening plies
-    (ai.py:1588-1608); MCTS() and battle_networks never do, whatever config.use_random_starting_moves says."""
+    (ai.py:1588-1608); MCTS() and battle_networks never do, whatever config.use_random_starting_moves says.
+    analysis: every game stops after its own search (TrlSearchParams.stop_after_search)."""
     from .const import MAX_MOVES
     p = _native.SearchParams()
     p.seed = int(seed)
@@ -99,6 +111,9 @@ def search_params_from_config(config, seed=0, restart_finished=True, game_id_str
     # random opening plies sampled from the raw policy (ai.py:1588-1608); scale = 0.04 * DIRICHLET_S
     p.use_random_start = int(bool(random_openings) and bool(getattr(config, "use_random_starting_moves", False)))
     p.random_start_scale = 0.04 * float(config.DIRICHLET_S)
+    p.stop_after_search = int(bool(analysis))
+    if p.stop_after_search and p.use_random_start:
+        raise ValueError("analysis mode searches the given positions only: random opening plies cannot run in it")
     return p
 
 
@@ -108,13 +123,19 @@ class SelfPlayEngine:
     evaluator(grids [2G,1,40,10], extras [G,105]) -> (values [G] or [G,1], logits [G,11583]);
     tensors of `feature_dtype` in, float32 or bfloat16 out.  Normally a network's
     `forward_packed` (see make_net_evaluator); tests inject a deterministic function.
+
+    analysis=True: analysis mode (include/trl.h, TrlSearchParams.stop_after_search): each game runs one search
+    of the position it holds, emits its sample and goes inactive; the games are left as they were.
+    root_stats=True: every sample also gets a TrlRootStats record (priors, Q values, root value, principal
+    variation), read with drain_root_stats() after drain().
     """
 
     def __init__(self, config, evaluator, n_games, device="cuda:0", seed=0, first_game_id=0, game_id_stride=1,
                  feature_dtype=torch.float32, node_cap=None, sample_cap=None, restart_finished=True, save_all=None,
                  max_rounds=None, use_cuda_graph=True, overlap_movegen=True, reuse_trunk_features=True,
                  reuse_sibling_placements=True, compact_movegen=True, fuse_expand_select=True, fuse_encode=True,
-                 steps_per_graph=4, parallel_backup=True, random_openings=False, gather_policy=True):
+                 steps_per_graph=4, parallel_backup=True, random_openings=False, gather_policy=True, analysis=False,
+                 root_stats=False):
         from .state import ruleset_id
         self.ruleset = ruleset_id(config.ruleset)   # 's2' (default) or 's1': attack table + all-spin rule
         if config.move_algorithm != "convolutional":
@@ -124,7 +145,8 @@ class SelfPlayEngine:
         self.G = int(n_games)
         self.device = torch.device(device)
         self.params = search_params_from_config(config, seed, restart_finished, game_id_stride, save_all, max_rounds,
-                                                random_openings)
+                                                random_openings, analysis)
+        self.analysis = bool(analysis)
         self.seed = int(seed)
         self.feature_dtype = feature_dtype
         self.use_cuda_graph = use_cuda_graph
@@ -154,6 +176,10 @@ class SelfPlayEngine:
             "next_game_id": z(1, torch.int32), "leaf_parent": z(G, torch.int32), "path": z(G * 64, torch.int32),
             "movegen_status": z(G, torch.int32),
         }
+        self.root_stats = bool(root_stats)
+        if self.root_stats:
+            self.t["root_stats"] = z(self.sample_cap * ROOT_STATS_DTYPE.itemsize, torch.uint8)
+        self._last_root_stats = np.zeros(0, ROOT_STATS_DTYPE)
         # exact reuse of legal-placement lists between siblings (include/trl.h, TrlSearchBuffers.legal_cache)
         self.reuse_sibling_placements = bool(reuse_sibling_placements)
         if self.reuse_sibling_placements:
@@ -189,6 +215,7 @@ class SelfPlayEngine:
         self.gather_policy = bool(gather_policy) and self.cached_eval is not None and getattr(self.cached_eval, "gather_policy", False)
         self._cache_bufs = self.cached_eval.make_buffers(ns, G, dev, self.moves_cap) if self.cached_eval is not None else None
         assert self.lib.trl_sizeof_search_ctl() == CTL_DTYPE.itemsize and self.lib.trl_sizeof_sample() == SAMPLE_DTYPE.itemsize
+        assert self.lib.trl_sizeof_root_stats() == ROOT_STATS_DTYPE.itemsize
         self._pinned, self._pinned_i = None, 0      # host staging of drain()
         self._graph = None
         self._graph_k = None                        # steps_per_graph consecutive steps as ONE graph launch
@@ -431,12 +458,19 @@ class SelfPlayEngine:
         nsb, neb = ns * SAMPLE_DTYPE.itemsize, ne * GAME_END_DTYPE.itemsize
         hs[:nsb].copy_(self.t["samples"][:nsb], non_blocking=True)
         he[:neb].copy_(self.t["ends"][:neb], non_blocking=True)
+        if self.root_stats:
+            self._last_root_stats = self.t["root_stats"][:ns * ROOT_STATS_DTYPE.itemsize].cpu().numpy().view(ROOT_STATS_DTYPE).copy()
         self.t["sample_count"].zero_()
         self.t["end_count"].zero_()
         torch.cuda.synchronize(self.device)
         samples = hs[:nsb].numpy().view(SAMPLE_DTYPE)
         ends = he[:neb].numpy().view(GAME_END_DTYPE)
         return (samples.copy(), ends.copy()) if copy else (samples, ends)
+
+    def drain_root_stats(self):
+        """-> ROOT_STATS_DTYPE[k]: the root statistics of the k samples the last drain() returned, in the same order
+        (record i belongs to sample i).  Empty unless the engine was built with root_stats=True."""
+        return self._last_root_stats
 
     def status_bits(self):
         """OR of the sticky TRL_ST_* bits of all games (0 = clean)."""

@@ -130,6 +130,24 @@ def pack_game(game, game_id=0, rng_ctr=0, bag_ctr=0, out=None):
     return rec
 
 
+def unpack_game(rec):
+    """GAME_DTYPE scalar -> a duck-typed reference Game (game.py:6-26, player.py:10-27) carrying exactly the fields
+    pack_game reads, e.g. to hand stored positions to MCTS().  pack_game(unpack_game(r)) == r except for the history
+    length and the RNG counters, which a Game does not carry."""
+    from types import SimpleNamespace as NS
+    players = []
+    for pr in rec["players"]:
+        players.append(NS(board=NS(grid=rows_to_grid(pr["rows"])),
+                          queue=NS(pieces=[MINOS[int(v)] for v in pr["queue"][:int(pr["qlen"])]]),
+                          piece=None if int(pr["piece"]) == NONE else NS(type=MINOS[int(pr["piece"])]),
+                          held_piece=piece_name(pr["held"]), game_over=bool(pr["game_over"]),
+                          garbage_to_receive=[int(v) for v in pr["recv"][:int(pr["n_recv"])]],
+                          stats=NS(pieces=int(pr["pieces"]), b2b=int(pr["b2b"]), combo=int(pr["combo"]),
+                                   b2b_level=int(pr["b2b_level"]))))
+    ruleset = {v: k for k, v in RULESETS.items()}[int(rec["ruleset"])]
+    return NS(players=players, turn=int(rec["turn"]), ruleset=ruleset)
+
+
 def player_state_dict(rec):
     """PLAYER_DTYPE scalar -> plain dict in the reference's vocabulary (for diffs / debugging)."""
     return {
