@@ -184,9 +184,10 @@ void trl_movegen_select_kernel(int kernel);
 
 /* Form of the warp-cooperative enumeration (csrc/movegen_warp.cu): 0 = two warps per call, one per piece
  * type (lowest latency: the few-thousand-call batches of a self-play step), 1 = one warp per call,
- * both piece searches back to back, 2 = two passes: a small kernel with the row-parallel closure search
- * alone, then the exact FIFO search for the calls it could not decide (highest throughput: the
- * multi-million-call sweeps of move_generation.py:752-789), -1 = by batch size (default).
+ * both piece searches back to back, 2 = passes: a small kernel with the row-parallel closure search
+ * alone, then the T order analysis and the exact T search for the T searches it deferred, and one warp per call
+ * for the few calls it could not handle (highest throughput: the multi-million-call sweeps of
+ * move_generation.py:752-789), -1 = by batch size (default).
  * Bit-identical outputs. */
 void trl_movegen_warp_form(int form);
 

@@ -31,9 +31,11 @@
 //       is applied with shared-memory atomics, the mixed case serially in reference order.
 //
 //   movegen_warp_kernel   two warps per call, one per piece type (latency form: self-play batches);
-//   movegen_solo_kernel   one warp per call; also the clean-up pass of the two-pass form;
-//   movegen_rows_kernel   the closure search alone, undecided calls appended to a list (throughput form: the
-//                         multi-million-call sweep); movegen_list_kernel is the enumeration inside a self-play step.
+//   movegen_solo_kernel   one warp per call; also the legacy route of the pass form;
+//   movegen_rows_kernel   the closure search alone, deferred T searches and undecided calls appended to lists, then
+//                         movegen_t_order_kernel and movegen_t_exact_kernel for the deferred T searches (the pass
+//                         form, for throughput: the multi-million-call sweep); movegen_list_kernel is the enumeration
+//                         inside a self-play step.
 // In every form the answer placed = visited & ~valid[row+1] is OR-ed into a per-call bit mask in shared
 // memory, written out coalesced, and turned into the ascending move list (= np.argwhere order).
 #include <cuda_runtime.h>
@@ -552,8 +554,11 @@ __device__ __forceinline__ void validity_rows(const uint32_t (&e)[4], uint32_t (
     v[3] = validity_row<TYPE, 3>(e);
 }
 
-// SPECIAL: kick passes of the non-I pieces with compile-time tables, twin passes packed (the closure kernel).
-template <bool SPECIAL, class St>
+// SPECIAL: kick passes of the non-I pieces with compile-time tables, twin passes packed (the closure kernels).
+// T_ORDER: a T search with mixed flags goes through t_order_decide (St needs tsnap and tp).  Without it the search
+// keeps no snapshot of the first two kick rounds and returns false ("deferred") for every T search with mixed flags:
+// the sweep's first pass, which leaves the order analysis to a kernel of its own.
+template <bool SPECIAL, bool T_ORDER, class St>
 __device__ __forceinline__ bool search_piece_rows(St& S, const uint16_t* rows, int hi, int type, bool via_hold, uint32_t* mask) {
     const int lane = threadIdx.x & 31;
     const int sx = trl_spawn_x(type);
@@ -765,13 +770,15 @@ __device__ __forceinline__ bool search_piece_rows(St& S, const uint16_t* rows, i
 #endif
             RA |= a0A | ((f0 | (f0 >> 16)) & 0xFFFFu) | ((f2 | (f2 >> 16)) << 16);
             RB |= a0B | ((f1 | (f1 >> 16)) & 0xFFFFu) | ((f3 | (f3 >> 16)) << 16);
-            if (is_T && ++kick_rounds == 2) {   // later rounds accumulate from zero
-                S.tsnap[0][lane] = f0 | (a0A & 0xFFFFu); S.tsnap[1][lane] = f1 | (a0B & 0xFFFFu);
-                S.tsnap[2][lane] = f2 | (a0A >> 16); S.tsnap[3][lane] = f3 | (a0B >> 16);
-                S.fu[0][lane + 2] = 0u; S.fu[1][lane + 2] = 0u; S.fu[2][lane + 2] = 0u; S.fu[3][lane + 2] = 0u;
-                a0A = 0u; a0B = 0u;
-                snapped = true;
-                __syncwarp();
+            if constexpr (T_ORDER) {
+                if (is_T && ++kick_rounds == 2) {   // later rounds accumulate from zero
+                    S.tsnap[0][lane] = f0 | (a0A & 0xFFFFu); S.tsnap[1][lane] = f1 | (a0B & 0xFFFFu);
+                    S.tsnap[2][lane] = f2 | (a0A >> 16); S.tsnap[3][lane] = f3 | (a0B >> 16);
+                    S.fu[0][lane + 2] = 0u; S.fu[1][lane + 2] = 0u; S.fu[2][lane + 2] = 0u; S.fu[3][lane + 2] = 0u;
+                    a0A = 0u; a0B = 0u;
+                    snapped = true;
+                    __syncwarp();
+                }
             }
         }
     }
@@ -797,7 +804,8 @@ __device__ __forceinline__ bool search_piece_rows(St& S, const uint16_t* rows, i
         uint32_t nA = a0A, nB = a0B, uA = 0u, uB = 0u;
 #pragma unroll
         for (int r = 0; r < 4; ++r) {
-            const uint32_t fw = S.fu[r][lane + 2] | (snapped ? S.tsnap[r][lane] : 0u);
+            uint32_t fw = S.fu[r][lane + 2];
+            if constexpr (T_ORDER) fw |= snapped ? S.tsnap[r][lane] : 0u;
             const uint32_t n = (fw & 0xFFFFu) << (16 * (r >> 1)), u = (fw >> 16) << (16 * (r >> 1));
             if (r & 1) { nB |= n; uB |= u; } else { nA |= n; uA |= u; }
         }
@@ -808,7 +816,8 @@ __device__ __forceinline__ bool search_piece_rows(St& S, const uint16_t* rows, i
                                     (__any_sync(0xffffffffu, mxA >> 16) ? 4u : 0u) | (__any_sync(0xffffffffu, mxB >> 16) ? 8u : 0u);
         if (mixed_rots) {
             // cells with both flag values: the order of emissions decides (:671-677)
-            if (!t_order_decide(S, lane, VA, VB, slane, sx + 2, placedA, placedB, a0A, a0B, snapped, mixed_rots, ulkA, ulkB)) return false;
+            if constexpr (!T_ORDER) return false;
+            else if (!t_order_decide(S, lane, VA, VB, slane, sx + 2, placedA, placedB, a0A, a0B, snapped, mixed_rots, ulkA, ulkB)) return false;
         }
     }
     // ---- _convert_placements_to_policy (move_generation.py:650-749): lane = row ----
@@ -843,12 +852,12 @@ __device__ __forceinline__ bool search_piece_rows(St& S, const uint16_t* rows, i
 
 // out-of-line copy for the kernels that also carry the FIFO form
 __device__ __noinline__ bool search_piece_rows_call(PieceState& S, const uint16_t* rows, int type, bool via_hold, uint32_t* mask) {
-    return search_piece_rows<false>(S, rows, first_block_row(rows, threadIdx.x & 31), type, via_hold, mask);
+    return search_piece_rows<false, true>(S, rows, first_block_row(rows, threadIdx.x & 31), type, via_hold, mask);
 }
 
-// One piece type of one call, executed by one converged warp.
-__device__ __noinline__ void search_piece_fifo(PieceState& S, const uint16_t* rows, int type, bool via_hold, uint32_t* mask,
-                                  uint32_t& status, const uint32_t (*kpack)[4][3][2]) {
+// One piece type of one call, executed by one converged warp.  Inlined with a constant `type` by the exact T kernel.
+__device__ __forceinline__ void search_piece_fifo_body(PieceState& S, const uint16_t* rows, int type, bool via_hold, uint32_t* mask,
+                                                       uint32_t& status, const uint32_t (*kpack)[4][3][2]) {
     const int lane = threadIdx.x & 31;
     uint32_t minos[4];
 #pragma unroll
@@ -1155,6 +1164,11 @@ __device__ __noinline__ void search_piece_fifo(PieceState& S, const uint16_t* ro
     }
 }
 
+__device__ __noinline__ void search_piece_fifo(PieceState& S, const uint16_t* rows, int type, bool via_hold, uint32_t* mask,
+                                              uint32_t& status, const uint32_t (*kpack)[4][3][2]) {
+    search_piece_fifo_body(S, rows, type, via_hold, mask, status, kpack);
+}
+
 // One piece type of one call: the row-parallel closure form, or the exact FIFO form where that one cannot decide.
 __device__ __forceinline__ void search_piece_warp(PieceState& S, const uint16_t* rows, int type, bool via_hold, uint32_t* mask,
                                                   uint32_t& status, const uint32_t (*kpack)[4][3][2], bool exact_only = false) {
@@ -1383,7 +1397,7 @@ movegen_solo_kernel(const uint16_t* __restrict__ boards, const uint8_t* __restri
                     uint16_t* __restrict__ moves, int moves_cap, uint16_t* __restrict__ n_moves,
                     uint32_t* __restrict__ status, uint16_t* __restrict__ compact, unsigned long long compact_cap,
                     unsigned long long* __restrict__ compact_total, unsigned long long* __restrict__ offsets,
-                    // clean-up mode (second pass of the two-pass form): only the calls call_list[0 .. *call_count),
+                    // clean-up mode (the legacy route of the pass form): only the calls call_list[0 .. *call_count),
                     // T searches straight through the exact FIFO form, a fixed grid striding over the list
                     const int32_t* __restrict__ call_list, const uint32_t* __restrict__ call_count) {
     extern __shared__ __align__(16) uint8_t smem_raw[];
@@ -1432,15 +1446,25 @@ movegen_solo_kernel(const uint16_t* __restrict__ boards, const uint8_t* __restri
 }
 
 // ---------------------------------------------------------------------------------------
-// Throughput form, two passes: the row-parallel closure search alone in a small kernel, then the exact
-// FIFO search for the few calls it could not decide.
+// Throughput form, in passes: the row-parallel closure search alone in a small kernel, then the T order analysis
+// and the exact T search for the few calls whose T search it deferred.
 //
-// movegen_rows_kernel carries no FIFO code: 48 registers instead of 64 (40 resident warps per SM instead
-// of 32), 2.8 KB of shared memory per warp, and a loop nest small enough to stay in the instruction caches
-// (the one-kernel forms lose a quarter of their issue slots to instruction fetch).  A call one of whose
-// piece searches returns "undecided" (mixed T-spin flags on a cell, or a climb out of the row window) is
-// appended to a list and produces no output here; movegen_solo_kernel in clean-up mode then handles
-// exactly those calls (T searches straight through the FIFO form).
+//   pass 1  movegen_rows_kernel: both piece searches through the closure form without the T order analysis
+//           (T_ORDER = false): 48 registers, no FIFO code, no cold analysis code, a loop nest small enough to stay
+//           in the instruction caches (the one-kernel forms lose a quarter of their issue slots to instruction
+//           fetch).  A T search with mixed flags, or one that climbed out of the row window, is DEFERRED: the other
+//           piece is still searched, the call's partial mask (the other piece's bits only) is stored and the call
+//           appended to the deferred list;
+//   pass 2  movegen_t_order_kernel: the T search alone, closure form with the order analysis (t_order_decide).
+//           Decided: merged into the partial mask, outputs written.  Undecided: appended to the exact list;
+//   pass 3  movegen_t_exact_kernel: the exact FIFO search specialised for T (piece and kick table fixed at compile
+//           time; no closure form, no other piece), merged into the partial mask, outputs written;
+//   legacy  movegen_solo_kernel in clean-up mode: calls whose NON-T search is undecided (a climb out of the row
+//           window) or whose partial mask found no room redo the whole call as before (T straight through the FIFO
+//           form).  It is launched every sweep and exits at once when its list is empty.
+// Only the pass that finishes a call writes n_moves, status and the move list.  The partial mask lives in the call's
+// own mask_bits row when there is a mask output, otherwise in a bounded scratch (PassLists.partial).
+// Passes 2 and 3 hand out their work through ticket counters (the counts exist only on the device).
 // ---------------------------------------------------------------------------------------
 #ifndef TRL_ROWS_SPECIAL
 #define TRL_ROWS_SPECIAL 1
@@ -1452,18 +1476,50 @@ movegen_solo_kernel(const uint16_t* __restrict__ boards, const uint8_t* __restri
 #define TRL_ROWS_MIN_BLOCKS 10
 #endif
 constexpr int kRowsWarps = TRL_ROWS_WARPS;
+constexpr int kTWarps = 4;   // warps per block of passes 2 and 3
+
+// pass bookkeeping in the per-stream scratch: counters, then the lists
+enum : int { kCntLegacy = 0, kCntDeferred = 1, kCntExact = 2, kTicketOrder = 3, kTicketExact = 4, kCounters = 16 };
+struct PassLists {
+    uint32_t* counts;     // [kCounters], zeroed before pass 1
+    int32_t* legacy;      // call indices for movegen_solo_kernel in clean-up mode
+    int32_t* deferred;    // call indices whose T search pass 1 deferred; position j = partial-mask slot j
+    int32_t* exact;       // positions j of the deferred list that pass 2 left undecided
+    uint32_t* partial;    // nullptr: partial masks in mask_bits; else [deferred_cap][TRL_MASK_WORDS]
+    unsigned deferred_cap;
+};
 
 struct RowsState {
     uint32_t vv[2][kWinRows];   // packed validity planes (0 | 2, 1 | 3), TRL_VV
     uint32_t fu[4][kWinRows];
-    uint32_t tsnap[4][32];
-    uint32_t tp[4][2][36];
 };
 
 struct RowsWarp {
     RowsState P;
     CallState C;
 };
+
+// The call's mask row to / from global memory, coalesced (words TRL_MASK_WORDS.. stay zero).
+__device__ __forceinline__ void store_mask(const CallState& C, uint32_t* __restrict__ g, int lane) {
+#pragma unroll 1
+    for (int w = lane; w < TRL_MASK_WORDS; w += 32) g[w] = C.mask[w];
+}
+
+__device__ __forceinline__ void load_mask(CallState& C, const uint32_t* __restrict__ g, int lane) {
+#pragma unroll 1
+    for (int w = lane; w < TRL_MASK_WORDS + 2; w += 32) C.mask[w] = w < TRL_MASK_WORDS ? g[w] : 0u;
+}
+
+__device__ __forceinline__ uint32_t* partial_mask(const PassLists& pl, uint32_t* mask_bits, int i, unsigned j) {
+    return pl.partial ? pl.partial + (size_t)j * TRL_MASK_WORDS : mask_bits + (size_t)i * TRL_MASK_WORDS;
+}
+
+// the next item of a pass-2 / pass-3 list for this warp: a ticket (a warp that drew short searches takes more)
+__device__ __forceinline__ unsigned next_item(uint32_t* ticket, int lane) {
+    unsigned j = 0;
+    if (lane == 0) j = atomicAdd(ticket, 1u);
+    return __shfl_sync(0xffffffffu, j, 0);
+}
 
 template <bool WANT_LIST>   // two instantiations: every instruction less in this kernel is instruction-cache room
 __global__ void __launch_bounds__(kRowsWarps * 32, TRL_ROWS_MIN_BLOCKS)
@@ -1473,7 +1529,7 @@ movegen_rows_kernel(const uint16_t* __restrict__ boards, const uint8_t* __restri
                     uint16_t* __restrict__ moves, int moves_cap, uint16_t* __restrict__ n_moves,
                     uint32_t* __restrict__ status, uint16_t* __restrict__ compact, unsigned long long compact_cap,
                     unsigned long long* __restrict__ compact_total, unsigned long long* __restrict__ offsets,
-                    int32_t* __restrict__ undecided, uint32_t* __restrict__ undecided_count) {
+                    const PassLists pl) {
     extern __shared__ __align__(16) uint8_t smem_raw[];
     const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
     RowsWarp& S = reinterpret_cast<RowsWarp*>(smem_raw)[warp];
@@ -1486,22 +1542,132 @@ movegen_rows_kernel(const uint16_t* __restrict__ boards, const uint8_t* __restri
     __syncwarp();
     if (!skip) {
         const int hi = first_block_row(C.rows, lane);
-        bool ok = true;
+        bool legacy = false, t_deferred = false;
         // the current piece, then the hold-or-next piece (de-duplicated, move_generation.py:103-105)
 #pragma unroll 1
-        for (int which = 0; which < 2 && ok; ++which) {
+        for (int which = 0; which < 2 && !legacy; ++which) {
             const int type = which ? a : c;
             if (type == TRL_NONE || (which && a == c)) continue;
-            ok = search_piece_rows<TRL_ROWS_SPECIAL != 0>(S.P, C.rows, hi, type, which != 0, C.mask);
-            if (ok) TRL_REASON(0); else TRL_REASON(1);   // instrumented builds (the clean-up pass sends T straight to the FIFO form)
+            const bool ok = search_piece_rows<TRL_ROWS_SPECIAL != 0, false>(S.P, C.rows, hi, type, which != 0, C.mask);
+            if (ok) TRL_REASON(0); else TRL_REASON(1);   // instrumented builds
             __syncwarp();
+            if (!ok) {
+                if (type == P_T) t_deferred = true;
+                else legacy = true;
+            }
         }
-        if (!ok) {
-            if (lane == 0) undecided[atomicAdd(undecided_count, 1u)] = i;
+        if (t_deferred && !legacy) {
+            unsigned j = 0;
+            if (lane == 0) j = atomicAdd(&pl.counts[kCntDeferred], 1u);
+            j = __shfl_sync(0xffffffffu, j, 0);
+            if (j < pl.deferred_cap) {
+                store_mask(C, partial_mask(pl, mask_bits, i, j), lane);
+                if (lane == 0) pl.deferred[j] = i;
+                return;
+            }
+            legacy = true;   // no room for the partial mask
+        }
+        if (legacy) {
+            if (lane == 0) pl.legacy[atomicAdd(&pl.counts[kCntLegacy], 1u)] = i;
             return;
         }
     }
     write_call_outputs<WANT_LIST ? 2 : 1>(C, i, lane, mask_bits, moves, moves_cap, n_moves, status, compact, compact_cap, compact_total, offsets);
+}
+
+// kick offsets of the common wall-kick table packed 4 bits each (+2), for the FIFO form of the T search
+__device__ __forceinline__ void stage_wall_kpack(uint32_t (&kp)[4][3][2], int tid) {
+    if (tid < 12) {
+        const int r = tid / 3, kd = tid % 3;
+        const TrlKicks& K = c_kicks[0][r][kd];
+        uint32_t px = 0, py = 0;
+        for (int ki = 0; ki < K.n; ++ki) {
+            px |= (uint32_t)(K.k[ki][0] + 2) << (4 * ki);
+            py |= (uint32_t)(K.k[ki][1] + 2) << (4 * ki);
+        }
+        kp[r][kd][0] = px;
+        kp[r][kd][1] = py;
+    }
+}
+
+// Stage deferred call j of the list for a T search: board rows, pieces, the partial mask of pass 1.  Returns via_hold
+// of the T search (T is the hold-or-next piece unless it is the current one).
+__device__ __forceinline__ bool stage_deferred(CallState& C, const PassLists& pl, unsigned j, int lane, const uint16_t* __restrict__ boards,
+                                               const uint8_t* __restrict__ cur, const uint8_t* __restrict__ alt,
+                                               const TrlGame* __restrict__ games, const int32_t* __restrict__ index,
+                                               uint32_t* mask_bits, int& i) {
+    i = pl.deferred[j];
+    int c, a, skip;
+    stage_call(C, i, lane, boards, cur, alt, games, index, c, a, skip);
+    load_mask(C, partial_mask(pl, mask_bits, i, j), lane);
+    __syncwarp();
+    return c != P_T;
+}
+
+// Pass 2: the T search of every deferred call, closure form with the order analysis.
+template <bool WANT_LIST>
+__global__ void __launch_bounds__(kTWarps * 32, 8)
+movegen_t_order_kernel(const uint16_t* __restrict__ boards, const uint8_t* __restrict__ cur,
+                       const uint8_t* __restrict__ alt, const TrlGame* __restrict__ games,
+                       const int32_t* __restrict__ index, uint32_t* __restrict__ mask_bits,
+                       uint16_t* __restrict__ moves, int moves_cap, uint16_t* __restrict__ n_moves,
+                       uint32_t* __restrict__ status, uint16_t* __restrict__ compact, unsigned long long compact_cap,
+                       unsigned long long* __restrict__ compact_total, unsigned long long* __restrict__ offsets,
+                       const PassLists pl) {
+    extern __shared__ __align__(16) uint8_t smem_raw[];
+    const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
+    SoloState& S = reinterpret_cast<SoloState*>(smem_raw)[warp];
+    CallState& C = S.C;
+    const unsigned count = min(pl.counts[kCntDeferred], pl.deferred_cap);
+#pragma unroll 1
+    while (true) {
+        const unsigned j = next_item(&pl.counts[kTicketOrder], lane);
+        if (j >= count) break;
+        int i;
+        const bool via_hold = stage_deferred(C, pl, j, lane, boards, cur, alt, games, index, mask_bits, i);
+        const bool ok = search_piece_rows<true, true>(S.P, C.rows, first_block_row(C.rows, lane), P_T, via_hold, C.mask);
+        __syncwarp();
+        if (!ok) {   // nothing was merged into the mask
+            if (lane == 0) pl.exact[atomicAdd(&pl.counts[kCntExact], 1u)] = (int32_t)j;
+            continue;
+        }
+        write_call_outputs<WANT_LIST ? 2 : 1>(C, i, lane, mask_bits, moves, moves_cap, n_moves, status, compact, compact_cap, compact_total, offsets);
+        __syncwarp();
+    }
+}
+
+// Pass 3: the exact FIFO search of the T piece for the calls pass 2 left undecided.
+template <bool WANT_LIST>
+__global__ void __launch_bounds__(kTWarps * 32, 8)
+movegen_t_exact_kernel(const uint16_t* __restrict__ boards, const uint8_t* __restrict__ cur,
+                       const uint8_t* __restrict__ alt, const TrlGame* __restrict__ games,
+                       const int32_t* __restrict__ index, uint32_t* __restrict__ mask_bits,
+                       uint16_t* __restrict__ moves, int moves_cap, uint16_t* __restrict__ n_moves,
+                       uint32_t* __restrict__ status, uint16_t* __restrict__ compact, unsigned long long compact_cap,
+                       unsigned long long* __restrict__ compact_total, unsigned long long* __restrict__ offsets,
+                       const PassLists pl) {
+    extern __shared__ __align__(16) uint8_t smem_raw[];
+    __shared__ uint32_t s_kpack[4][3][2];
+    const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
+    SoloState& S = reinterpret_cast<SoloState*>(smem_raw)[warp];
+    CallState& C = S.C;
+    stage_wall_kpack(s_kpack, tid);
+    __syncthreads();   // kick table staged; the only block-wide barrier
+    const unsigned count = pl.counts[kCntExact];
+#pragma unroll 1
+    while (true) {
+        const unsigned e = next_item(&pl.counts[kTicketExact], lane);
+        if (e >= count) break;
+        int i;
+        const bool via_hold = stage_deferred(C, pl, (unsigned)pl.exact[e], lane, boards, cur, alt, games, index, mask_bits, i);
+        uint32_t st = 0;
+        search_piece_fifo_body(S.P, C.rows, P_T, via_hold, C.mask, st, &s_kpack);
+        st = __reduce_or_sync(0xffffffffu, st);
+        if (st && lane == 0) C.status |= st;
+        __syncwarp();
+        write_call_outputs<WANT_LIST ? 2 : 1>(C, i, lane, mask_bits, moves, moves_cap, n_moves, status, compact, compact_cap, compact_total, offsets);
+        __syncwarp();
+    }
 }
 
 // ---------------------------------------------------------------------------------------
@@ -1703,24 +1869,24 @@ int trl_launch_movegen_listed(const TrlGame* games, const int32_t* index, const 
 }
 
 // Which form of the warp-cooperative enumeration runs: -1 automatic (by batch size), 0 = two warps per call
-// (latency form), 1 = one warp per call, 2 = two passes (closure-search kernel + exact clean-up; the
+// (latency form), 1 = one warp per call, 2 = the pass form (closure-search kernel + T passes + legacy route; the
 // throughput form).  Tests force all of them.
 static int g_form = -1;
 extern "C" void trl_movegen_warp_form(int form) { g_form = form; }
 
-// per-stream scratch of the two-pass form: [0] = undecided count, [16..] = undecided call indices
+// per-stream scratch of the pass form (PassLists): kCounters counters, the legacy, deferred and exact lists of n entries
+// each, then (only without a mask output) the partial masks
 struct TwoPassScratch { cudaStream_t stream; uint32_t* buf; size_t cap; bool used; };
 static TwoPassScratch g_scratch[8];
 
 static std::mutex g_scratch_mutex;   // device entry points are re-entrant per stream: the table is shared
 
-static uint32_t* two_pass_scratch(cudaStream_t stream, int n) {
+static uint32_t* two_pass_scratch(cudaStream_t stream, size_t need) {
     std::lock_guard<std::mutex> lock(g_scratch_mutex);
     TwoPassScratch* slot = nullptr;
     for (auto& e : g_scratch) if (e.used && e.stream == stream) { slot = &e; break; }
     if (!slot) for (auto& e : g_scratch) if (!e.used) { slot = &e; e.used = true; e.stream = stream; e.buf = nullptr; e.cap = 0; break; }
     if (!slot) return nullptr;
-    const size_t need = (size_t)n + 16;
     if (slot->cap < need) {
         cudaStreamCaptureStatus cs = cudaStreamCaptureStatusNone;
         if (cudaStreamIsCapturing(stream, &cs) != cudaSuccess || cs != cudaStreamCaptureStatusNone) return nullptr;
@@ -1731,17 +1897,44 @@ static uint32_t* two_pass_scratch(cudaStream_t stream, int n) {
     return slot->buf;
 }
 
+// partial masks without a mask output: max(64 Ki, n / 8) entries of 1448 B (the config-2 boards defer 6 % of the calls);
+// trl_debug_movegen_partial_cap lowers the capacity so that tests reach the legacy route of a full scratch
+static unsigned g_partial_cap_debug = 0;
+extern "C" int trl_debug_movegen_partial_cap(int cap) {
+    g_partial_cap_debug = cap > 0 ? (unsigned)cap : 0u;
+    return 0;
+}
+
+// counters of the last launch of the pass form (trl_debug_movegen_pass_counts)
+static uint32_t* g_last_counts = nullptr;
+static unsigned g_last_deferred_cap = 0;
+
+// counts[0] = calls whose T search pass 1 deferred (and found room), [1] = of those, calls pass 2 left to the exact T
+// search, [2] = calls on the legacy route; of the last launch of the pass form.  Synchronises the device.
+extern "C" int trl_debug_movegen_pass_counts(uint32_t* counts) {
+    if (!counts || !g_last_counts) return TRL_E_ARG;
+    uint32_t h[kCounters];
+    int rc = trl_check(cudaDeviceSynchronize());
+    if (!rc) rc = trl_check(cudaMemcpy(h, g_last_counts, sizeof(h), cudaMemcpyDeviceToHost));
+    if (rc) return rc;
+    counts[0] = h[kCntDeferred] < g_last_deferred_cap ? h[kCntDeferred] : g_last_deferred_cap;
+    counts[1] = h[kCntExact];
+    counts[2] = h[kCntLegacy];
+    return 0;
+}
+
 // Launch the warp-cooperative enumeration (same argument contract as movegen.cu's launch_movegen).
 int trl_launch_movegen_warp(const uint16_t* boards, const uint8_t* cur, const uint8_t* alt, const TrlGame* games,
                             const int32_t* index, int n, uint32_t* mask_bits, uint16_t* moves, int moves_cap,
                             uint16_t* n_moves, uint32_t* status, cudaStream_t stream, uint16_t* compact,
                             unsigned long long compact_cap, unsigned long long* compact_total,
                             unsigned long long* offsets) {
-    static int n_sm = 0;
+    static int n_sm = 0, t_order_blocks = 0, t_exact_blocks = 0;   // resident blocks of passes 2 and 3 per SM
     static bool configured = false;
     const size_t smem_warp = sizeof(PieceState) * kWarps + sizeof(CallState) * kCallsPerBlock;
     const size_t smem_solo = sizeof(SoloState) * kSoloWarps;
     const size_t smem_rows = sizeof(RowsWarp) * kRowsWarps;
+    const size_t smem_t = sizeof(SoloState) * kTWarps;
     if (!configured) {
         int dev = 0;
         int rc = trl_check(cudaGetDevice(&dev));
@@ -1753,6 +1946,14 @@ int trl_launch_movegen_warp(const uint16_t* boards, const uint8_t* cur, const ui
         if (!rc) rc = trl_check(cudaFuncSetAttribute(movegen_rows_kernel<false>, cudaFuncAttributePreferredSharedMemoryCarveout, 100));
         if (!rc) rc = trl_check(cudaFuncSetAttribute(movegen_rows_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_rows));
         if (!rc) rc = trl_check(cudaFuncSetAttribute(movegen_rows_kernel<true>, cudaFuncAttributePreferredSharedMemoryCarveout, 100));
+        for (const void* f : {(const void*)movegen_t_order_kernel<false>, (const void*)movegen_t_order_kernel<true>,
+                              (const void*)movegen_t_exact_kernel<false>, (const void*)movegen_t_exact_kernel<true>}) {
+            if (!rc) rc = trl_check(cudaFuncSetAttribute(f, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_t));
+            if (!rc) rc = trl_check(cudaFuncSetAttribute(f, cudaFuncAttributePreferredSharedMemoryCarveout, 100));
+        }
+        // the two instantiations of a pass differ only in the list writer: the mask-mode one sizes the grid
+        if (!rc) rc = trl_check(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&t_order_blocks, movegen_t_order_kernel<false>, kTWarps * 32, smem_t));
+        if (!rc) rc = trl_check(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&t_exact_blocks, movegen_t_exact_kernel<false>, kTWarps * 32, smem_t));
         if (rc) return rc;
         configured = true;
     }
@@ -1761,25 +1962,41 @@ int trl_launch_movegen_warp(const uint16_t* boards, const uint8_t* cur, const ui
     int form = g_form < 0 ? (n >= 3 * 4736 ? 2 : 0) : g_form;
     // the debug switches (FIFO form only / lowered FIFO capacity) are served by the one-kernel forms
     if (form == 2 && (!g_fast_path_host || g_fifo_limit_host != kFifoCap)) form = 1;
-    uint32_t* scratch = form == 2 ? two_pass_scratch(stream, n) : nullptr;
+    // pass form: counters, three lists of n entries, and without a mask output the partial masks
+    unsigned deferred_cap = (unsigned)n;
+    if (!mask_bits) deferred_cap = (unsigned)min(n, max(64 * 1024, n / 8));
+    if (g_partial_cap_debug) deferred_cap = min(deferred_cap, g_partial_cap_debug);
+    const size_t lists = kCounters + 3 * (size_t)n;
+    uint32_t* scratch = form == 2 ? two_pass_scratch(stream, lists + (mask_bits ? 0 : (size_t)deferred_cap * TRL_MASK_WORDS)) : nullptr;
     if (form == 2 && !scratch) form = 1;
     if (form == 2) {
-        int rc = trl_check(cudaMemsetAsync(scratch, 0, sizeof(uint32_t), stream));
+        const PassLists pl{scratch, (int32_t*)scratch + kCounters, (int32_t*)scratch + kCounters + n,
+                           (int32_t*)scratch + kCounters + 2 * (size_t)n, mask_bits ? nullptr : scratch + lists, deferred_cap};
+        g_last_counts = scratch;
+        g_last_deferred_cap = deferred_cap;
+        int rc = trl_check(cudaMemsetAsync(scratch, 0, kCounters * sizeof(uint32_t), stream));
         if (rc) return rc;
-        if (moves || compact)
-            movegen_rows_kernel<true><<<(n + kRowsWarps - 1) / kRowsWarps, kRowsWarps * 32, smem_rows, stream>>>(
-                boards, cur, alt, games, index, n, mask_bits, moves, moves_cap, n_moves, status, compact, compact_cap,
-                compact_total, offsets, (int32_t*)(scratch + 16), scratch);
-        else
-            movegen_rows_kernel<false><<<(n + kRowsWarps - 1) / kRowsWarps, kRowsWarps * 32, smem_rows, stream>>>(
-                boards, cur, alt, games, index, n, mask_bits, moves, moves_cap, n_moves, status, compact, compact_cap,
-                compact_total, offsets, (int32_t*)(scratch + 16), scratch);
+        const bool want_list = moves || compact;
+        const int rows_blocks = (n + kRowsWarps - 1) / kRowsWarps;
+        (want_list ? movegen_rows_kernel<true> : movegen_rows_kernel<false>)<<<rows_blocks, kRowsWarps * 32, smem_rows, stream>>>(
+            boards, cur, alt, games, index, n, mask_bits, moves, moves_cap, n_moves, status, compact, compact_cap,
+            compact_total, offsets, pl);
+        rc = trl_check(cudaGetLastError());
+        if (rc) return rc;
+        (want_list ? movegen_t_order_kernel<true> : movegen_t_order_kernel<false>)<<<t_order_blocks * n_sm, kTWarps * 32, smem_t, stream>>>(
+            boards, cur, alt, games, index, mask_bits, moves, moves_cap, n_moves, status, compact, compact_cap,
+            compact_total, offsets, pl);
+        rc = trl_check(cudaGetLastError());
+        if (rc) return rc;
+        (want_list ? movegen_t_exact_kernel<true> : movegen_t_exact_kernel<false>)<<<t_exact_blocks * n_sm, kTWarps * 32, smem_t, stream>>>(
+            boards, cur, alt, games, index, mask_bits, moves, moves_cap, n_moves, status, compact, compact_cap,
+            compact_total, offsets, pl);
         rc = trl_check(cudaGetLastError());
         if (rc) return rc;
         const int blocks = min(8 * n_sm, (n + kSoloWarps - 1) / kSoloWarps);
         movegen_solo_kernel<<<blocks, kSoloWarps * 32, smem_solo, stream>>>(
             boards, cur, alt, games, index, n, mask_bits, moves, moves_cap, n_moves, status, compact, compact_cap,
-            compact_total, offsets, (const int32_t*)(scratch + 16), scratch);
+            compact_total, offsets, pl.legacy, pl.counts + kCntLegacy);
         return trl_check(cudaGetLastError());
     }
     if (form == 1) {

@@ -1,9 +1,9 @@
 """Search statistics of the movegen sweep's kernel (needs a build with TRL_NVCC_EXTRA=-DTRL_MOVEGEN_STATS):
-python tools/movegen_stats.py.  Runs the two-pass form, as the sweep does: rounds, fill iterations, (rotation, direction)
-passes and kick tests are those of movegen_rows_kernel's specialised closure search; a pair of twin passes packed into
-one word counts as one pass.  The first line mixes two piece types per call, so it also counts the searches the clean-up
-pass repeats for the other piece of an undecided call; the per-piece lines search one piece per call and count each
-search once."""
+python tools/movegen_stats.py.  Runs the pass form, as the sweep does: rounds, fill iterations, (rotation, direction)
+passes and kick tests are those of the specialised closure search in movegen_rows_kernel and, for the T searches it
+deferred, once more in movegen_t_order_kernel; a pair of twin passes packed into one word counts as one pass.  The first
+line mixes two piece types per call, so it also counts the searches the legacy route repeats for the other piece of an
+undecided call; the per-piece lines search one piece per call (the T line counts a deferred search twice)."""
 import ctypes, sys, os
 import numpy as np, torch
 sys.path.insert(0, os.getcwd())
