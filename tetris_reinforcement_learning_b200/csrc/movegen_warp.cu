@@ -115,7 +115,8 @@ __device__ __forceinline__ void flag_cell(uint32_t* fu_row, uint32_t bit, bool u
 //
 //   * two rotations share a register (16 bits each, validity rows are 14 bits wide, the two spare bits
 //     stop the carries of hflood): VA/VB validity, RA/RB reached; A holds rotations 0 | 2 << 16, B 1 | 3 << 16,
-//     so that each pair of kick passes with equal kick lists runs in one word (kick_pass_pair);
+//     so that each pair of kick passes with equal kick lists runs in one word (kick_pass_pair; the I piece's pairs run
+//     on planes of their own, kick_pass_pair_i);
 //   * fill = alternate "expand along rows" (hflood, O(1)) and "fall straight down" (a segmented
 //     Hillis-Steele OR-scan over lanes, 5 shuffles, propagate masks precomputed) until nothing changes —
 //     all four rotations at once, instead of one serial row scan per queue entry;
@@ -134,9 +135,6 @@ __device__ __forceinline__ void flag_cell(uint32_t* fu_row, uint32_t bit, bool u
 // above the window are not represented).  Counted in g_fast_stats: 24 % of the T searches, 0 of the others,
 // on the BASELINE config-2 boards.
 // ---------------------------------------------------------------------------------------
-#ifndef TRL_ROWS_SPECIAL_I
-#define TRL_ROWS_SPECIAL_I 0   // closure kernel: compile-time kick tables for the I piece too: measured SLOWER (4.63 vs 4.12 ms per 700 k calls: the code outgrows the instruction cache)
-#endif
 #ifndef TRL_ROWS_SPECIAL_V
 #define TRL_ROWS_SPECIAL_V 1   // closure kernel: validity rows with compile-time cell offsets (A/B switch)
 #endif
@@ -204,7 +202,7 @@ constexpr KickList kIKicks[4][3] = {
     {{5, {{0, 0}, {1, 0}, {-2, 0}, {1, -2}, {-2, 1}, {0, 0}}}, {2, {{0, 0}, {-1, 0}, {0, 0}, {0, 0}, {0, 0}, {0, 0}}}, {5, {{0, 0}, {-2, 0}, {1, 0}, {-2, -1}, {1, 2}, {0, 0}}}},
 };
 
-constexpr bool same_kicks(const KickList& a, const KickList& b) {
+__host__ __device__ constexpr bool same_kicks(const KickList& a, const KickList& b) {
     if (a.n != b.n) return false;
     for (int ki = 0; ki < a.n; ++ki)
         if (a.k[ki][0] != b.k[ki][0] || a.k[ki][1] != b.k[ki][1]) return false;
@@ -215,6 +213,11 @@ static_assert(same_kicks(kWallKicks[0][0], kWallKicks[2][2]), "twin pair (0, 0) 
 static_assert(same_kicks(kWallKicks[0][2], kWallKicks[2][0]), "twin pair (0, 2) / (2, 0)");
 static_assert(same_kicks(kWallKicks[1][0], kWallKicks[1][2]), "twin pair (1, 0) / (1, 2)");
 static_assert(same_kicks(kWallKicks[3][0], kWallKicks[3][2]), "twin pair (3, 0) / (3, 2)");
+// ... and the four of the I piece that kick_pass_pair_i runs in one word (const.py:214-235)
+static_assert(same_kicks(kIKicks[0][0], kIKicks[3][2]), "I twin pair (0, 0) / (3, 2)");
+static_assert(same_kicks(kIKicks[1][0], kIKicks[0][2]), "I twin pair (1, 0) / (0, 2)");
+static_assert(same_kicks(kIKicks[2][0], kIKicks[1][2]), "I twin pair (2, 0) / (1, 2)");
+static_assert(same_kicks(kIKicks[3][0], kIKicks[2][2]), "I twin pair (3, 0) / (2, 2)");
 
 #ifdef TRL_MOVEGEN_STATS
 #define TRL_COUNT(x) (++(x))
@@ -227,8 +230,16 @@ static_assert(same_kicks(kWallKicks[3][0], kWallKicks[3][2]), "twin pair (3, 0) 
 // row reaches with kx <= 2.
 #define TRL_VV(S, r, row, sh) ((S).vv[(r) & 1][row] >> ((sh) + 16 * ((r) >> 1)))
 
+// PRMT selector of __byte_perm(A, B, .) for words packed like VA / VB (A = rot0 | rot2 << 16, B = rot1 | rot3 << 16):
+// rotation lo's half into the low half of the result, rotation hi's into the high half.
+__host__ __device__ constexpr uint32_t half_sel(int lo, int hi) {
+    const uint32_t bl = 4 * (lo & 1) + 2 * (lo >> 1), bh = 4 * (hi & 1) + 2 * (hi >> 1);
+    return bl | (bl + 1) << 4 | bh << 8 | (bh + 1) << 12;
+}
+
 // One (source rotation R, direction KD) pass over the new edge cells `ne` of this lane's row; TAB 0 = the six pieces
-// with the common wall-kick table, 1 = the I piece.
+// with the common wall-kick table (validity planes TRL_VV), 1 = the I piece (its four planes, kick_pass_pair_i: rotation
+// nrot is the low half of plane nrot).
 template <int TAB, int R, int KD, class St>
 __device__ __forceinline__ void kick_pass_wall(St& S, int lane, uint32_t ne, uint32_t VA, uint32_t VB, uint32_t& a0A, uint32_t& a0B, bool is_T,
                                                unsigned& n_pass, unsigned& n_test) {
@@ -247,7 +258,10 @@ __device__ __forceinline__ void kick_pass_wall(St& S, int lane, uint32_t ne, uin
     for (int ki = 1; ki < K.n; ++ki) {
         TRL_COUNT(n_test);
         const int kx = K.k[ki][0], ky = K.k[ki][1];
-        const uint32_t cand = rem & TRL_VV(S, nrot, lane + 2 - ky, kx + 2);   // source bit ex <-> target bit ex + kx
+        uint32_t tv;   // source bit ex <-> target bit ex + kx
+        if constexpr (TAB) tv = S.vv[nrot][lane + 2 - ky] >> (kx + 2);
+        else tv = TRL_VV(S, nrot, lane + 2 - ky, kx + 2);
+        const uint32_t cand = rem & tv;
         rem &= ~cand;
         if (cand) {
             uint32_t arr = kx >= 0 ? (cand << kx) : (cand >> -kx);
@@ -256,14 +270,6 @@ __device__ __forceinline__ void kick_pass_wall(St& S, int lane, uint32_t ne, uin
         }
         if (ki + 1 < K.n && !__any_sync(0xffffffffu, rem)) return;              // every edge cell has found its kick
     }
-}
-
-template <int TAB, int R, class St>
-__device__ __forceinline__ void kick_passes_wall(St& S, int lane, uint32_t ne, uint32_t VA, uint32_t VB, uint32_t& a0A, uint32_t& a0B, bool is_T,
-                                                 unsigned& n_pass, unsigned& n_test) {
-    kick_pass_wall<TAB, R, 0>(S, lane, ne, VA, VB, a0A, a0B, is_T, n_pass, n_test);
-    kick_pass_wall<TAB, R, 1>(S, lane, ne, VA, VB, a0A, a0B, is_T, n_pass, n_test);
-    kick_pass_wall<TAB, R, 2>(S, lane, ne, VA, VB, a0A, a0B, is_T, n_pass, n_test);
 }
 
 // Two (source rotation, direction) passes of the common wall-kick table with equal kick lists, one per 16-bit half:
@@ -323,6 +329,48 @@ __device__ __forceinline__ void kick_pass_pair(St& S, int lane, uint32_t src, ui
     }
 }
 
+// Two passes of the I piece with equal kick lists, one per 16-bit half.  Every I twin pair has an even and an odd source
+// rotation and an even and an odd target, so the closure search stores the I piece's validity in four planes instead of
+// two: plane p = (rotation p | rotation p + 1 << 16) << 2.  Pass pair P targets plane P as it is: the low half runs
+// (P - 1, 0) -> P, the high half (P - 2, 2) -> P + 1 (rotations mod 4); the source word takes one half of nA and one of
+// nB (one PRMT per pass), and arrivals split into the two target rotations.  Exact like kick_pass_pair: "first valid kick
+// wins" runs per bit; the edge bits of the low half sit in 0..13 and a kick test reads target bits ex + kx + 2 <= 17
+// (|kx| <= 2), and bits 16 and 17 of a plane are 0 (the << 2), so the low half never reads the high half; the high half
+// reads bits >= 16 only; an arrival stays in its half since `cand` implies a valid target bit.  No I pass sets a
+// used-last-kick flag (that is T only).
+template <int P, class St>
+__device__ __forceinline__ void kick_pass_pair_i(St& S, int lane, uint32_t nA, uint32_t nB, uint32_t& a0A, uint32_t& a0B,
+                                                 unsigned& n_pass, unsigned& n_test) {
+    constexpr int RL = (P + 3) & 3, RH = (P + 2) & 3, Q = (P + 1) & 3;   // low / high half: sources RL, RH, targets P, Q
+    constexpr KickList K = kIKicks[RL][0];
+    static_assert(same_kicks(K, kIKicks[RH][2]) && ((RL + 1) & 3) == P && ((RH + 3) & 3) == Q, "an I twin pair targeting plane P");
+    const uint32_t src = __byte_perm(nA, nB, half_sel(RL, RH));
+#ifdef TRL_MOVEGEN_STATS
+    if (__any_sync(0xffffffffu, src)) TRL_COUNT(n_pass);
+#endif
+    const uint32_t c0 = src & (S.vv[P][lane + 2] >> 2);   // from the plane: a PRMT of VA, VB would be hoisted out of the round loop
+    const uint32_t c0l = (c0 & 0xFFFFu) << (16 * (P >> 1)), c0h = (c0 >> 16) << (16 * (Q >> 1));
+    if (P & 1) a0B |= c0l; else a0A |= c0l;
+    if (Q & 1) a0B |= c0h; else a0A |= c0h;
+    uint32_t rem = src & ~c0;
+    if (!__any_sync(0xffffffffu, rem)) return;
+#pragma unroll
+    for (int ki = 1; ki < K.n; ++ki) {
+        TRL_COUNT(n_test);
+        const int kx = K.k[ki][0], ky = K.k[ki][1];
+        const int row = lane + 2 - ky;
+        const uint32_t cand = rem & (S.vv[P][row] >> (kx + 2));
+        rem &= ~cand;
+        if (cand) {
+            const uint32_t arr = kx >= 0 ? (cand << kx) : (cand >> -kx);
+            const uint32_t lo = arr & 0xFFFFu, hi = arr >> 16;
+            if (lo) atomicOr(&S.fu[P][row], lo);
+            if (hi) atomicOr(&S.fu[Q][row], hi);
+        }
+        if (ki + 1 < K.n && !__any_sync(0xffffffffu, rem)) return;
+    }
+}
+
 // (rot0 | rot2 << 16, rot1 | rot3 << 16) <-> (rot0 | rot1 << 16, rot2 | rot3 << 16): exchange the high half of A with the
 // low half of B (its own inverse)
 __device__ __forceinline__ void swap_mid_halves(uint32_t& A, uint32_t& B) {
@@ -331,7 +379,7 @@ __device__ __forceinline__ void swap_mid_halves(uint32_t& A, uint32_t& B) {
     B = b;
 }
 
-// St: anything with uint32_t vv[>= 2][>= kWinRows], fu[4][>= kWinRows] in shared memory.  The loops are kept
+// St: anything with uint32_t vv[4][>= kWinRows], fu[4][>= kWinRows] in shared memory.  The loops are kept
 // rolled on purpose: the kernels that call this are bound by instruction fetch, not by loop overhead.
 // ---------------------------------------------------------------------------------------
 // T: which flag did the LAST rotation-flagged emission of a cell carry, when it received both?
@@ -554,7 +602,8 @@ __device__ __forceinline__ void validity_rows(const uint32_t (&e)[4], uint32_t (
     v[3] = validity_row<TYPE, 3>(e);
 }
 
-// SPECIAL: kick passes of the non-I pieces with compile-time tables, twin passes packed (the closure kernels).
+// SPECIAL: kick passes with compile-time tables, twin passes packed (the closure kernels); without it the generic loop
+// over c_kicks (the kernels that also carry the FIFO form).
 // T_ORDER: a T search with mixed flags goes through t_order_decide (St needs tsnap and tp).  Without it the search
 // keeps no snapshot of the first two kick rounds and returns false ("deferred") for every T search with mixed flags:
 // the sweep's first pass, which leaves the order analysis to a kernel of its own.
@@ -597,13 +646,22 @@ __device__ __forceinline__ bool search_piece_rows(St& S, const uint16_t* rows, i
         if (r & 1) VB |= sh; else VA |= sh;
     }
     }
-    // shared planes, row index lane + 2: validity << 2 for the kick tests, packed like VA / VB (TRL_VV); arrivals per
-    // rotation (T: low half = flag clear, high half = used-last-kick)
+    // shared planes, row index lane + 2: validity << 2 for the kick tests, packed like VA / VB (TRL_VV), or for the I piece
+    // in the specialised search as four planes (kick_pass_pair_i); arrivals per rotation (T: low half = flag clear, high
+    // half = used-last-kick)
     {
         const int pad = lane < 2 ? lane : lane + 32;
-        S.vv[0][lane + 2] = VA << 2;
-        S.vv[1][lane + 2] = VB << 2;
-        if (lane < 4) { S.vv[0][pad] = 0u; S.vv[1][pad] = 0u; }
+        if (SPECIAL && type == P_I) {
+#pragma unroll
+            for (int p = 0; p < 4; ++p) {
+                S.vv[p][lane + 2] = __byte_perm(VA, VB, half_sel(p, (p + 1) & 3)) << 2;
+                if (lane < 4) S.vv[p][pad] = 0u;
+            }
+        } else {
+            S.vv[0][lane + 2] = VA << 2;
+            S.vv[1][lane + 2] = VB << 2;
+            if (lane < 4) { S.vv[0][pad] = 0u; S.vv[1][pad] = 0u; }
+        }
 #pragma unroll
         for (int r = 0; r < 4; ++r) {
             S.fu[r][lane + 2] = 0u;
@@ -672,7 +730,18 @@ __device__ __forceinline__ bool search_piece_rows(St& S, const uint16_t* rows, i
         const uint32_t nA = EA & ~doneA, nB = EB & ~doneB;
         doneA = EA; doneB = EB;
         if (!__any_sync(0xffffffffu, nA | nB)) break;
-        if (SPECIAL && tab == 0) {
+        if constexpr (SPECIAL) {
+          if (tab == 1) {
+            // the I piece: its eight passes with a twin as four packed passes, then the four 180-degree passes (one kick each)
+            kick_pass_pair_i<0>(S, lane, nA, nB, a0A, a0B, stat_4, stat_5);   // (3, 0) -> 0 | (2, 2) -> 1
+            kick_pass_pair_i<1>(S, lane, nA, nB, a0A, a0B, stat_4, stat_5);   // (0, 0) -> 1 | (3, 2) -> 2
+            kick_pass_pair_i<2>(S, lane, nA, nB, a0A, a0B, stat_4, stat_5);   // (1, 0) -> 2 | (0, 2) -> 3
+            kick_pass_pair_i<3>(S, lane, nA, nB, a0A, a0B, stat_4, stat_5);   // (2, 0) -> 3 | (1, 2) -> 0
+            kick_pass_wall<1, 0, 1>(S, lane, nA & 0xFFFFu, VA, VB, a0A, a0B, false, stat_4, stat_5);
+            kick_pass_wall<1, 1, 1>(S, lane, nB & 0xFFFFu, VA, VB, a0A, a0B, false, stat_4, stat_5);
+            kick_pass_wall<1, 2, 1>(S, lane, nA >> 16, VA, VB, a0A, a0B, false, stat_4, stat_5);
+            kick_pass_wall<1, 3, 1>(S, lane, nB >> 16, VA, VB, a0A, a0B, false, stat_4, stat_5);
+          } else {
             // the eight passes with a twin as four packed passes, then the four 180-degree passes
             if (__any_sync(0xffffffffu, nA)) {
                 kick_pass_pair<0, 0>(S, lane, nA, VA, VB, a0A, a0B, is_T, stat_4, stat_5);   // + (2, 2): target 1
@@ -689,21 +758,13 @@ __device__ __forceinline__ bool search_piece_rows(St& S, const uint16_t* rows, i
                 kick_pass_pair<3, 0>(S, lane, n3 | (n3 << 16), VA, VB, a0A, a0B, is_T, stat_4, stat_5);   // + (3, 2): targets 0 | 2
                 kick_pass_wall<0, 3, 1>(S, lane, n3, VA, VB, a0A, a0B, is_T, stat_4, stat_5);
             }
+          }
         } else {
 #pragma unroll 1
         for (int r = 0; r < 4; ++r) {
             const uint32_t X = (r & 1) ? nB : nA;
             const uint32_t ne = (r & 2) ? (X >> 16) : (X & 0xFFFFu);
             if (!__any_sync(0xffffffffu, ne)) continue;
-            if (SPECIAL && TRL_ROWS_SPECIAL_I) {
-                switch (r) {
-                    case 0: kick_passes_wall<1, 0>(S, lane, ne, VA, VB, a0A, a0B, false, stat_4, stat_5); break;
-                    case 1: kick_passes_wall<1, 1>(S, lane, ne, VA, VB, a0A, a0B, false, stat_4, stat_5); break;
-                    case 2: kick_passes_wall<1, 2>(S, lane, ne, VA, VB, a0A, a0B, false, stat_4, stat_5); break;
-                    default: kick_passes_wall<1, 3>(S, lane, ne, VA, VB, a0A, a0B, false, stat_4, stat_5); break;
-                }
-                continue;
-            }
 #pragma unroll 1
             for (int kd = 0; kd < 3; ++kd) {
                 TRL_STAT(4);
@@ -1490,7 +1551,7 @@ struct PassLists {
 };
 
 struct RowsState {
-    uint32_t vv[2][kWinRows];   // packed validity planes (0 | 2, 1 | 3), TRL_VV
+    uint32_t vv[4][kWinRows];   // packed validity planes (0 | 2, 1 | 3), TRL_VV; the I piece uses four (kick_pass_pair_i)
     uint32_t fu[4][kWinRows];
 };
 

@@ -1,11 +1,14 @@
 """Per-kernel time of the config-2 movegen sweep and the work that reaches each pass.
 
-    python tools/movegen_passes.py [--boards 1000000] [--sweeps 10] [--out DIR]
+    python tools/movegen_passes.py [--boards 1000000] [--sweeps 10] [--out DIR] [--per-piece]
 
 Runs the sweep bench.py times (mask output, device-resident inputs) under torch.profiler with CUDA activities and
 prints every kernel's time per sweep, then the pass counts of one sweep outside the profiler: calls whose T search
 pass 1 deferred, calls the T order analysis left undecided (they take the exact T search), and calls on the legacy
 route (movegen_solo_kernel in clean-up mode).  A library without the pass-count getter prints only the kernel times.
+
+--per-piece instead times the sweep's boards once per piece type t with cur = alt = t, so that every call is one search
+of that piece, with CUDA events around `--sweeps` sweeps after three warm-up sweeps, and prints ms per sweep per piece.
 """
 import argparse
 import ctypes
@@ -41,11 +44,38 @@ def pass_counts(L):
     return tuple(int(v) for v in c)
 
 
+def per_piece(args, d_b, d_mask, d_n, d_st):
+    from tetris_reinforcement_learning_b200.const import MINOS
+    n = d_b.shape[0]
+    res = {"card": card(), "calls": n, "sweeps": args.sweeps, "ms_per_sweep": {}}
+    print(f"card: {res['card']}")
+    print(f"config-2 boards, {n} calls with cur = alt = t (one search per call), {args.sweeps} sweeps, CUDA events")
+    start, stop = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+    for t in range(7):
+        d_t = torch.full((n,), t, dtype=torch.uint8, device=d_b.device)
+        for _ in range(3):
+            move_generation.movegen_device(d_b, d_t, d_t, d_mask, None, d_n, d_st)
+        start.record()
+        for _ in range(args.sweeps):
+            move_generation.movegen_device(d_b, d_t, d_t, d_mask, None, d_n, d_st)
+        stop.record()
+        stop.synchronize()
+        ms = start.elapsed_time(stop) / args.sweeps
+        res["ms_per_sweep"][MINOS[t]] = ms
+        print(f"  {MINOS[t]}  {ms:9.3f} ms/sweep  {1e6 * ms / n:7.3f} ns/search")
+    print(f"  sum of the seven: {sum(res['ms_per_sweep'].values()):.3f} ms")
+    if args.out:
+        os.makedirs(args.out, exist_ok=True)
+        with open(os.path.join(args.out, "movegen_per_piece.json"), "w") as f:
+            json.dump(res, f, indent=1)
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--boards", type=int, default=1_000_000)
     ap.add_argument("--sweeps", type=int, default=10)
     ap.add_argument("--out", default=None, help="also write the result as JSON into this directory")
+    ap.add_argument("--per-piece", action="store_true", help="time one search per call, per piece type (cur = alt = t)")
     args = ap.parse_args()
     assert torch.cuda.is_available(), "movegen_passes.py needs a CUDA device"
     L = _native.lib()
@@ -60,6 +90,10 @@ def main():
 
     def sweep():
         move_generation.movegen_device(d_b, d_c, d_a, d_mask, None, d_n, d_st)
+
+    if args.per_piece:
+        per_piece(args, d_b, d_mask, d_n, d_st)
+        return
 
     for _ in range(3):
         sweep()
