@@ -14,6 +14,10 @@
  *   - `*_host` entry points take HOST pointers, stage through an internal device
  *     workspace and synchronise before returning (this is what a reference-side caller
  *     such as get_move_matrix(player) binds to).
+ *   - devices: a call runs on the CUDA device current in the calling thread, and every
+ *     device pointer and stream it receives must belong to that device.  What the library
+ *     keeps between calls (workspace, host streams, kernel attributes, debug switches) is
+ *     kept per device, so one process may drive several devices (device index < 64).
  *   - return value: 0 = TRL_OK, negative = error (see TRL_E_*); never throws.
  *   - per-item anomalies (queue overflow, no legal move, ...) are reported in a per-item
  *     `status` word (TRL_ST_* bits), not in the return value.

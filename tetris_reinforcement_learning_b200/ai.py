@@ -255,20 +255,40 @@ def samples_from_search(state_rec, moves, visits, augment=True):
 # self-play
 # ---------------------------------------------------------------------------------------------
 
-def _engine_for(config, net, n_games, seed=None, **kw):
+def _time_seed(seed):
+    return int(time.time_ns() & 0x7FFFFFFF) if seed is None else seed
+
+
+def _engine_for(config, net, n_games, seed=None, device=None, **kw):
+    """Engine of n_games on `device` (default: the current device).  A network is copied to that device; a callable
+    evaluator is used as given and must accept inputs on it."""
     from .selfplay import SelfPlayEngine, best_evaluator
     if not torch.cuda.is_available():
         raise RuntimeError("self-play needs a CUDA device: the search, rules and placements run in libtrl_b200.so "
                            "(there is no CPU fallback)")
-    seed = int(time.time_ns() & 0x7FFFFFFF) if seed is None else seed
+    seed = _time_seed(seed)
     dtype = kw.pop("dtype", torch.bfloat16)
-    if callable(net) and not isinstance(net, torch.nn.Module):
-        evaluator = net
-    else:
-        import copy
-        evaluator = best_evaluator(copy.deepcopy(net).to("cuda"), dtype)  # the caller's module is left untouched
-    kw.setdefault("device", torch.device("cuda", torch.cuda.current_device()))   # one process per GPU: the current device
-    return SelfPlayEngine(config, evaluator, n_games, seed=seed, feature_dtype=dtype, **kw)
+    device = torch.device("cuda", torch.cuda.current_device()) if device is None else torch.device(device)
+    with torch.cuda.device(device):
+        if callable(net) and not isinstance(net, torch.nn.Module):
+            evaluator = net
+        else:
+            import copy
+            evaluator = best_evaluator(copy.deepcopy(net).to(device), dtype)  # the caller's module is left untouched
+        return SelfPlayEngine(config, evaluator, n_games, seed=seed, feature_dtype=dtype, device=device, **kw)
+
+
+def _shard_engines(config, net, num_games, concurrent, seed, first_game_id, game_id_stride, **kw):
+    """One engine per entry of config.engine_devices, each playing its devices.shard_games share of the ids (finished
+    games restart while the shard has more games than slots).  -> [(engine, shard)]."""
+    from .devices import engine_devices, shard_games
+    devs = engine_devices(config)
+    out = []
+    for sh in shard_games(num_games, concurrent, first_game_id, game_id_stride, len(devs)):
+        eng = _engine_for(config, net, sh["concurrent"], seed=seed, device=devs[sh["shard"]], first_game_id=sh["first_game_id"],
+                          game_id_stride=sh["game_id_stride"], restart_finished=sh["concurrent"] < sh["num_games"], **kw)
+        out.append((eng, sh))
+    return out
 
 
 def generate_games(config, net, num_games, seed=None, concurrent=None, augment=None, dtype=torch.bfloat16,
@@ -278,35 +298,42 @@ def generate_games(config, net, num_games, seed=None, concurrent=None, augment=N
     (ai.py:1817-1820): series_data = 13-element samples grouped per game (player 0's samples,
     then player 1's), series_stats = one APP/DSPP dict per game.  compact=True: series_data is a
     compact.CompactSet holding the same samples in the same order (sample i of the list =
-    CompactSet.batch_tensors([i])), without building Python lists."""
+    CompactSet.batch_tensors([i])), without building Python lists.
+
+    config.engine_devices: the games are sharded by id over the listed devices (devices.shard_games), all engines
+    stepped from this thread, and the records merged; the set is the one a single device plays (see Config)."""
     augment = config.augment_data if augment is None else augment
     G = int(concurrent or num_games)
-    eng = _engine_for(config, net, G, seed=seed, dtype=dtype, first_game_id=first_game_id,
-                      game_id_stride=game_id_stride, restart_finished=(G < num_games), random_openings=True)
+    shards = _shard_engines(config, net, num_games, G, _time_seed(seed), first_game_id, game_id_stride, dtype=dtype,
+                            random_openings=True)
     # steps between two drains: a game finishes at most one search per `iters_min` steps and the sample ring holds
     # 4 records per game, so at most 3 * iters_min steps may pass (random opening plies leave no record)
     iters_min = config.playout_iterations()[1] if (config.training and config.use_playout_cap_randomization) else config.MAX_ITER
     chunk = max(1, min(max(8, config.MAX_ITER // 2), 3 * max(1, iters_min)))
     per_game, finished = {}, {}
     all_samples, all_ends = [], []
+    running = [(eng, sh["num_games"], set()) for eng, sh in shards]   # (engine, its share, ids it finished)
     steps = 0
-    while len(finished) < num_games:
-        eng.step(chunk)
+    while running:
+        for eng, _, _ in running:    # queue every engine's graphs before the first drain waits for its device
+            eng.step(chunk)
         steps += chunk
-        samples, ends = eng.drain()
-        eng.check_status()   # overflowed FIFO / arena / rings, a root without a move: the reference asserts (ai.py:417,1347)
-        if compact:       # no per-record Python: the set is assembled from the arrays at the end
-            all_samples.append(samples)
-            all_ends.append(ends)
-        else:
-            for s in samples:
-                per_game.setdefault(int(s["game_id"]), []).append(s)
-        for e in ends:
-            finished[int(e["game_id"])] = e
-        if max_steps is not None and steps >= max_steps:
-            break
-        if not eng.get_ctl()["active"].any():
-            break
+        still = []
+        for eng, quota, done in running:
+            samples, ends = eng.drain()
+            eng.check_status()   # overflowed FIFO / arena / rings, a root without a move: the reference asserts (ai.py:417,1347)
+            if compact:       # no per-record Python: the set is assembled from the arrays at the end
+                all_samples.append(samples)
+                all_ends.append(ends)
+            else:
+                for s in samples:
+                    per_game.setdefault(int(s["game_id"]), []).append(s)
+            for e in ends:
+                finished[int(e["game_id"])] = e
+                done.add(int(e["game_id"]))
+            if len(done) < quota and (max_steps is None or steps < max_steps) and eng.get_ctl()["active"].any():
+                still.append((eng, quota, done))
+        running = still
     data_number, model_number = highest_data_number(config) + 1, highest_model_number(config)
     series_data, series_stats = [], []
     for gid in sorted(finished)[:num_games]:
@@ -421,8 +448,8 @@ _CACHE_ENTRIES = 4
 # Engines and evaluators are built from a copy of the caller's network and kept between calls.  An entry is
 # (weak reference to the network, value): it serves only the very object it was built for, so a network freed and
 # replaced by another one at the same address (same id, same parameter versions after load_state_dict) misses.
-_search_engines = {}   # (network identity + weight versions, search settings, seed, batch) -> entry
-_evaluators = {}       # network identity + weight versions -> entry of evaluate() / evaluate_positions()
+_search_engines = {}   # (network identity + weight versions, search settings, seed, batch, device, block) -> entry
+_evaluators = {}       # (network identity + weight versions, device) -> entry of evaluate() / evaluate_positions()
 
 
 def _net_identity(net):
@@ -444,31 +471,45 @@ def _cache_get(cache, key, net):
     return entry[1] if entry is not None and entry[0]() is net else None
 
 
-def _cache_put(cache, key, net, value):
+def _cache_put(cache, key, net, value, device=None):
+    """At most _CACHE_ENTRIES entries per device, the oldest leaving first."""
     cache.pop(key, None)
-    while len(cache) >= _CACHE_ENTRIES:
-        cache.pop(next(iter(cache)))
-    cache[key] = (_net_ref(net), value)
+    same_device = [k for k, entry in cache.items() if entry[2] == device]
+    for k in same_device[:max(0, len(same_device) - _CACHE_ENTRIES + 1)]:
+        cache.pop(k)
+    cache[key] = (_net_ref(net), value, device)
 
 
 def release_cached_engines():
     """Drop the search engines and evaluators that MCTS(), analyse(), evaluate() and evaluate_positions() keep
-    between calls (tree arenas of several GB for thousands of positions) and return their device memory."""
+    between calls (tree arenas of several GB for thousands of positions) and return their memory on every device."""
     _search_engines.clear()
     _evaluators.clear()
     if torch.cuda.is_available():
-        torch.cuda.empty_cache()
+        for d in range(torch.cuda.device_count()):
+            if torch.cuda.memory_reserved(d):      # empty_cache() would create a context on a device never used
+                with torch.cuda.device(d):
+                    torch.cuda.empty_cache()
 
 
-def _search_engine(config, net, seed, n_games):
+_process_seed = []     # the time-based Philox key of every analysis engine built with seed=None in this process
+
+
+def _search_engine(config, net, seed, n_games, device, block):
     """main.py-style callers search move after move with the same network (reference main.py:80,145): keep the
-    analysis engine (evaluator, packed weights, tree buffers, CUDA graphs) instead of rebuilding it per call."""
-    key = (_net_identity(net), tuple(repr(getattr(config, k, None)) for k in _SEARCH_KEYS), seed, int(n_games))
+    analysis engine (evaluator, packed weights, tree buffers, CUDA graphs) instead of rebuilding it per call.
+    `block`: the index of the caller's block of positions; every block of one call has its own engine, also when
+    config.engine_devices names a device twice.  seed=None: one time-based key shared by all of them."""
+    key = (_net_identity(net), tuple(repr(getattr(config, k, None)) for k in _SEARCH_KEYS), seed, int(n_games), str(device),
+           int(block))
     eng = _cache_get(_search_engines, key, net)
     if eng is None:
         _search_engines.pop(key, None)      # a stale entry of a freed network frees its buffers before the new one
-        eng = _engine_for(config, net, n_games, seed=seed, restart_finished=False, analysis=True, root_stats=True)
-        _cache_put(_search_engines, key, net, eng)
+        if seed is None and not _process_seed:
+            _process_seed.append(_time_seed(None))
+        eng = _engine_for(config, net, n_games, seed=_process_seed[0] if seed is None else seed, device=device,
+                          restart_finished=False, analysis=True, root_stats=True)
+        _cache_put(_search_engines, key, net, eng, str(device))
     return eng
 
 
@@ -499,35 +540,49 @@ def _analyse_packed(config, recs, network, seed, search_no, strict):
     """One analysis-mode search per packed position, chunks of _ANALYSE_MAX_BATCH games stepped under CUDA graphs
     until every game has finished its own search.  -> [SearchResult or None] in input order.  strict: any device
     status bit raises (MCTS); otherwise a root without a legal move (NO_PIECE, also set for a terminal root) only
-    yields None."""
+    yields None.  config.engine_devices: the positions are split into contiguous blocks, one per device, searched
+    concurrently."""
+    from .devices import contiguous_blocks, engine_devices
     from .selfplay import CTL_DTYPE, EngineStatusError
     n = len(recs)
     if n == 0:
         return []
-    cap = _engine_batch(n)
-    eng = _search_engine(config, network, seed, cap)
+    devs = engine_devices(config)
+    # (engine, first position, end) per block with positions; no two blocks share an engine
+    jobs = [(_search_engine(config, network, seed, _engine_batch(hi - lo), dev, k), lo, hi)
+            for k, (dev, (lo, hi)) in enumerate(zip(devs, contiguous_blocks(n, len(devs)))) if hi > lo]
     long_iters, _ = config.playout_iterations()
     budget = long_iters if (config.training and config.use_playout_cap_randomization) else config.MAX_ITER
     out = [None] * n
-    for lo in range(0, n, cap):     # cap >= n unless n > _ANALYSE_MAX_BATCH
-        k = min(n, lo + cap) - lo
-        games = np.zeros(cap, dtype=GAME_DTYPE)
-        games[:k] = recs[lo:lo + k]
-        ctl = np.zeros(cap, dtype=CTL_DTYPE)
-        ctl["active"][:k] = 1
-        ctl["search_no"][:k] = search_no[lo:lo + k]
-        eng.drain()
-        eng.set_games(games)
-        eng.set_ctl(ctl)
-        eng.step(budget)      # one simulation per game and step: every search ends within the largest budget
-        if eng.get_ctl()["active"].any():
-            raise EngineStatusError("analysis engine: a search did not finish within its iteration budget")
-        samples, _ = eng.drain()
-        stats = eng.drain_root_stats()
-        eng.check_status(ignore=0 if strict else 0x4)
-        for smp, st in zip(samples, stats):
-            out[lo + int(st["slot"])] = SearchResult(smp, st)
-    return out
+    rnd = 0
+    while True:     # round r: chunk r of every block (one round unless a block exceeds _ANALYSE_MAX_BATCH)
+        live = []
+        for eng, lo, hi in jobs:
+            c0 = lo + rnd * eng.G
+            if c0 >= hi:
+                continue
+            k = min(hi, c0 + eng.G) - c0
+            games = np.zeros(eng.G, dtype=GAME_DTYPE)
+            games[:k] = recs[c0:c0 + k]
+            ctl = np.zeros(eng.G, dtype=CTL_DTYPE)
+            ctl["active"][:k] = 1
+            ctl["search_no"][:k] = search_no[c0:c0 + k]
+            eng.drain()
+            eng.set_games(games)
+            eng.set_ctl(ctl)
+            eng.step(budget)      # one simulation per game and step: every search ends within the largest budget
+            live.append((eng, c0))
+        if not live:
+            return out
+        for eng, c0 in live:
+            if eng.get_ctl()["active"].any():
+                raise EngineStatusError("analysis engine: a search did not finish within its iteration budget")
+            samples, _ = eng.drain()
+            stats = eng.drain_root_stats()
+            eng.check_status(ignore=0 if strict else 0x4)
+            for smp, st in zip(samples, stats):
+                out[c0 + int(st["slot"])] = SearchResult(smp, st)
+        rnd += 1
 
 
 def analyse(config, games, network, seed=None, game_ids=None, search_no=0):
@@ -538,7 +593,7 @@ def analyse(config, games, network, seed=None, game_ids=None, search_no=0):
     game_ids, search_no: scalars or per-position arrays keying the Philox streams of each search (playout-cap coin,
     Gamma noise, temperature choice, garbage columns) exactly as MCTS()'s game_id / search_no do.  By default a
     GAME_DTYPE array keeps the game_id of its records and Game objects are numbered 0, 1, ...
-    seed: the Philox key (None: a time-based one, as MCTS).
+    seed: the Philox key (None: a time-based one drawn once per process, shared by every block and every call).
     -> one SearchResult per position, in input order; None for a position that is already over or has no legal
     move at the root (MCTS raises there).  Any other device status raises EngineStatusError."""
     _require_pytorch(config)
@@ -565,55 +620,68 @@ def MCTS(config, game, interference_network, seed=None, game_id=0, search_no=0):
     return res.move, res, res.saved
 
 
-def _evaluator_for(network):
-    """best_evaluator of a copy of `network` in bf16 (fused trunk + heads where supported), cached per network."""
+def _evaluator_for(network, device):
+    """best_evaluator of a copy of `network` on `device` in bf16 (fused trunk + heads where supported), cached per
+    network and device.  A callable evaluator is used as given."""
     from .selfplay import best_evaluator
     if callable(network) and not isinstance(network, torch.nn.Module):
         return network
-    key = _net_identity(network)
+    key = (_net_identity(network), str(device))
     ev = _cache_get(_evaluators, key, network)
     if ev is None:
         import copy
         _evaluators.pop(key, None)
-        ev = best_evaluator(copy.deepcopy(network).to("cuda"), torch.bfloat16)
-        _cache_put(_evaluators, key, network, ev)
+        with torch.cuda.device(device):
+            ev = best_evaluator(copy.deepcopy(network).to(device), torch.bfloat16)
+        _cache_put(_evaluators, key, network, ev, str(device))
     return ev
 
 
-def _evaluate_packed(network, recs):
-    """Network outputs for packed positions: trl_encode_features (bf16) on the device, then the network's
-    best_evaluator.  -> (values float32 [n], logits float32 [n, 11583]) on the device."""
+def _evaluate_packed(network, recs, device=None):
+    """Network outputs for packed positions: trl_encode_features (bf16) on `device` (default: the current one), then
+    the network's best_evaluator there.  -> (values float32 [n], logits float32 [n, 11583]) on that device."""
     from . import _native
     from .const import POLICY_SIZE
     if not torch.cuda.is_available():
         raise RuntimeError("evaluate needs a CUDA device: the feature encoder and the network kernels run in "
                            "libtrl_b200.so (there is no CPU fallback)")
-    dev = torch.device("cuda", torch.cuda.current_device())
+    dev = torch.device("cuda", torch.cuda.current_device()) if device is None else torch.device(device)
     n = len(recs)
-    d_games = torch.from_numpy(np.ascontiguousarray(recs).view(np.uint8).reshape(-1)).to(dev)
-    grids = torch.empty((2 * n, 1, 40, 10), dtype=torch.bfloat16, device=dev)
-    extras = torch.empty((n, 105), dtype=torch.bfloat16, device=dev)
-    rc = _native.lib().trl_encode_features(d_games.data_ptr(), None, n, grids.data_ptr(), extras.data_ptr(), 1,
-                                           torch.cuda.current_stream(dev).cuda_stream)
-    _native.check(rc, "trl_encode_features")
-    with torch.no_grad():
-        values, logits = _evaluator_for(network)(grids, extras)
-    return values.reshape(-1).float(), logits[:, :POLICY_SIZE].float()
+    with torch.cuda.device(dev):
+        d_games = torch.from_numpy(np.ascontiguousarray(recs).view(np.uint8).reshape(-1)).to(dev)
+        grids = torch.empty((2 * n, 1, 40, 10), dtype=torch.bfloat16, device=dev)
+        extras = torch.empty((n, 105), dtype=torch.bfloat16, device=dev)
+        rc = _native.lib().trl_encode_features(d_games.data_ptr(), None, n, grids.data_ptr(), extras.data_ptr(), 1,
+                                               torch.cuda.current_stream(dev).cuda_stream)
+        _native.check(rc, "trl_encode_features")
+        with torch.no_grad():
+            values, logits = _evaluator_for(network, dev)(grids, extras)
+        return values.reshape(-1).float(), logits[:, :POLICY_SIZE].float()
 
 
 def evaluate_positions(config, games, network):
     """Batched evaluate(): games = a list of reference-style Game objects or a GAME_DTYPE array.
-    -> (values float32 [N], policies float32 [N, 27, 39, 11], each the softmax over all 11583 logits)."""
+    -> (values float32 [N], policies float32 [N, 27, 39, 11], each the softmax over all 11583 logits).
+    config.engine_devices: the positions are split into contiguous blocks, one per device."""
+    from .devices import contiguous_blocks, engine_devices
     _require_pytorch(config)
     recs = _pack_positions(games)
     n = len(recs)
     values = np.zeros(n, dtype=np.float32)
     policies = np.zeros((n,) + tuple(POLICY_SHAPE), dtype=np.float32)
-    for lo in range(0, n, _ANALYSE_MAX_BATCH):
-        v, logits = _evaluate_packed(network, recs[lo:lo + _ANALYSE_MAX_BATCH])
-        k = v.shape[0]
-        values[lo:lo + k] = v.cpu().numpy()
-        policies[lo:lo + k] = torch.softmax(logits, dim=1).cpu().numpy().reshape((k,) + tuple(POLICY_SHAPE))
+    devs = engine_devices(config)
+    blocks = [(dev, lo, hi) for dev, (lo, hi) in zip(devs, contiguous_blocks(n, len(devs))) if hi > lo]
+    for start in range(0, max([hi - lo for _, lo, hi in blocks], default=0), _ANALYSE_MAX_BATCH):
+        outs = []
+        for dev, lo, hi in blocks:     # queue chunk `start` of every block, then copy the results back
+            c0, c1 = lo + start, min(hi, lo + start + _ANALYSE_MAX_BATCH)
+            if c0 < c1:
+                v, logits = _evaluate_packed(network, recs[c0:c1], dev)
+                with torch.cuda.device(dev):
+                    outs.append((c0, c1, v, torch.softmax(logits, dim=1)))
+        for c0, c1, v, p in outs:
+            values[c0:c1] = v.cpu().numpy()
+            policies[c0:c1] = p.cpu().numpy().reshape((c1 - c0,) + tuple(POLICY_SHAPE))
     return values, policies
 
 

@@ -47,6 +47,13 @@ class Config:
     # None = the caller's default: make_training_set writes JSON (drop-in for the reference's trainer), self_play_loop
     # (whose trainer reads both) writes compact sets; ai.export_training_set_json turns a compact set into <n>.txt.
     engine_data_format = None
+    # B200-only knob: the devices generate_games / make_training_set, battle_networks, analyse / MCTS and
+    # evaluate_positions run on, from one process (devices.parse_engine_devices).  None = the current device, "all" =
+    # every visible device, or a list of device indices (duplicates put several engines on one device).  Games are
+    # sharded by id and positions by contiguous block; the merged results equal one device's for the fused-trunk
+    # networks (selfplay.best_evaluator), except evaluate_positions' policies (cuBLAS policy GEMM: one bf16 rounding),
+    # and are not promised bit for bit for networks on the PyTorch / cuDNN evaluator (INTEGRATION.md section 1).
+    engine_devices = None
 
     def __init__(self, **kwargs):
         unknown = set(kwargs) - set(_DEFAULTS)

@@ -1,15 +1,20 @@
 // capi.cu — library plumbing of libtrl_b200.so: version, errors, workspace.
 #include <cuda_runtime.h>
 #include <mutex>
+#include <stdio.h>
 #include <string.h>
 
 #include "trl_common.cuh"
 
 static thread_local char g_err[256] = "";
 static std::mutex g_ws_mutex;
-static void* g_ws_ptr[TRL_WS_SLOTS] = {};
-static size_t g_ws_size[TRL_WS_SLOTS] = {};
-static cudaStream_t g_host_stream[TRL_HOST_STREAMS] = {};
+// per device: workspace slots and host streams, created under that device
+struct DeviceSlots {
+    void* ws_ptr[TRL_WS_SLOTS];
+    size_t ws_size[TRL_WS_SLOTS];
+    cudaStream_t host_stream[TRL_HOST_STREAMS];
+};
+static DeviceSlots g_dev[TRL_MAX_DEVICES] = {};
 
 int trl_check(cudaError_t e) {
     if (e == cudaSuccess) return TRL_OK;
@@ -18,29 +23,45 @@ int trl_check(cudaError_t e) {
     return TRL_E_CUDA;
 }
 
+int trl_device() {
+    int dev = -1;
+    if (trl_check(cudaGetDevice(&dev)) != TRL_OK) return -1;
+    if (dev < 0 || dev >= TRL_MAX_DEVICES) {
+        snprintf(g_err, sizeof(g_err), "device %d lies past the library's per-device tables (%d entries)", dev, TRL_MAX_DEVICES);
+        return -1;
+    }
+    return dev;
+}
+
 void* trl_workspace(int slot, size_t bytes) {
     std::lock_guard<std::mutex> lock(g_ws_mutex);
     if (slot < 0 || slot >= TRL_WS_SLOTS) return nullptr;
-    if (g_ws_size[slot] >= bytes && g_ws_ptr[slot]) return g_ws_ptr[slot];
-    if (g_ws_ptr[slot]) { cudaFree(g_ws_ptr[slot]); g_ws_ptr[slot] = nullptr; g_ws_size[slot] = 0; }
+    const int dev = trl_device();
+    if (dev < 0) return nullptr;
+    void*& ptr = g_dev[dev].ws_ptr[slot];
+    size_t& size = g_dev[dev].ws_size[slot];
+    if (size >= bytes && ptr) return ptr;
+    if (ptr) { cudaFree(ptr); ptr = nullptr; size = 0; }
     void* p = nullptr;
     if (trl_check(cudaMalloc(&p, bytes)) != TRL_OK) return nullptr;
     // counters start at zero.  cudaMemset runs on the legacy default stream, which the library's non-blocking
     // streams do not wait for: without the synchronisation the memset can land AFTER the first H2D copy into
     // the new buffer (seen as wrong answers for the first calls after a re-allocation).
     if (trl_check(cudaMemset(p, 0, bytes)) != TRL_OK || trl_check(cudaDeviceSynchronize()) != TRL_OK) { cudaFree(p); return nullptr; }
-    g_ws_ptr[slot] = p;
-    g_ws_size[slot] = bytes;
+    ptr = p;
+    size = bytes;
     return p;
 }
 
 cudaStream_t trl_host_stream(int which) {
     std::lock_guard<std::mutex> lock(g_ws_mutex);
-    which &= TRL_HOST_STREAMS - 1;
-    if (!g_host_stream[which]) {
-        if (trl_check(cudaStreamCreateWithFlags(&g_host_stream[which], cudaStreamNonBlocking)) != TRL_OK) return nullptr;
+    const int dev = trl_device();
+    if (dev < 0) return nullptr;
+    cudaStream_t& s = g_dev[dev].host_stream[which & (TRL_HOST_STREAMS - 1)];
+    if (!s) {
+        if (trl_check(cudaStreamCreateWithFlags(&s, cudaStreamNonBlocking)) != TRL_OK) return nullptr;
     }
-    return g_host_stream[which];
+    return s;
 }
 
 int g_trl_pdl = 1;

@@ -217,14 +217,15 @@ static int launch_heads(const void* feats_bf16, const int32_t* own_row, const in
     if (n_leaves < 0 || !feats_bf16 || !extras_bf16 || !weights || !x_out_bf16 || !value_out_bf16) return TRL_E_ARG;
     if (n_leaves == 0) return TRL_OK;
     const int smem = (kWFloats + kWarpsPerBlock * kLeaves * (kPad + kFeat)) * 4;
-    static bool configured = false;
-    if (!configured) {
+    static bool configured[TRL_MAX_DEVICES] = {};   // the attribute is per device
+    const int dev = trl_device();
+    if (dev < 0) return TRL_E_CUDA;
+    if (!configured[dev]) {
         int rc = trl_check(cudaFuncSetAttribute(alphasame_heads_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
         if (rc) return rc;
-        configured = true;
+        configured[dev] = true;
     }
-    int dev = 0, sms = 148;
-    cudaGetDevice(&dev);
+    int sms = 148;
     cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
     int blocks = ((n_leaves + kLeaves - 1) / kLeaves + kWarpsPerBlock - 1) / kWarpsPerBlock;
     if (blocks > sms) blocks = sms;

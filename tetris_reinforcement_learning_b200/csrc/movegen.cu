@@ -360,7 +360,10 @@ extern "C" int trl_movegen_host_compact(const uint16_t* boards, const uint8_t* c
     if (!ws) return TRL_E_NOMEM;
     cudaStream_t st[TRL_HOST_STREAMS];
     for (int k = 0; k < TRL_HOST_STREAMS; ++k) if (!(st[k] = trl_host_stream(k))) return TRL_E_CUDA;
-    static unsigned long long* h_total = nullptr;   // pinned: the per-chunk totals come back through it
+    static unsigned long long* h_total_of[TRL_MAX_DEVICES] = {};   // pinned: the per-chunk totals come back through it
+    const int dev = trl_device();
+    if (dev < 0) return TRL_E_CUDA;
+    unsigned long long*& h_total = h_total_of[dev];
     if (!h_total && trl_check(cudaMallocHost(&h_total, TRL_HOST_STREAMS * sizeof(unsigned long long))) != TRL_OK) return TRL_E_CUDA;
     struct Pending { int off, m; uint16_t* d_list; bool live; } pend[TRL_HOST_STREAMS] = {};
     uint64_t base = 0;

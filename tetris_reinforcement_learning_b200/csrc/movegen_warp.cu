@@ -1868,13 +1868,42 @@ static int g_list_rounds = 1;
 extern "C" void trl_search_movegen_rounds(int rounds) { g_list_rounds = rounds < 1 ? 1 : (rounds > 16 ? 16 : rounds); }
 
 // host-side shadows of the two debug switches (the launcher must not read device symbols: that would be a
-// synchronous copy on the legacy stream at every launch)
+// synchronous copy on the legacy stream at every launch), and what each device's constant memory holds.  A switch is
+// written to the current device when it is set; the launchers bring any other device up to date before they use it.
 static int g_fast_path_host = 1, g_fifo_limit_host = kFifoCap;
+struct DeviceSwitches { int fast_path = 1, fifo_limit = kFifoCap; };   // the initialisers of c_fast_path / c_fifo_limit
+static DeviceSwitches g_dev_switches[TRL_MAX_DEVICES];
+
+static int push_switches(int dev) {
+    DeviceSwitches& d = g_dev_switches[dev];
+    int rc = TRL_OK;
+    if (d.fast_path != g_fast_path_host) {
+        rc = trl_check(cudaMemcpyToSymbol(c_fast_path, &g_fast_path_host, sizeof(int)));
+        if (!rc) d.fast_path = g_fast_path_host;
+    }
+    if (!rc && d.fifo_limit != g_fifo_limit_host) {
+        rc = trl_check(cudaMemcpyToSymbol(c_fifo_limit, &g_fifo_limit_host, sizeof(int)));
+        if (!rc) d.fifo_limit = g_fifo_limit_host;
+    }
+    return rc;
+}
+
+// Launchers: the current device's switches match the host shadows.  The copy is synchronous, so it cannot happen while
+// `stream` is being captured: a device that first meets a changed switch inside a capture fails the launch.
+static int sync_switches(int dev, cudaStream_t stream) {
+    const DeviceSwitches& d = g_dev_switches[dev];
+    if (d.fast_path == g_fast_path_host && d.fifo_limit == g_fifo_limit_host) return TRL_OK;
+    cudaStreamCaptureStatus cs = cudaStreamCaptureStatusNone;
+    int rc = trl_check(cudaStreamIsCapturing(stream, &cs));
+    if (rc) return rc;
+    if (cs != cudaStreamCaptureStatusNone) return trl_check(cudaErrorStreamCaptureUnsupported);
+    return push_switches(dev);
+}
 
 extern "C" int trl_debug_movegen_fast_path(int on) {
-    const int v = on ? 1 : 0;
-    g_fast_path_host = v;
-    return trl_check(cudaMemcpyToSymbol(c_fast_path, &v, sizeof(int)));
+    g_fast_path_host = on ? 1 : 0;
+    const int dev = trl_device();
+    return dev < 0 ? TRL_E_CUDA : push_switches(dev);
 }
 
 // answered[0] = piece searches answered by the row-parallel closure form, answered[1] = handed to the FIFO
@@ -1908,23 +1937,27 @@ extern "C" int trl_debug_movegen_t_trace(uint32_t* device_buffer, unsigned cap) 
 extern "C" int trl_debug_movegen_fifo_limit(int limit) {
     if (limit < 1 || limit > kFifoCap) limit = kFifoCap;
     g_fifo_limit_host = limit;
-    return trl_check(cudaMemcpyToSymbol(c_fifo_limit, &limit, sizeof(int)));
+    const int dev = trl_device();
+    return dev < 0 ? TRL_E_CUDA : push_switches(dev);
 }
 
 int trl_launch_movegen_listed(const TrlGame* games, const int32_t* index, const int32_t* list, uint32_t* count_done,
                               uint16_t* moves, int moves_cap, uint16_t* n_moves, TrlSearchCtl* ctl, cudaStream_t stream) {
     if (!games || !index || !list || !count_done || !moves || !n_moves || moves_cap <= 0) return TRL_E_ARG;
     const size_t smem = sizeof(PieceState) * kListSlots * 2 + sizeof(CallState) * kListSlots;
-    static int n_sm = 0;
-    if (!n_sm) {
-        int dev = 0, sms = 0;
-        int rc = trl_check(cudaGetDevice(&dev));
-        if (!rc) rc = trl_check(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
+    static int n_sm_of[TRL_MAX_DEVICES] = {};   // SM count, cached once the device's kernel attribute is set
+    const int dev = trl_device();
+    if (dev < 0) return TRL_E_CUDA;
+    if (!n_sm_of[dev]) {
+        int sms = 0;
+        int rc = trl_check(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
         if (!rc) rc = trl_check(cudaFuncSetAttribute(movegen_list_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
         if (rc) return rc;
-        n_sm = sms;
+        n_sm_of[dev] = sms;
     }
-    movegen_list_kernel<<<n_sm, kListSlots * 64, smem, stream>>>(games, index, list, count_done, moves, moves_cap, n_moves,
+    int rc = sync_switches(dev, stream);
+    if (rc) return rc;
+    movegen_list_kernel<<<n_sm_of[dev], kListSlots * 64, smem, stream>>>(games, index, list, count_done, moves, moves_cap, n_moves,
                                                                 g_list_rounds, ctl);
     return trl_check(cudaGetLastError());
 }
@@ -1935,18 +1968,20 @@ int trl_launch_movegen_listed(const TrlGame* games, const int32_t* index, const 
 static int g_form = -1;
 extern "C" void trl_movegen_warp_form(int form) { g_form = form; }
 
-// per-stream scratch of the pass form (PassLists): kCounters counters, the legacy, deferred and exact lists of n entries
-// each, then (only without a mask output) the partial masks
-struct TwoPassScratch { cudaStream_t stream; uint32_t* buf; size_t cap; bool used; };
-static TwoPassScratch g_scratch[8];
+// per-(device, stream) scratch of the pass form (PassLists): kCounters counters, the legacy, deferred and exact lists of
+// n entries each, then (only without a mask output) the partial masks.  The device is part of the key: the legacy and
+// per-thread default streams have one handle on every device.  Allocated and freed under the current device, which
+// owns `stream`.
+struct TwoPassScratch { int dev; cudaStream_t stream; uint32_t* buf; size_t cap; bool used; };
+static TwoPassScratch g_scratch[8 * 8];
 
 static std::mutex g_scratch_mutex;   // device entry points are re-entrant per stream: the table is shared
 
-static uint32_t* two_pass_scratch(cudaStream_t stream, size_t need) {
+static uint32_t* two_pass_scratch(int dev, cudaStream_t stream, size_t need) {
     std::lock_guard<std::mutex> lock(g_scratch_mutex);
     TwoPassScratch* slot = nullptr;
-    for (auto& e : g_scratch) if (e.used && e.stream == stream) { slot = &e; break; }
-    if (!slot) for (auto& e : g_scratch) if (!e.used) { slot = &e; e.used = true; e.stream = stream; e.buf = nullptr; e.cap = 0; break; }
+    for (auto& e : g_scratch) if (e.used && e.dev == dev && e.stream == stream) { slot = &e; break; }
+    if (!slot) for (auto& e : g_scratch) if (!e.used) { slot = &e; e.used = true; e.dev = dev; e.stream = stream; e.buf = nullptr; e.cap = 0; break; }
     if (!slot) return nullptr;
     if (slot->cap < need) {
         cudaStreamCaptureStatus cs = cudaStreamCaptureStatusNone;
@@ -1966,19 +2001,22 @@ extern "C" int trl_debug_movegen_partial_cap(int cap) {
     return 0;
 }
 
-// counters of the last launch of the pass form (trl_debug_movegen_pass_counts)
-static uint32_t* g_last_counts = nullptr;
-static unsigned g_last_deferred_cap = 0;
+// counters of the last launch of the pass form on each device (trl_debug_movegen_pass_counts)
+static uint32_t* g_last_counts[TRL_MAX_DEVICES] = {};
+static unsigned g_last_deferred_cap[TRL_MAX_DEVICES] = {};
 
 // counts[0] = calls whose T search pass 1 deferred (and found room), [1] = of those, calls pass 2 left to the exact T
-// search, [2] = calls on the legacy route; of the last launch of the pass form.  Synchronises the device.
+// search, [2] = calls on the legacy route; of the last launch of the pass form on the current device.  Synchronises the
+// device.
 extern "C" int trl_debug_movegen_pass_counts(uint32_t* counts) {
-    if (!counts || !g_last_counts) return TRL_E_ARG;
+    const int dev = trl_device();
+    if (dev < 0) return TRL_E_CUDA;
+    if (!counts || !g_last_counts[dev]) return TRL_E_ARG;
     uint32_t h[kCounters];
     int rc = trl_check(cudaDeviceSynchronize());
-    if (!rc) rc = trl_check(cudaMemcpy(h, g_last_counts, sizeof(h), cudaMemcpyDeviceToHost));
+    if (!rc) rc = trl_check(cudaMemcpy(h, g_last_counts[dev], sizeof(h), cudaMemcpyDeviceToHost));
     if (rc) return rc;
-    counts[0] = h[kCntDeferred] < g_last_deferred_cap ? h[kCntDeferred] : g_last_deferred_cap;
+    counts[0] = h[kCntDeferred] < g_last_deferred_cap[dev] ? h[kCntDeferred] : g_last_deferred_cap[dev];
     counts[1] = h[kCntExact];
     counts[2] = h[kCntLegacy];
     return 0;
@@ -1990,16 +2028,21 @@ int trl_launch_movegen_warp(const uint16_t* boards, const uint8_t* cur, const ui
                             uint16_t* n_moves, uint32_t* status, cudaStream_t stream, uint16_t* compact,
                             unsigned long long compact_cap, unsigned long long* compact_total,
                             unsigned long long* offsets) {
-    static int n_sm = 0, t_order_blocks = 0, t_exact_blocks = 0;   // resident blocks of passes 2 and 3 per SM
-    static bool configured = false;
+    // per device: SM count, resident blocks of passes 2 and 3 per SM, kernel attributes set
+    struct WarpConfig { int n_sm, t_order_blocks, t_exact_blocks; bool configured; };
+    static WarpConfig cfg_of[TRL_MAX_DEVICES] = {};
+    const int dev = trl_device();
+    if (dev < 0) return TRL_E_CUDA;
+    int& n_sm = cfg_of[dev].n_sm;
+    int& t_order_blocks = cfg_of[dev].t_order_blocks;
+    int& t_exact_blocks = cfg_of[dev].t_exact_blocks;
+    bool& configured = cfg_of[dev].configured;
     const size_t smem_warp = sizeof(PieceState) * kWarps + sizeof(CallState) * kCallsPerBlock;
     const size_t smem_solo = sizeof(SoloState) * kSoloWarps;
     const size_t smem_rows = sizeof(RowsWarp) * kRowsWarps;
     const size_t smem_t = sizeof(SoloState) * kTWarps;
     if (!configured) {
-        int dev = 0;
-        int rc = trl_check(cudaGetDevice(&dev));
-        if (!rc) rc = trl_check(cudaDeviceGetAttribute(&n_sm, cudaDevAttrMultiProcessorCount, dev));
+        int rc = trl_check(cudaDeviceGetAttribute(&n_sm, cudaDevAttrMultiProcessorCount, dev));
         if (!rc) rc = trl_check(cudaFuncSetAttribute(movegen_warp_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_warp));
         if (!rc) rc = trl_check(cudaFuncSetAttribute(movegen_solo_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_solo));
         if (!rc) rc = trl_check(cudaFuncSetAttribute(movegen_solo_kernel, cudaFuncAttributePreferredSharedMemoryCarveout, 100));
@@ -2018,6 +2061,10 @@ int trl_launch_movegen_warp(const uint16_t* boards, const uint8_t* cur, const ui
         if (rc) return rc;
         configured = true;
     }
+    {
+        const int rc = sync_switches(dev, stream);
+        if (rc) return rc;
+    }
     // the throughput forms once every SM is full of warps anyway (148 SMs x 32 resident warps = 4736 calls
     // in flight): below that the two-warp form halves the latency of a batch
     int form = g_form < 0 ? (n >= 3 * 4736 ? 2 : 0) : g_form;
@@ -2028,13 +2075,13 @@ int trl_launch_movegen_warp(const uint16_t* boards, const uint8_t* cur, const ui
     if (!mask_bits) deferred_cap = (unsigned)min(n, max(64 * 1024, n / 8));
     if (g_partial_cap_debug) deferred_cap = min(deferred_cap, g_partial_cap_debug);
     const size_t lists = kCounters + 3 * (size_t)n;
-    uint32_t* scratch = form == 2 ? two_pass_scratch(stream, lists + (mask_bits ? 0 : (size_t)deferred_cap * TRL_MASK_WORDS)) : nullptr;
+    uint32_t* scratch = form == 2 ? two_pass_scratch(dev, stream, lists + (mask_bits ? 0 : (size_t)deferred_cap * TRL_MASK_WORDS)) : nullptr;
     if (form == 2 && !scratch) form = 1;
     if (form == 2) {
         const PassLists pl{scratch, (int32_t*)scratch + kCounters, (int32_t*)scratch + kCounters + n,
                            (int32_t*)scratch + kCounters + 2 * (size_t)n, mask_bits ? nullptr : scratch + lists, deferred_cap};
-        g_last_counts = scratch;
-        g_last_deferred_cap = deferred_cap;
+        g_last_counts[dev] = scratch;
+        g_last_deferred_cap[dev] = deferred_cap;
         int rc = trl_check(cudaMemsetAsync(scratch, 0, kCounters * sizeof(uint32_t), stream));
         if (rc) return rc;
         const bool want_list = moves || compact;

@@ -7,12 +7,20 @@
 // Records the error text for trl_last_error(); returns TRL_OK or TRL_E_CUDA.
 int trl_check(cudaError_t e);
 
-// Library-owned, grow-only device scratch (used only by the *_host entry points and by
-// trl_movegen when the caller passes no mask buffer).  Returns nullptr on failure.
+// Every call runs on the current device.  State the library keeps between calls (workspace, host streams, kernel
+// attributes, SM counts, pushed debug switches) is kept per device, in tables of TRL_MAX_DEVICES entries.
+#define TRL_MAX_DEVICES 64
+// Index of the current device; -1 (error text set, the caller returns TRL_E_CUDA) if it cannot be read or lies past
+// the tables.
+int trl_device();
+
+// Library-owned, grow-only device scratch of the current device (used only by the *_host entry points, the trunk work
+// counters and trl_movegen when the caller passes no mask buffer).  Returns nullptr on failure.
 enum TrlWorkspaceSlot { TRL_WS_MOVEGEN_MASK = 0, TRL_WS_HOST_STAGE = 1, TRL_WS_TRUNK_COUNTER = 2, TRL_WS_TRUNK_COUNTER_TAPS = 3, TRL_WS_TRUNK_COUNTER_WIDE = 4, TRL_WS_SLOTS = 5 };
 void* trl_workspace(int slot, size_t bytes);
 
-// Streams (0 .. TRL_HOST_STREAMS - 1) used by the *_host entry points (created on first use, non-blocking).
+// Streams (0 .. TRL_HOST_STREAMS - 1) of the current device used by the *_host entry points (created on first use,
+// non-blocking).  nullptr on failure.
 #ifndef TRL_HOST_STREAMS
 #define TRL_HOST_STREAMS 4
 #endif

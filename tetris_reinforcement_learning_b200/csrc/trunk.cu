@@ -301,14 +301,15 @@ extern "C" int trl_alphasame_trunk(const void* grids_bf16, int n_images, int n_b
     if (n_images < 0 || n_blocks < 1 || n_blocks > kMaxBlocks || !grids_bf16 || !w_packed || !consts || !stem_lut || !out_bf16)
         return TRL_E_ARG;
     if (n_images == 0) return TRL_OK;
-    static bool configured = false;
-    if (!configured) {
+    static bool configured[TRL_MAX_DEVICES] = {};   // the attribute is per device
+    const int dev = trl_device();
+    if (dev < 0) return TRL_E_CUDA;
+    if (!configured[dev]) {
         int rc = trl_check(cudaFuncSetAttribute(alphasame_trunk_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBytes));
         if (rc) return rc;
-        configured = true;
+        configured[dev] = true;
     }
-    int dev = 0, sms = 148;
-    cudaGetDevice(&dev);
+    int sms = 148;
     cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
     int grid = sms * kCtasPerSm;  // resident CTAs per SM (TMEM / register bound), persistent over images
     if (grid > n_images) grid = n_images;

@@ -516,14 +516,17 @@ extern "C" int trl_alphasame_trunk_rows(const void* grids_bf16, int n_images, in
     return trl_check(cudaGetLastError());
 }
 
-static int* g_last_counter = nullptr;
-static int g_last_grid = 0;
+// the most recent trl_alphasame_trunk_rows_indexed launch of each device
+static int* g_last_counter[TRL_MAX_DEVICES] = {};
+static int g_last_grid[TRL_MAX_DEVICES] = {};
 
 // Work submitted to `stream` after this call starts only when all CTAs of the most recent
-// trl_alphasame_trunk_rows_indexed launch are resident on their SMs (or after 100 us).
+// trl_alphasame_trunk_rows_indexed launch on the current device are resident on their SMs (or after 100 us).
 extern "C" int trl_alphasame_trunk_rows_gate(void* stream) {
-    if (!g_last_counter) return TRL_E_ARG;
-    trunk_gate_kernel<<<1, 1, 0, (cudaStream_t)stream>>>(g_last_counter, g_last_grid, 100000ull);
+    const int dev = trl_device();
+    if (dev < 0) return TRL_E_CUDA;
+    if (!g_last_counter[dev]) return TRL_E_ARG;
+    trunk_gate_kernel<<<1, 1, 0, (cudaStream_t)stream>>>(g_last_counter[dev], g_last_grid[dev], 100000ull);
     return trl_check(cudaGetLastError());
 }
 
@@ -536,17 +539,18 @@ extern "C" int trl_alphasame_trunk_rows_indexed(const void* images_bf16, int32_t
     if (max_images == 0) return TRL_OK;
     const int n_lanes = lanes_for(n_blocks);
     const int smem = smem_bytes(n_blocks, n_lanes);
+    const int dev = trl_device();
+    if (dev < 0) return TRL_E_CUDA;
     int rc = trl_check(cudaFuncSetAttribute(alphasame_trunk_rows_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
     if (rc) return rc;
-    int dev = 0, sms = 148;
-    cudaGetDevice(&dev);
+    int sms = 148;
     cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
     const int n_units = ((max_images + kImgs - 1) / kImgs + n_lanes - 1) / n_lanes;
     const int grid = sms < n_units ? sms : n_units;
     int* counter = next_counter();   // zero on entry: the previous launch on this slot reset it
     if (!counter) return TRL_E_NOMEM;
-    g_last_counter = counter;
-    g_last_grid = grid;
+    g_last_counter[dev] = counter;
+    g_last_grid[dev] = grid;
     // Highest launch priority: inside a self-play step the leaf enumeration becomes ready at about the same
     // time on a forked stream, and its blocks must queue BEHIND the trunk's CTAs.  Programmatic dependent
     // launch: the CTAs move in and set themselves up while the search kernel before them drains.

@@ -611,20 +611,23 @@ template <int F, bool POST>
 int launch(const WideArgs& a, int grid, cudaStream_t stream, bool pdl) {
     int rc = trl_check(cudaFuncSetAttribute(trunk_wide_kernel<F, POST>, cudaFuncAttributeMaxDynamicSharedMemorySize, Geo<F>::kSmem));
     if (rc) return rc;
-    static size_t persist_bytes = 0, window_max = 0;
-    static bool probed = false;
-    if (!probed) {
-        probed = true;
-        int dev = 0, pmax = 0, wmax = 0;
-        if (cudaGetDevice(&dev) == cudaSuccess &&
-            cudaDeviceGetAttribute(&pmax, cudaDevAttrMaxPersistingL2CacheSize, dev) == cudaSuccess &&
+    // the persisting-L2 limit is set, and its size probed, once per device
+    static size_t persist_of[TRL_MAX_DEVICES] = {}, window_of[TRL_MAX_DEVICES] = {};
+    static bool probed[TRL_MAX_DEVICES] = {};
+    const int dev = trl_device();
+    if (dev < 0) return TRL_E_CUDA;
+    if (!probed[dev]) {
+        probed[dev] = true;
+        int pmax = 0, wmax = 0;
+        if (cudaDeviceGetAttribute(&pmax, cudaDevAttrMaxPersistingL2CacheSize, dev) == cudaSuccess &&
             cudaDeviceGetAttribute(&wmax, cudaDevAttrMaxAccessPolicyWindowSize, dev) == cudaSuccess && pmax > 0 && wmax > 0 &&
             cudaDeviceSetLimit(cudaLimitPersistingL2CacheSize, (size_t)pmax) == cudaSuccess) {
-            persist_bytes = (size_t)pmax;
-            window_max = (size_t)wmax;
+            persist_of[dev] = (size_t)pmax;
+            window_of[dev] = (size_t)wmax;
         }
         cudaGetLastError();
     }
+    const size_t persist_bytes = persist_of[dev], window_max = window_of[dev];
     cudaLaunchConfig_t cfg = {};
     cfg.gridDim = dim3(grid); cfg.blockDim = dim3(kThreads); cfg.dynamicSmemBytes = (size_t)Geo<F>::kSmem; cfg.stream = stream;
     cudaLaunchAttribute attr[3];

@@ -39,18 +39,21 @@ def env_step_host(games, moves, add_bag=True, seed=0):
 
 
 def game_setup_device(games, first_game_id=0, seed=0, id_stride=1, ruleset="s2"):
-    """games: uint8[n,400] CUDA tensor, filled in place on the current stream."""
+    """games: uint8[n,400] CUDA tensor, filled in place on the current stream of its device."""
     import torch
-    rc = _native.lib().trl_game_setup(games.data_ptr(), games.shape[0], int(first_game_id), int(id_stride), int(seed),
-                                      torch.cuda.current_stream().cuda_stream)
+    with torch.cuda.device(games.device):
+        rc = _native.lib().trl_game_setup(games.data_ptr(), games.shape[0], int(first_game_id), int(id_stride), int(seed),
+                                          torch.cuda.current_stream().cuda_stream)
     _native.check(rc, "trl_game_setup")
     games.view(games.shape[0], GAME_DTYPE.itemsize)[:, _RULESET_BYTE] = ruleset_id(ruleset)
 
 
 def env_step_device(games, moves, out=None, add_bag=True, seed=0):
-    """games uint8[n,400], moves int16/uint16[n], out uint8[n,8] | None — CUDA tensors."""
+    """games uint8[n,400], moves int16/uint16[n], out uint8[n,8] | None — CUDA tensors of one device, stepped on the
+    current stream of that device."""
     import torch
-    rc = _native.lib().trl_env_step(games.data_ptr(), moves.data_ptr(), games.shape[0],
-                                    out.data_ptr() if out is not None else None, int(bool(add_bag)),
-                                    int(seed), torch.cuda.current_stream().cuda_stream)
+    with torch.cuda.device(games.device):
+        rc = _native.lib().trl_env_step(games.data_ptr(), moves.data_ptr(), games.shape[0],
+                                        out.data_ptr() if out is not None else None, int(bool(add_bag)),
+                                        int(seed), torch.cuda.current_stream().cuda_stream)
     _native.check(rc, "trl_env_step")

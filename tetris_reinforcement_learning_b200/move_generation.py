@@ -77,7 +77,7 @@ def movegen_host_compact(boards, cur, alt, capacity=None, out=None):
 
 
 def movegen_device(boards, cur, alt, mask_bits=None, moves=None, n_moves=None, status=None):
-    """Batched movegen on torch CUDA tensors, stream-ordered on the current stream.
+    """Batched movegen on torch CUDA tensors of one device, stream-ordered on the current stream of that device.
 
     boards: uint16/int16 [n,40]; cur, alt: uint8 [n]; outputs are caller-allocated tensors
     (mask_bits int32/uint32 [n,362], moves int16/uint16 [n,cap], n_moves int16/uint16 [n],
@@ -90,8 +90,9 @@ def movegen_device(boards, cur, alt, mask_bits=None, moves=None, n_moves=None, s
             raise ValueError("movegen_device needs contiguous CUDA tensors")
     cap = moves.shape[1] if moves is not None else 0
     dp = lambda t: t.data_ptr() if t is not None else None  # noqa: E731
-    rc = _native.lib().trl_movegen(dp(boards), dp(cur), dp(alt), n, dp(mask_bits), dp(moves), cap,
-                                   dp(n_moves), dp(status), torch.cuda.current_stream().cuda_stream)
+    with torch.cuda.device(boards.device):
+        rc = _native.lib().trl_movegen(dp(boards), dp(cur), dp(alt), n, dp(mask_bits), dp(moves), cap,
+                                       dp(n_moves), dp(status), torch.cuda.current_stream().cuda_stream)
     _native.check(rc, "trl_movegen")
 
 
@@ -101,8 +102,9 @@ def movegen_games_device(games, mask_bits=None, moves=None, n_moves=None, status
     n = games.shape[0]
     cap = moves.shape[1] if moves is not None else 0
     dp = lambda t: t.data_ptr() if t is not None else None  # noqa: E731
-    rc = _native.lib().trl_movegen_games(dp(games), n, dp(mask_bits), dp(moves), cap, dp(n_moves),
-                                         dp(status), torch.cuda.current_stream().cuda_stream)
+    with torch.cuda.device(games.device):
+        rc = _native.lib().trl_movegen_games(dp(games), n, dp(mask_bits), dp(moves), cap, dp(n_moves),
+                                             dp(status), torch.cuda.current_stream().cuda_stream)
     _native.check(rc, "trl_movegen_games")
 
 

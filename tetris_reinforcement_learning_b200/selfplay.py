@@ -17,6 +17,7 @@ post-prune visit counts) and finished games `TrlGameEnd` records in HBM ring buf
 drains between graph replays (drain(): pinned, double-buffered).
 """
 import ctypes
+import functools
 
 import numpy as np
 import torch
@@ -117,8 +118,18 @@ def search_params_from_config(config, seed=0, restart_finished=True, game_id_str
     return p
 
 
+def _on_device(method):
+    """Run an engine method with the engine's device current: the library launches on, and allocates for, the current
+    device, and graph capture takes its stream from it.  An engine on cuda:1 then works while cuda:0 is current."""
+    @functools.wraps(method)
+    def run(self, *args, **kwargs):
+        with torch.cuda.device(self.device):
+            return method(self, *args, **kwargs)
+    return run
+
+
 class SelfPlayEngine:
-    """G concurrent self-play games on one GPU.
+    """G concurrent self-play games on one GPU (`device`; every method runs with it current).
 
     evaluator(grids [2G,1,40,10], extras [G,105]) -> (values [G] or [G,1], logits [G,11583]);
     tensors of `feature_dtype` in, float32 or bfloat16 out.  Normally a network's
@@ -228,6 +239,7 @@ class SelfPlayEngine:
         self.new_games(first_game_id, game_id_stride)
 
     # ---- state access -----------------------------------------------------------------
+    @_on_device
     def new_games(self, first_game_id=0, stride=1):
         """Fresh Game.setup() in every slot; ids first, first+stride, ..."""
         games = self.t["games"].view(self.G, 400)
@@ -253,22 +265,27 @@ class SelfPlayEngine:
         if getattr(self, "_cache_bufs", None) is not None:
             self._cache_bufs["count"].zero_()    # images queued by a fused encode of the stale selection
 
+    @_on_device
     def set_games(self, games_np):
         assert games_np.dtype == GAME_DTYPE and games_np.shape == (self.G,)
         self.t["games"].copy_(torch.from_numpy(np.ascontiguousarray(games_np).view(np.uint8).reshape(-1)).to(self.device))
         self._invalidate_selection()
 
+    @_on_device
     def get_games(self):
         return self.t["games"].cpu().numpy().view(GAME_DTYPE).reshape(-1)
 
+    @_on_device
     def set_ctl(self, ctl_np):
         assert ctl_np.dtype == CTL_DTYPE and ctl_np.shape == (self.G,)
         self.t["ctl"].copy_(torch.from_numpy(np.ascontiguousarray(ctl_np).view(np.uint8).reshape(-1)).to(self.device))
         self._invalidate_selection()
 
+    @_on_device
     def get_ctl(self):
         return self.t["ctl"].cpu().numpy().view(CTL_DTYPE).reshape(-1)
 
+    @_on_device
     def set_noise_override(self, noise):
         """noise: float64 [G, moves_cap] Gamma draws used instead of the in-kernel sampler (tests)."""
         self.noise_override = torch.as_tensor(noise, dtype=torch.float64, device=self.device).contiguous()
@@ -374,6 +391,7 @@ class SelfPlayEngine:
         self._encoded = self.fuse_encode
         stamp(6, st)
 
+    @_on_device
     def enable_timeline(self):
         """Profiling: %globaltimer stamps between the kernels of a step (slots: 0 start, 1 after select,
         2 after encode, 3 after trunk, 4 after heads, 5 after policy GEMM, 6 after expand(+select), 8/9 around
@@ -388,6 +406,7 @@ class SelfPlayEngine:
         if self._stamps is not None:
             _native.check(self.lib.trl_stamp_globaltimer(self._stamps.data_ptr() + 8 * k, stream), "trl_stamp_globaltimer")
 
+    @_on_device
     def step(self, n=1):
         """Advance every game by n simulations."""
         if not self.use_cuda_graph:
@@ -434,6 +453,7 @@ class SelfPlayEngine:
             self._graph.replay()
 
     # ---- outputs ----------------------------------------------------------------------------
+    @_on_device
     def drain(self, copy=True):
         """-> (samples SAMPLE_DTYPE[k], game_ends GAME_END_DTYPE[m]) accumulated since the last drain.
 
@@ -476,6 +496,7 @@ class SelfPlayEngine:
         """OR of the sticky TRL_ST_* bits of all games (0 = clean)."""
         return int(np.bitwise_or.reduce(self.get_ctl()["status"])) if self.G else 0
 
+    @_on_device
     def check_status(self, ignore=0):
         """Raise EngineStatusError if any game carries a status bit outside `ignore`."""
         st = self.get_ctl()["status"]

@@ -301,6 +301,12 @@ class DualCachedEvaluator:
 
     def __call__(self, b, states, leaf_state, leaf_parent, extras, after_trunk=None, before_trunk=None, encoded=False,
                  search_buffers=None, join_movegen=None):
+        with torch.cuda.device(extras.device):
+            return self._evaluate(b, states, leaf_state, leaf_parent, extras, after_trunk, before_trunk, encoded,
+                                  search_buffers, join_movegen)
+
+    def _evaluate(self, b, states, leaf_state, leaf_parent, extras, after_trunk, before_trunk, encoded, search_buffers,
+                  join_movegen):
         G = leaf_state.numel()
         if not encoded:
             self.encode(b, states, leaf_state, leaf_parent, extras)
@@ -332,31 +338,22 @@ class DualCachedEvaluator:
         return torch.where(use2, v2, v1), torch.where(use2[:, None], l2, l1)
 
 
-def battle_networks(NN_1, config_1, NN_2, config_2, threshold, threshold_type, games,
-                    network_1_title="Network 1", network_2_title="Network 2", screen=None, seed=None,
-                    first_game_id=0, game_id_stride=1):
-    """All `games` battles run concurrently on the GPU (the reference's batched variant, ai.py:2071-2114: network 1
-    plays player (game index & 1), no early termination, post-hoc threshold).  Every search runs with the network AND
-    the search settings (config_1 / config_2) of the side to move at the root (ai.py:2012-2016); the two configs may
-    differ in anything but the ruleset.  No random opening plies (ai.py:1588-1608 is play_game only).
-    first_game_id / game_id_stride shard the battles over ranks (ids first, first + stride, ...)."""
+def _battle_engine(NN_1, config_1, NN_2, config_2, n_games, seed, device, first_game_id, game_id_stride):
+    """The engine of one shard of a gating battle on `device`: both networks' evaluators there, one engine sized for the
+    larger of the two search budgets, the per-search settings of either side in params2.  -> (engine, params2)."""
     from .ai import _engine_for
     import copy
-    import ctypes
     from . import _native
     from .selfplay import best_evaluator, search_params_from_config
-    if config_1.ruleset != config_2.ruleset:
-        raise NotImplementedError("Ruleset's aren't equal")
-    dev = torch.device("cuda", torch.cuda.current_device())
 
     def as_evaluator(nn_):
         if callable(nn_) and not isinstance(nn_, torch.nn.Module):
             return nn_
-        return best_evaluator(copy.deepcopy(nn_).to(dev), torch.bfloat16)
+        with torch.cuda.device(device):
+            return best_evaluator(copy.deepcopy(nn_).to(device), torch.bfloat16)
 
     ev1, ev2 = as_evaluator(NN_1), as_evaluator(NN_2)
     both_cached = getattr(ev1, "cached", None) is not None and getattr(ev2, "cached", None) is not None
-    holder = {}
     if both_cached:
         evaluator = lambda grids, extras: ev1(grids, extras)      # noqa: E731  (never called: the engine uses .cached)
         evaluator.cached = DualCachedEvaluator(ev1.cached, ev2.cached)
@@ -371,8 +368,8 @@ def battle_networks(NN_1, config_1, NN_2, config_2, threshold, threshold_type, g
     # the engine is sized for the larger of the two search budgets; the per-search settings come from params2
     big = config_1 if max(config_1.playout_iterations()[0], config_1.MAX_ITER) >= max(config_2.playout_iterations()[0], config_2.MAX_ITER) \
         else config_2
-    eng = _engine_for(big, evaluator, games, seed=seed, restart_finished=False, dtype=dtype, first_game_id=first_game_id,
-                      game_id_stride=game_id_stride)
+    eng = _engine_for(big, evaluator, n_games, seed=seed, device=device, restart_finished=False, dtype=dtype,
+                      first_game_id=first_game_id, game_id_stride=game_id_stride)
     if both_cached:
         evaluator.cached.engine = eng
     else:
@@ -383,14 +380,39 @@ def battle_networks(NN_1, config_1, NN_2, config_2, threshold, threshold_type, g
                                       search_params_from_config(config_2, eng.seed, False, game_id_stride))
     for p in pair:
         p.seed = eng.seed
-    params2 = torch.frombuffer(bytearray(bytes(pair)), dtype=torch.uint8).to(dev)
+    params2 = torch.frombuffer(bytearray(bytes(pair)), dtype=torch.uint8).to(device)
     eng.buf.params2 = params2.data_ptr()
-    holder["params2"] = params2
+    return eng, params2
+
+
+def battle_networks(NN_1, config_1, NN_2, config_2, threshold, threshold_type, games,
+                    network_1_title="Network 1", network_2_title="Network 2", screen=None, seed=None,
+                    first_game_id=0, game_id_stride=1):
+    """All `games` battles run concurrently on the GPU (the reference's batched variant, ai.py:2071-2114: network 1
+    plays player (game index & 1), no early termination, post-hoc threshold).  Every search runs with the network AND
+    the search settings (config_1 / config_2) of the side to move at the root (ai.py:2012-2016); the two configs may
+    differ in anything but the ruleset.  No random opening plies (ai.py:1588-1608 is play_game only).
+    first_game_id / game_id_stride shard the battles over ranks (ids first, first + stride, ...).
+    config_1.engine_devices: the battles are further sharded by id over those devices (devices.shard_games), all
+    engines stepped from this thread; the tallies are summed and the threshold applies to the merged tally."""
+    from .ai import _time_seed
+    from .devices import engine_devices, shard_games
+    if config_1.ruleset != config_2.ruleset:
+        raise NotImplementedError("Ruleset's aren't equal")
+    seed = _time_seed(seed)      # one key for every shard
+    devs = engine_devices(config_1)
+    shards = [_battle_engine(NN_1, config_1, NN_2, config_2, sh["num_games"], seed, devs[sh["shard"]], sh["first_game_id"],
+                             sh["game_id_stride"])
+              for sh in shard_games(games, games, first_game_id, game_id_stride, len(devs))]
     ends = []
     chunk = max(8, min(config_1.MAX_ITER, config_2.MAX_ITER))
-    while eng.get_ctl()["active"].any():
-        eng.step(chunk)
-        ends.extend(eng.drain()[1])
-        eng.check_status(ignore=0x20)        # sample records are not read here: a full sample ring is harmless
+    running = [eng for eng, _ in shards]
+    while running:
+        for eng in running:     # queue every engine's graphs before the first drain waits for its device
+            eng.step(chunk)
+        for eng in running:
+            ends.extend(eng.drain()[1])
+            eng.check_status(ignore=0x20)        # sample records are not read here: a full sample ring is harmless
+        running = [eng for eng in running if eng.get_ctl()["active"].any()]
     wins = tally_battle_results((int(e["winner"]), int(e["game_id"]) % 2) for e in ends)
     return wins, _check_threshold(wins, games, threshold, threshold_type)

@@ -93,8 +93,9 @@ def trunk_forward(packed, grids, out=None):
     fn = _native.lib().trl_alphasame_trunk_rows if rows else _native.lib().trl_alphasame_trunk
     stem = packed["stem_w"] if rows else packed["stem_lut"]
     consts = packed["consts_host"] if rows else packed["consts"]   # rows kernel: by-value kernel parameter
-    rc = fn(grids.data_ptr(), n, packed["n_blocks"], packed["w_packed"].data_ptr(), consts.data_ptr(),
-            stem.data_ptr(), out.data_ptr(), torch.cuda.current_stream(grids.device).cuda_stream)
+    with torch.cuda.device(grids.device):   # the library launches on the current device
+        rc = fn(grids.data_ptr(), n, packed["n_blocks"], packed["w_packed"].data_ptr(), consts.data_ptr(),
+                stem.data_ptr(), out.data_ptr(), torch.cuda.current_stream(grids.device).cuda_stream)
     _native.check(rc, "trl_alphasame_trunk")
     return out
 
@@ -153,8 +154,9 @@ def make_fused_evaluator(net, dtype=torch.bfloat16, layout=None, fused_heads=Tru
             value = torch.empty(b, dtype=dtype, device=extras.device)
             if extras.dtype != dtype or not extras.is_contiguous():
                 extras = extras.to(dtype).contiguous()
-            rc = lib.trl_alphasame_heads(feats.data_ptr(), extras.data_ptr(), b, w_heads.data_ptr(), use_tanh,
-                                         x.data_ptr(), value.data_ptr(), torch.cuda.current_stream(extras.device).cuda_stream)
+            with torch.cuda.device(extras.device):
+                rc = lib.trl_alphasame_heads(feats.data_ptr(), extras.data_ptr(), b, w_heads.data_ptr(), use_tanh,
+                                             x.data_ptr(), value.data_ptr(), torch.cuda.current_stream(extras.device).cuda_stream)
             _native.check(rc, "trl_alphasame_heads")
             return value, torch.nn.functional.linear(x, w_pol, b_pol)   # logits [G, 11584], last column unused
     else:
@@ -182,7 +184,8 @@ class CachedTrunkEvaluator:
     """Network evaluation for SelfPlayEngine with exact trunk-feature reuse (include/trl.h,
     trl_encode_features_cached): per simulation only the board that the last move changed goes
     through the trunk; the features of the other board are the parent state's.  Outputs are
-    bit-identical to the plain fused evaluator (same kernels, same per-image arithmetic)."""
+    bit-identical to the plain fused evaluator (same kernels, same per-image arithmetic).
+    Every library call runs on the device of the buffers it is handed."""
 
     gather_policy = True   # policy head on the legal moves only (trl_search_policy_legal) instead of the dense GEMM
 
@@ -207,36 +210,40 @@ class CachedTrunkEvaluator:
         if self.gather_policy and search_buffers is not None:
             if join_movegen is not None:
                 join_movegen()      # the legal lists of this step come from the forked enumeration
-            _native.check(_native.lib().trl_search_policy_legal(
-                search_buffers, b["x"].data_ptr(), self.k_pad, self.w_pol.data_ptr(), self.b_pol.data_ptr(),
-                b["logits_legal"].data_ptr(), torch.cuda.current_stream(b["x"].device).cuda_stream), "trl_search_policy_legal")
+            with torch.cuda.device(b["x"].device):
+                _native.check(_native.lib().trl_search_policy_legal(
+                    search_buffers, b["x"].data_ptr(), self.k_pad, self.w_pol.data_ptr(), self.b_pol.data_ptr(),
+                    b["logits_legal"].data_ptr(), torch.cuda.current_stream(b["x"].device).cuda_stream), "trl_search_policy_legal")
             return b["logits_legal"]
         return torch.nn.functional.linear(b["x"], self.w_pol, self.b_pol)
 
     def trunk_step(self, b, G):
         """Trunk over the queued images b["images"][: b["count"]] -> cache rows b["dest"] (resets the count)."""
         p = self.packed
-        _native.check(_native.lib().trl_alphasame_trunk_rows_indexed(
-            b["images"].data_ptr(), b["count"].data_ptr(), 2 * G, b["dest"].data_ptr(), p["n_blocks"],
-            p["w_packed"].data_ptr(), p["consts_host"].data_ptr(), p["stem_w"].data_ptr(), b["cache"].data_ptr(),
-            torch.cuda.current_stream(b["cache"].device).cuda_stream), "trl_alphasame_trunk_rows_indexed")
+        with torch.cuda.device(b["cache"].device):
+            _native.check(_native.lib().trl_alphasame_trunk_rows_indexed(
+                b["images"].data_ptr(), b["count"].data_ptr(), 2 * G, b["dest"].data_ptr(), p["n_blocks"],
+                p["w_packed"].data_ptr(), p["consts_host"].data_ptr(), p["stem_w"].data_ptr(), b["cache"].data_ptr(),
+                torch.cuda.current_stream(b["cache"].device).cuda_stream), "trl_alphasame_trunk_rows_indexed")
 
     def heads_step(self, b, extras, G):
         """Opponent summary, head input b["x"] and value b["value"] of the leaves whose b["own"] row is >= 0."""
-        _native.check(_native.lib().trl_alphasame_heads_indexed(
-            b["cache"].data_ptr(), b["own"].data_ptr(), b["opp"].data_ptr(), extras.data_ptr(), G,
-            self.w_heads.data_ptr(), self.use_tanh, b["x"].data_ptr(), b["value"].data_ptr(),
-            torch.cuda.current_stream(extras.device).cuda_stream), "trl_alphasame_heads_indexed")
+        with torch.cuda.device(extras.device):
+            _native.check(_native.lib().trl_alphasame_heads_indexed(
+                b["cache"].data_ptr(), b["own"].data_ptr(), b["opp"].data_ptr(), extras.data_ptr(), G,
+                self.w_heads.data_ptr(), self.use_tanh, b["x"].data_ptr(), b["value"].data_ptr(),
+                torch.cuda.current_stream(extras.device).cuda_stream), "trl_alphasame_heads_indexed")
         return b["value"]
 
     def encode(self, b, states, leaf_state, leaf_parent, extras):
         """Feature encoding of the selected leaves (a separate kernel; the engine normally has it done by
         the fused expand + select + encode kernel of the previous step)."""
         st = torch.cuda.current_stream(extras.device).cuda_stream   # b["count"] is zero here: the trunk kernel resets it
-        _native.check(_native.lib().trl_encode_features_cached(
-            states.data_ptr(), leaf_state.data_ptr(), leaf_parent.data_ptr(), leaf_state.numel(), b["cache"].data_ptr(),
-            b["images"].data_ptr(), b["dest"].data_ptr(), b["count"].data_ptr(), extras.data_ptr(),
-            b["own"].data_ptr(), b["opp"].data_ptr(), b["rowof"].data_ptr(), st), "trl_encode_features_cached")
+        with torch.cuda.device(extras.device):
+            _native.check(_native.lib().trl_encode_features_cached(
+                states.data_ptr(), leaf_state.data_ptr(), leaf_parent.data_ptr(), leaf_state.numel(), b["cache"].data_ptr(),
+                b["images"].data_ptr(), b["dest"].data_ptr(), b["count"].data_ptr(), extras.data_ptr(),
+                b["own"].data_ptr(), b["opp"].data_ptr(), b["rowof"].data_ptr(), st), "trl_encode_features_cached")
 
     def __call__(self, b, states, leaf_state, leaf_parent, extras, after_trunk=None, before_trunk=None, encoded=False,
                  search_buffers=None, join_movegen=None):

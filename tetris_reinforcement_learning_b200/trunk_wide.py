@@ -119,12 +119,13 @@ class WideTrunk:
         """images bf16 [>= n][400] -> out bf16 [rows][n_out * 400] (row k, or out_row[k] with a device count)."""
         p = self.p
         n = images.numel() // CELLS if n_images is None else int(n_images)
-        rc = _native.lib().trl_trunk_wide(
-            images.data_ptr(), n, n_images_dev.data_ptr() if n_images_dev is not None else None,
-            out_row.data_ptr() if out_row is not None else None, p["filters"], p["n_blocks"], p["post_act"], p["stem_taps"],
-            p["w_packed"].data_ptr(), p["consts"].data_ptr(), p["stem_lut"].data_ptr(), out.data_ptr(),
-            self.scratch.data_ptr(), self.scratch.numel(), self.status.data_ptr(), int(bool(pdl)),
-            torch.cuda.current_stream(self.device).cuda_stream)
+        with torch.cuda.device(self.device):    # the library launches on the current device
+            rc = _native.lib().trl_trunk_wide(
+                images.data_ptr(), n, n_images_dev.data_ptr() if n_images_dev is not None else None,
+                out_row.data_ptr() if out_row is not None else None, p["filters"], p["n_blocks"], p["post_act"], p["stem_taps"],
+                p["w_packed"].data_ptr(), p["consts"].data_ptr(), p["stem_lut"].data_ptr(), out.data_ptr(),
+                self.scratch.data_ptr(), self.scratch.numel(), self.status.data_ptr(), int(bool(pdl)),
+                torch.cuda.current_stream(self.device).cuda_stream)
         _native.check(rc, "trl_trunk_wide")
         return out
 
@@ -229,14 +230,17 @@ def make_wide_evaluator(net, dtype=torch.bfloat16):
             value = torch.empty(b, dtype=dtype, device=extras.device)
             if extras.dtype != dtype or not extras.is_contiguous():
                 extras = extras.to(dtype).contiguous()
-            _native.check(lib.trl_alphasame_heads(feats.data_ptr(), extras.data_ptr(), b, w_heads.data_ptr(), use_tanh, x.data_ptr(),
-                                                  value.data_ptr(), torch.cuda.current_stream(extras.device).cuda_stream), "trl_alphasame_heads")
+            with torch.cuda.device(extras.device):
+                _native.check(lib.trl_alphasame_heads(feats.data_ptr(), extras.data_ptr(), b, w_heads.data_ptr(), use_tanh,
+                                                      x.data_ptr(), value.data_ptr(), torch.cuda.current_stream(extras.device).cuda_stream),
+                              "trl_alphasame_heads")
             return value, torch.nn.functional.linear(x, w_pol, b_pol)
 
         def heads_indexed(b, extras, G, st):
-            _native.check(lib.trl_alphasame_heads_indexed(
-                b["cache"].data_ptr(), b["own"].data_ptr(), b["opp"].data_ptr(), extras.data_ptr(), G,
-                w_heads.data_ptr(), use_tanh, b["x"].data_ptr(), b["value"].data_ptr(), st), "trl_alphasame_heads_indexed")
+            with torch.cuda.device(extras.device):
+                _native.check(lib.trl_alphasame_heads_indexed(
+                    b["cache"].data_ptr(), b["own"].data_ptr(), b["opp"].data_ptr(), extras.data_ptr(), G,
+                    w_heads.data_ptr(), use_tanh, b["x"].data_ptr(), b["value"].data_ptr(), st), "trl_alphasame_heads_indexed")
             return b["value"]
     else:
         heads = BaseResNetHeads(net, dtype)
@@ -263,7 +267,8 @@ def make_wide_evaluator(net, dtype=torch.bfloat16):
 
 class CachedWideEvaluator:
     """trunk.CachedTrunkEvaluator for the wide nets (same engine contract: make_buffers / encode / __call__):
-    per simulation only the board the last move changed goes through the trunk (exact, include/trl.h)."""
+    per simulation only the board the last move changed goes through the trunk (exact, include/trl.h).  Every library
+    call runs on the device of the buffers it is handed."""
 
     overlap_mode = "heads"     # the leaf enumeration is forked after the trunk (its CTAs own the SMs)
     gather_policy = True       # policy head on the legal moves only (trl_search_policy_legal)
@@ -291,10 +296,11 @@ class CachedWideEvaluator:
 
     def encode(self, b, states, leaf_state, leaf_parent, extras):
         st = torch.cuda.current_stream(extras.device).cuda_stream
-        _native.check(_native.lib().trl_encode_features_cached(
-            states.data_ptr(), leaf_state.data_ptr(), leaf_parent.data_ptr(), leaf_state.numel(), b["cache"].data_ptr(),
-            b["images"].data_ptr(), b["dest"].data_ptr(), b["count"].data_ptr(), extras.data_ptr(),
-            b["own"].data_ptr(), b["opp"].data_ptr(), b["rowof"].data_ptr(), st), "trl_encode_features_cached")
+        with torch.cuda.device(extras.device):
+            _native.check(_native.lib().trl_encode_features_cached(
+                states.data_ptr(), leaf_state.data_ptr(), leaf_parent.data_ptr(), leaf_state.numel(), b["cache"].data_ptr(),
+                b["images"].data_ptr(), b["dest"].data_ptr(), b["count"].data_ptr(), extras.data_ptr(),
+                b["own"].data_ptr(), b["opp"].data_ptr(), b["rowof"].data_ptr(), st), "trl_encode_features_cached")
 
     def __call__(self, b, states, leaf_state, leaf_parent, extras, after_trunk=None, before_trunk=None, encoded=False,
                  search_buffers=None, join_movegen=None):
