@@ -181,6 +181,43 @@ int trl_movegen_host_compact(const uint16_t* boards, const uint8_t* cur, const u
                              uint16_t* moves_compact, uint64_t capacity, uint64_t* offsets,
                              uint16_t* n_moves, uint32_t* status, uint64_t* total_out);
 
+/*
+ * Host movegen over SHARED boards with byte-coded move lists.  Each distinct board crosses PCIe once:
+ * call i enumerates boards[board_index[i]] with cur[i] / alt[i] (so "every piece on each board" needs
+ * no copies of the board), and its ascending move list (np.argwhere order) comes back as about 1 B
+ * per placement.
+ *
+ * boards      [n_boards][40] uint16   the distinct boards
+ * board_index [n]  uint32             board of call i; an index >= n_boards reads nothing and the call
+ *                                     returns TRL_E_ARG once the run has finished (checked on the device)
+ * cur, alt    [n]  uint8              as in trl_movegen
+ * codes       [codes_cap] uint8       OUT, *codes_total bytes written
+ * escapes     [esc_cap]  uint16       OUT, *esc_total entries written
+ * n_moves     [n]  uint16             OUT number of placements of each call
+ * flag_index, flag_status [flag_cap] uint32  OUT, *n_flagged entries: the calls whose TRL_ST_* word is
+ *                                     not zero, as (call index, status) in ascending call index; every
+ *                                     other call has status 0
+ *
+ * Format.  Calls are encoded in call order into the two shared streams.  For each move m of call i let
+ * prev be the call's previous move (-1 before its first) and d = m - prev, 1 <= d <= 11583:
+ *     d <= 255:  byte d is appended to codes
+ *     d >  255:  byte 0 is appended to codes and d (uint16) to escapes
+ * A call has at most 45 escapes.  Decoding needs no per-call loop (numpy):
+ *     d = codes.astype(int64); d[codes == 0] = escapes
+ *     cs = cumsum(d); start = cumsum(n_moves) - n_moves
+ *     moves = cs - repeat(where(start > 0, cs[start - 1], 0), n_moves) - 1
+ * (move_generation.decode_move_codes).  The bytes depend on the input alone, not on the run.
+ *
+ * TRL_E_ARG: a NULL pointer, n < 0, n > 0 with n_boards <= 0, a board index out of range, an output
+ * buffer too small, or a chunk of 131072 calls averaging more than 512 placements per call (the
+ * device staging).  Runs on the current device and returns when every output has landed.
+ */
+int trl_movegen_host_boards(const uint16_t* boards, int n_boards, const uint32_t* board_index,
+                            const uint8_t* cur, const uint8_t* alt, int n, uint8_t* codes,
+                            uint64_t codes_cap, uint16_t* escapes, uint64_t esc_cap, uint16_t* n_moves,
+                            uint32_t* flag_index, uint32_t* flag_status, uint64_t flag_cap,
+                            uint64_t* codes_total, uint64_t* esc_total, uint64_t* n_flagged);
+
 /* Kernel used by every trl_movegen* entry point: 0 = one thread per call (csrc/movegen.cu),
  * 1 = one warp per piece search (csrc/movegen_warp.cu), -1 = automatic (default).  Both produce
  * bit-identical outputs; the choice only trades latency against throughput. */

@@ -29,6 +29,8 @@ SIGNATURES = {
     "trl_movegen_host": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_void_p, c_void_p, c_int,
                                  c_void_p, c_void_p]),
     "trl_movegen_host_compact": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_void_p, c_u64, c_void_p, c_void_p, c_void_p, c_void_p]),
+    "trl_movegen_host_boards": (c_int, [c_void_p, c_int, c_void_p, c_void_p, c_void_p, c_int, c_void_p, c_u64, c_void_p,
+                                        c_u64, c_void_p, c_void_p, c_void_p, c_u64, c_void_p, c_void_p, c_void_p]),
     "trl_movegen_select_kernel": (None, [c_int]),
     "trl_movegen_warp_form": (None, [c_int]),
     "trl_search_movegen_rounds": (None, [c_int]),

@@ -16,7 +16,7 @@ int trl_device();
 
 // Library-owned, grow-only device scratch of the current device (used only by the *_host entry points, the trunk work
 // counters and trl_movegen when the caller passes no mask buffer).  Returns nullptr on failure.
-enum TrlWorkspaceSlot { TRL_WS_MOVEGEN_MASK = 0, TRL_WS_HOST_STAGE = 1, TRL_WS_TRUNK_COUNTER = 2, TRL_WS_TRUNK_COUNTER_TAPS = 3, TRL_WS_TRUNK_COUNTER_WIDE = 4, TRL_WS_SLOTS = 5 };
+enum TrlWorkspaceSlot { TRL_WS_MOVEGEN_MASK = 0, TRL_WS_HOST_STAGE = 1, TRL_WS_TRUNK_COUNTER = 2, TRL_WS_TRUNK_COUNTER_TAPS = 3, TRL_WS_TRUNK_COUNTER_WIDE = 4, TRL_WS_HOST_BOARDS = 5, TRL_WS_SLOTS = 6 };
 void* trl_workspace(int slot, size_t bytes);
 
 // Streams (0 .. TRL_HOST_STREAMS - 1) of the current device used by the *_host entry points (created on first use,

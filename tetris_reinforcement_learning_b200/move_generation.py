@@ -76,6 +76,90 @@ def movegen_host_compact(boards, cur, alt, capacity=None, out=None):
     return {"moves": moves, "offsets": offsets, "n_moves": n_moves, "status": status, "total": int(total.value)}
 
 
+def decode_move_codes(codes, escapes, n_moves):
+    """Byte-coded move lists of trl_movegen_host_boards (format in include/trl.h) -> (moves uint16[total],
+    offsets uint64[n]): call i's ascending list is moves[offsets[i] : offsets[i] + n_moves[i]].  No per-call loop."""
+    codes = np.asarray(codes, dtype=np.uint8)
+    n_moves = np.asarray(n_moves)
+    counts = n_moves.astype(np.int64)
+    start = np.cumsum(counts) - counts
+    if codes.size != counts.sum():
+        raise ValueError(f"{codes.size} codes for {int(counts.sum())} moves")
+    d = codes.astype(np.int64)
+    zero = codes == 0
+    if int(zero.sum()) != np.asarray(escapes).size:
+        raise ValueError(f"{int(zero.sum())} escape codes for {np.asarray(escapes).size} escapes")
+    d[zero] = escapes
+    cs = np.cumsum(d)
+    if cs.size == 0:
+        return np.empty(0, dtype=np.uint16), start.astype(np.uint64)
+    moves = cs - np.repeat(np.where(start > 0, cs[start - 1], 0), counts) - 1
+    return moves.astype(np.uint16), start.astype(np.uint64)
+
+
+def movegen_host_boards(boards, board_index, cur, alt, decode=True, out=None):
+    """Batched movegen on HOST buffers over shared boards (trl_movegen_host_boards): call i enumerates
+    boards[board_index[i]] with cur[i] / alt[i], and each board crosses PCIe once.
+
+    boards uint16[n_boards,40]; board_index uint32[n] (< n_boards); cur, alt uint8[n] (255 = none).
+    decode=True -> the keys of movegen_host_compact: moves uint16[total], offsets uint64[n], n_moves
+    uint16[n], status uint32[n] (dense) and total.
+    decode=False -> the raw streams: codes uint8, escapes uint16, n_moves uint16[n], and the flagged calls
+    flag_index / flag_status uint32 (calls with a non-zero TRL_ST_* word, ascending).
+    `out` may carry preallocated (pinned) numpy arrays under the keys codes, escapes, n_moves, flag_index
+    and flag_status; their sizes are the capacities."""
+    import ctypes
+    boards = np.ascontiguousarray(boards, dtype=np.uint16)
+    board_index = np.asarray(board_index)
+    if board_index.dtype.kind not in "iu":
+        raise ValueError("board_index must be an integer array")
+    if board_index.dtype.itemsize > 4 and board_index.size and \
+            (board_index.min() < 0 or board_index.max() > np.iinfo(np.uint32).max):
+        raise ValueError("board_index out of range")   # would wrap into a valid index as uint32
+    # (a negative int32 index becomes >= 2^31 > n_boards, which the device rejects)
+    board_index = np.ascontiguousarray(board_index, dtype=np.uint32)
+    cur = np.ascontiguousarray(cur, dtype=np.uint8)
+    alt = np.ascontiguousarray(alt, dtype=np.uint8)
+    n_boards, n = boards.shape[0], board_index.shape[0]
+    if boards.shape != (n_boards, ROWS) or board_index.shape != (n,) or cur.shape != (n,) or alt.shape != (n,):
+        raise ValueError("expected boards[n_boards,40], board_index[n], cur[n], alt[n]")
+    out = out or {}
+
+    def buf(key, size, dtype):
+        a = out.get(key, None)
+        if a is None:
+            return np.empty(size, dtype=dtype)
+        if a.dtype != dtype or a.ndim != 1 or not a.flags.c_contiguous:
+            raise ValueError(f"out[{key!r}] must be a contiguous 1-D {np.dtype(dtype).name} array")
+        return a
+
+    # default capacities: the device staging's 512 codes per call, and the exact bounds of 45 escapes per call
+    # (each spans >= 256 of the 11583 indices) and one flag per call
+    codes = buf("codes", max(1024, 512 * n), np.uint8)
+    escapes = buf("escapes", max(64, 45 * n), np.uint16)
+    n_moves = buf("n_moves", n, np.uint16)
+    flag_index = buf("flag_index", n, np.uint32)
+    flag_status = buf("flag_status", flag_index.size, np.uint32)
+    if n_moves.size != n:
+        raise ValueError("out['n_moves'] must have n entries")
+    totals = (ctypes.c_uint64 * 3)()
+    addr = ctypes.addressof(totals)
+    rc = _native.lib().trl_movegen_host_boards(
+        _ptr(boards), n_boards, _ptr(board_index), _ptr(cur), _ptr(alt), n, _ptr(codes), codes.size, _ptr(escapes),
+        escapes.size, _ptr(n_moves), _ptr(flag_index), _ptr(flag_status), min(flag_index.size, flag_status.size),
+        addr, addr + 8, addr + 16)
+    _native.check(rc, "trl_movegen_host_boards")
+    n_codes, n_esc, n_flag = (int(v) for v in totals)
+    raw = {"codes": codes[:n_codes], "escapes": escapes[:n_esc], "n_moves": n_moves,
+           "flag_index": flag_index[:n_flag], "flag_status": flag_status[:n_flag]}
+    if not decode:
+        return raw
+    moves, offsets = decode_move_codes(raw["codes"], raw["escapes"], n_moves)
+    status = np.zeros(n, dtype=np.uint32)
+    status[raw["flag_index"]] = raw["flag_status"]
+    return {"moves": moves, "offsets": offsets, "n_moves": n_moves, "status": status, "total": int(moves.size)}
+
+
 def movegen_device(boards, cur, alt, mask_bits=None, moves=None, n_moves=None, status=None):
     """Batched movegen on torch CUDA tensors of one device, stream-ordered on the current stream of that device.
 
